@@ -15,6 +15,10 @@ inside the timed region; pinned and pageable, pipelined and synchronous), `roofl
 `roofline_attention`, `variants` (configs[3] hi-res and configs[4] ViT-B width at 32 images per GPU), `fp32` (the
 fp32-accumulate mode), `multi_gpu_parity` (N > 1: gathered records == one GPU's records for the same images),
 `cpu_baseline` (N = 1).
+
+`--dump-outputs DIR` writes what the last timed step returned (the detection records; N > 1: the gathered record
+block) as DIR/<name>.npy.  Weights and images are seeded, so two builds run with the same arguments can be compared
+output for output.
 """
 from __future__ import annotations
 
@@ -51,7 +55,14 @@ def parse_args():
     ap.add_argument("--no-variants", action="store_true", help="skip the hi-res / ViT-B-width / fp32 side measurements")
     ap.add_argument("--no-verify", action="store_true", help="N > 1: skip the gathered-records == single-GPU check")
     ap.add_argument("--breakdown", action="store_true", help="also print a per-kernel-category time table to stderr")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step returned as DIR/<name>.npy (float32 / float64, at most 64 MB in all)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
 
 
 def variant_config(vd, name):
@@ -293,7 +304,8 @@ class Bench:
 
     def time_device(self, model, step, steps, warmup, categories):
         """W untimed steps, then K steps between CUDA events on the launching stream, bracketed by barrier + synchronize;
-        max over ranks.  `categories` are timed by the engine's own events (None = none)."""
+        max over ranks.  `categories` are timed by the engine's own events (None = none).  What the last timed step
+        returned is kept in self.last_output."""
         torch = self.torch
         for _ in range(max(warmup, 3)):
             step()
@@ -306,9 +318,10 @@ class Bench:
         self.barrier()
         ev0.record()
         for _ in range(steps):
-            step()
+            out = step()
         ev1.record()
         self.barrier()
+        self.last_output = out
         clocks = sampler.stop() if sampler else None
         ms_total = self.max_over_ranks(ev0.elapsed_time(ev1))
         launches = model.launch_count(reset=True)      # kernels of this library only (NCCL not counted)
@@ -352,6 +365,37 @@ class Bench:
                 "d2h_bytes_per_step": int(world * B * S * (24 + 24 + 4 + 4 + 16 + 1 + (52 if world > 1 else 0))),
                 "timing": "host wall clock around K steps (the call is synchronous at collect), max over ranks",
                 "pipelined": pipelined}
+
+
+DUMP_LIMIT = 64 * 10**6
+
+
+def write_outputs(out, directory: str, limit: int = DUMP_LIMIT) -> dict:
+    """Writes what one step returned to its caller as directory/<name>.npy: the DetectionRecords fields (N = 1) or the
+    all-gathered record block `packed` (N > 1).  Floating arrays are written as float32, integer ones as float64 (exact).
+    When the files would exceed `limit` bytes in all, every array keeps the same fixed, seeded sample of rows (first
+    axis) and the row indices are written as sample_rows.npy.  Returns {name: shape}."""
+    import dataclasses
+    import numpy as np
+    fields = {f.name: getattr(out, f.name) for f in dataclasses.fields(out)} if dataclasses.is_dataclass(out) else {"packed": out}
+    arrays = {}
+    for name, a in fields.items():
+        if a is None:
+            continue
+        a = a.detach().cpu().numpy() if hasattr(a, "detach") else np.asarray(a)
+        arrays[name] = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+    total = sum(a.nbytes for a in arrays.values())
+    budget = limit - 128 * (len(arrays) + 1)                # the .npy header of each file, sample_rows.npy included
+    if total > budget:
+        (n,) = {a.shape[0] for a in arrays.values()}
+        keep = budget // (total // n + 8)                   # + 8 bytes per row for its index in sample_rows
+        rows = np.sort(np.random.default_rng(0).choice(n, keep, replace=False))
+        arrays = {k: a[rows] for k, a in arrays.items()}
+        arrays["sample_rows"] = rows.astype(np.float64)
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, f"{name}.npy"), a)
+    return {k: list(a.shape) for k, a in arrays.items()}
 
 
 def peaks():
@@ -430,6 +474,9 @@ def run_ours(args):
     ms_total, launches, prof, clocks = b.time_device(model, step, args.steps, args.warmup, [dominant])
     ms_step = ms_total / args.steps
     value = world * B * args.steps / (ms_total * 1e-3)
+    if args.dump_outputs and rank == 0:
+        shapes = write_outputs(b.last_output, args.dump_outputs)
+        print(f"bench: outputs of the last timed step written to {args.dump_outputs}: {shapes}", file=sys.stderr)
     ms_total_a, _, prof_a, clocks_a = b.time_device(model, step, args.steps, 1, ["attention"]) if args.mode == "bf16" else (None, None, {}, None)
     roofline = gemm_roofline(cfg, B, args.steps, prof, dominant, ms_total, pk) if args.mode == "bf16" else None
     if roofline is not None:

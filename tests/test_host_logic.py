@@ -118,13 +118,14 @@ def test_product_does_not_import_the_oracle():
 
 
 def test_category_names_match_the_reference_table():
-    """full_categories.csv of the reference (id_in_model -> name); only checkable where the reference is mounted."""
-    path = "/root/reference/full_categories.csv"
+    """tests/golden/coco_categories.csv: the 80 categories of the COCO 2017 instance annotations (id and name as in their
+    `categories` list), numbered 0..79 in ascending COCO id, which is the reference's `id_in_model` order
+    (full_categories.csv)."""
+    path = os.path.join(ROOT, "tests", "golden", "coco_categories.csv")
     assert len(vd.COCO_CATEGORY_NAMES) == 80 and vd.COCO_CATEGORY_NAMES[0] == "person" and vd.COCO_CATEGORY_NAMES[79] == "toothbrush"
-    if not os.path.exists(path):
-        pytest.skip("reference not mounted")
     import csv
     rows = list(csv.DictReader(open(path)))
+    assert [int(r["id_in_coco"]) for r in sorted(rows, key=lambda r: int(r["id_in_model"]))] == sorted(int(r["id_in_coco"]) for r in rows)
     assert [r["name"] for r in sorted(rows, key=lambda r: float(r["id_in_model"]))] == list(vd.COCO_CATEGORY_NAMES)
 
 
