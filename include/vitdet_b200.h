@@ -120,14 +120,12 @@ int64_t vitdet_launch_count(vitdet_handle* h, int reset);
 
 /* ---- run-time switches and debug taps (no reference counterpart; used by the parity tests and A/B measurements) ----
  * Options are per handle; changing one drops the cached launch plans.  Defaults come from the environment variables of
- * the same meaning (VITDET_FUSE_LN, VITDET_FUSE_TAIL, VITDET_GEMM_PAIR, VITDET_ATTN) and otherwise are the product path.
+ * the same meaning (VITDET_FUSE_LN, VITDET_FUSE_TAIL, VITDET_GEMM_PAIR, VITDET_FP32) and otherwise are the product path.
  *   "fuse_ln"    1 (default): LayerNorm runs in the epilogue of the GEMM that produces the residual-stream row; 0: stand-alone kernel
  *   "fuse_tail"  1 (default): the last three MLP layers of a block run as one kernel; 0: three GEMM launches
  *   "gemm_pair"  1 (default): CTA-pair GEMM for K >= 512 layers; 0: never; 2: wherever it is legal
  *   "fp32_tc"    1 (default): the fp32 mode's Dense layers run on the tensor cores as three-pass split-bf16 products with
- *                float32 accumulation; 0: IEEE float32 FMA kernels on the CUDA cores (the strict reference form)
- *   "attention"  4 (default and, in a product build, the only value): attention_tc.cu; builds made with
- *                VITDET_BUILD_EXPERIMENTS=1 also hold the measured-and-dropped kernels of experiments/attention/ */
+ *                float32 accumulation; 0: IEEE float32 FMA kernels on the CUDA cores (the strict reference form) */
 int vitdet_set_option(vitdet_handle* h, const char* key, int value);
 int vitdet_get_option(const vitdet_handle* h, const char* key, int* value);
 

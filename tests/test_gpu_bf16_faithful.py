@@ -9,7 +9,6 @@ tensor-core kernel the benchmark times is covered at operator level (both GEMM k
 LayerNorm / position-add epilogues, the fused MLP tail, the slot projection, all three attention kernels), then the
 whole model, fused against unfused builds, and batch independence.
 """
-import os
 
 import numpy as np
 import pytest
@@ -192,31 +191,17 @@ def test_head_slots_kernel(B, T, D, S, mode):
         _ulp_close(got, R(ref), ulps=1.0, frac_exact=0.98, abs_tol=2e-6 * float(np.abs(ref).max()))    # float32 dot product of D terms
 
 
-def _attention_kernels():
-    """The product kernel, plus the experimental ones when the library was built with VITDET_BUILD_EXPERIMENTS=1."""
-    return ["4", "40", "8", "80", "2", "1", "3"] if os.environ.get("VITDET_BUILD_EXPERIMENTS") == "1" else ["4"]
-
-
-@pytest.mark.parametrize("kernel", _attention_kernels())
 @pytest.mark.parametrize("B,T,H,d", [(2, 1296, 8, 40), (1, 4096, 2, 40), (2, 1600, 3, 64), (3, 100, 2, 40), (1, 64, 1, 8), (2, 65, 2, 24),
                                      (5, 129, 3, 40), (2, 300, 1, 16)])
-def test_attention_kernels_against_bf16_operands(B, T, H, d, kernel):
-    """The attention kernel (and, in an experiments build, its measured-and-dropped variants) with q, k, v already bf16 and
-    the probabilities rounded to bf16 in the oracle as in the kernel; image-boundary cases (T = 65, 129, 300) put keys
-    and queries of the NEXT image into the last tiles, which the masks must keep out."""
+def test_attention_kernels_against_bf16_operands(B, T, H, d):
+    """The attention kernel with q, k, v already bf16 and the probabilities rounded to bf16 in the oracle as in the kernel;
+    image-boundary cases (T = 65, 129, 300) put keys and queries of the NEXT image into the last tiles, which the masks must
+    keep out."""
     from vision_transformer_detector_b200 import ops
     rng = np.random.default_rng(B * T + d)
     q, k, v = (R(rng.normal(size=(B, T, H, d)) * 1.5) for _ in range(3))
     ref = R(oracle.attention_core_bf16(q, k, v))
-    old = os.environ.get("VITDET_ATTN")
-    os.environ["VITDET_ATTN"] = kernel
-    try:
-        got = ops.attention(_t(q), _t(k), _t(v), mode="bf16").cpu().numpy()
-    finally:
-        if old is None:
-            del os.environ["VITDET_ATTN"]
-        else:
-            os.environ["VITDET_ATTN"] = old
+    got = ops.attention(_t(q), _t(k), _t(v), mode="bf16").cpu().numpy()
     err = np.abs(got - ref)
     # the stored context is bf16 (one ulp of slack per element); P is rounded against a different reference point
     assert (err <= bf16_ulp(ref) + 2e-3 * np.abs(ref).max()).all(), float((err / np.abs(ref).max()).max())
@@ -304,12 +289,11 @@ def test_default_model_against_the_bf16_faithful_oracle_per_block():
     m.close()
 
 
-@pytest.mark.parametrize("option,value", [("fuse_ln", 0), ("fuse_tail", 0), ("gemm_pair", 0), ("gemm_pair", 2)]
-                         + [("attention", int(k)) for k in _attention_kernels() if k != "4"])
+@pytest.mark.parametrize("option,value", [("fuse_ln", 0), ("fuse_tail", 0), ("gemm_pair", 0), ("gemm_pair", 2)])
 def test_fused_and_unfused_builds_agree(option, value):
     """Every fusion / kernel-selection switch must leave the result unchanged up to bf16 rounding: the stand-alone
-    LayerNorm kernel vs the GEMM epilogue, three GEMM launches vs the fused MLP tail, single-CTA vs CTA-pair GEMM,
-    the three attention kernels — per encoder block (taps) and on the logits."""
+    LayerNorm kernel vs the GEMM epilogue, three GEMM launches vs the fused MLP tail, single-CTA vs CTA-pair GEMM — per
+    encoder block (taps) and on the logits."""
     cfg = vd.DetectorConfig()
     w = vd.random_weights(cfg, seed=1, spread=True)
     x = images(cfg, 2)

@@ -24,15 +24,6 @@ NVCC_FLAGS = [
 ]
 
 
-# VITDET_BUILD_EXPERIMENTS=1 also compiles the measured-and-dropped attention kernels of experiments/attention/ and lets the
-# "attention" option (VITDET_ATTN) select them, so that profiles/r02_attention_analysis.md can be reproduced.
-EXPERIMENTS_DIR = os.path.join(os.path.dirname(PKG_DIR), "experiments", "attention")
-EXPERIMENT_SOURCES = ["attention_tc8.cu", "attention_tcp.cu", "attention_tc8p.cu", "attention_pp.cu", "attention_sw.cu", "attention_tc3.cu"]
-
-
-def _with_experiments() -> bool:
-    return os.environ.get("VITDET_BUILD_EXPERIMENTS", "0") == "1"
-
 
 def _nvcc() -> str:
     for cand in (os.environ.get("NVCC"), "/usr/local/cuda/bin/nvcc", "nvcc"):
@@ -52,11 +43,6 @@ def _source_hash() -> str:
         with open(path, "rb") as f:
             h.update(f.read())
     h.update(" ".join(NVCC_FLAGS).encode())
-    if _with_experiments():
-        h.update(b"experiments")
-        for name in EXPERIMENT_SOURCES:
-            with open(os.path.join(EXPERIMENTS_DIR, name), "rb") as f:
-                h.update(f.read())
     return h.hexdigest()
 
 
@@ -91,13 +77,10 @@ def build(force: bool = False, verbose: bool = False) -> str:
     os.makedirs(obj_dir, exist_ok=True)
     procs = []
     objs = []
-    extra = ["-DVITDET_EXPERIMENTS"] if _with_experiments() else []
     # A/B builds (scripts/gpu_ab_lib.sh): extra -D switches; such a build is never stamped as current
-    extra += os.environ.get("VITDET_EXTRA_NVCC_FLAGS", "").split()
-    jobs = [(src, os.path.join(CSRC, src)) for src in SOURCES]
-    if _with_experiments():
-        jobs += [(src, os.path.join(EXPERIMENTS_DIR, src)) for src in EXPERIMENT_SOURCES]
-    for src, path in jobs:
+    extra = os.environ.get("VITDET_EXTRA_NVCC_FLAGS", "").split()
+    for src in SOURCES:
+        path = os.path.join(CSRC, src)
         obj = os.path.join(obj_dir, src.replace(".cu", ".o"))
         objs.append(obj)
         cmd = [nvcc, *NVCC_FLAGS, *extra, "-I", INCLUDE, "-I", CSRC, "-c", path, "-o", obj]

@@ -5,7 +5,7 @@
 //   det.py:417-495 -> transform_predictions det.py:586-647 + thresholds det.py:2257-2283/1359-1384.
 //
 // Data layout in HBM (bf16 mode; the fp32 mode uses the same shapes with 4 bytes per element: IEEE float32 for the
-// CUDA-core kernels, or two bf16 planes (hi | lo) per buffer for the tensor-core form, see forward_fp32_tc):
+// CUDA-core kernels, or two bf16 planes (hi | lo) per buffer for the tensor-core form, see Form):
 //   x     f32  [B*T, D4]        residual stream, kept in f32 for the whole batch (145 KB / image)
 //   per encoder chunk of Bc images (Mc = Bc*T rows), reused by every chunk:
 //   patch bf16 [Mc, P8]         extract_patches output, (row, col, channel) order
@@ -33,6 +33,7 @@
 #include <mutex>
 #include <string>
 #include <thread>
+#include <tuple>
 #include <vector>
 
 #include "../../include/vitdet_b200.h"
@@ -71,8 +72,6 @@ struct Options {
     int fuse_tail = 1;     // VITDET_FUSE_TAIL=0: the last three MLP layers as separate GEMM launches
     int gemm_pair = 1;     // VITDET_GEMM_PAIR=0 never / all (2) wherever legal / default: K >= 512 layers
     int fp32_tc = 1;       // VITDET_FP32=simt: the fp32 mode on CUDA-core IEEE kernels instead of split-bf16 tensor-core GEMMs
-    int attention = 4;     // VITDET_ATTN: 4 = attention_tc.cu (the product kernel); builds with VITDET_BUILD_EXPERIMENTS=1 also take
-                           // 40 persistent, 8 / 80 split score rows, 2 ping-pong, 1 software-pipelined, 3 three CTAs per SM
 };
 
 static Options env_options() {
@@ -81,24 +80,7 @@ static Options env_options() {
     if (const char* e = getenv("VITDET_FUSE_TAIL")) o.fuse_tail = strcmp(e, "0") != 0;
     if (const char* e = getenv("VITDET_GEMM_PAIR")) o.gemm_pair = strcmp(e, "0") == 0 ? 0 : (strcmp(e, "all") == 0 ? 2 : 1);
     if (const char* e = getenv("VITDET_FP32")) o.fp32_tc = strcmp(e, "simt") != 0;
-#ifdef VITDET_EXPERIMENTS
-    if (const char* e = getenv("VITDET_ATTN")) { const int v = atoi(e); if (v == 1 || v == 2 || v == 3 || v == 4 || v == 8 || v == 40 || v == 80) o.attention = v; }
-#endif
     return o;
-}
-
-static cudaError_t attn_launch(int version, const AttnPlan& plan, int num_sms, cudaStream_t st) {
-#ifdef VITDET_EXPERIMENTS
-    // measured-and-dropped kernels of experiments/attention/ (profiles/r02_attention_analysis.md)
-    if (version == 8) return attn_tc8_launch(plan, st);
-    if (version == 80) return attn_tc8p_launch(plan, num_sms, st);
-    if (version == 2) return attn_pp_launch(plan, num_sms, st);
-    if (version == 1) return attn_sw_launch(plan, num_sms, st);
-    if (version == 3) return attn_tc3_launch(plan, st);
-    if (version == 40) return attn_tcp_launch(plan, num_sms, st);
-#endif
-    (void)version; (void)num_sms;
-    return attn_tc_launch(plan, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -341,6 +323,18 @@ struct HostSlot {
     }
 };
 
+// Launch plans of the tensor-core forms for one encoder chunk or for the head, in launch order (see plan_cursor)
+struct AttnTcPlan {
+    AttnPlan plan;
+    CUtensorMap lo;                // Split form: tensor map of the lo plane of qkv
+};
+struct Plans {
+    bool complete = false;         // a whole pass has been recorded
+    std::vector<TcGemmPlan> gemm;
+    std::vector<AttnTcPlan> attn;
+    std::vector<MlpTailPlan> tail;
+};
+
 }  // namespace vitdet
 
 using namespace vitdet;
@@ -371,27 +365,12 @@ struct vitdet_handle {
     // workspace (grow-only)
     DevBuf x, patch, y, qkv, ctx, u0, u1, s, h0, h1;
     DevBuf tmp32;                       // fp32 tensor-core mode: float32 staging of the patches / LayerNorm rows before their split, planes of the slot matrix
-    // cached plans
-    struct EncPlans {
-        bool valid = false;
-        TcGemmPlan proj;
-        std::vector<TcGemmPlan> qkv, out;
-        std::vector<std::vector<TcGemmPlan>> mlp;
-        std::vector<AttnPlan> attn;
-        bool tail_fused = false;              // last three MLP layers (+ residual + next LayerNorm) run as mlp_tail_kernel
-        std::vector<MlpTailPlan> tail;
-    };
-    std::map<int, EncPlans> enc_plans;      // key: images in the chunk
-    struct HeadPlans {
-        bool valid = false;
-        std::vector<TcGemmPlan> dense;
-    };
-    std::map<int, HeadPlans> head_plans;    // key: batch
-    std::map<long long, std::vector<TcGemmPlan>> plans32;    // fp32-accumulate mode on the tensor cores: GEMM plans in launch order, key (B << 20) | chunk
+    // cached plans, key (encoder chunk / head, arithmetic form, images in the chunk / batch); cleared when a buffer moves
+    std::map<std::tuple<int, int, int>, Plans> plans;
 
     // debug taps (vitdet_debug_taps): residual stream after the patch embedding and after every block, of the last forward
     bool weights_dirty = false;         // set_weight ran since the last forward: the pack kernels (legacy stream) must finish first
-    int s_layout_mode = -1;             // arithmetic mode the slot matrix `s` was last laid out for (its pad columns are zeroed per layout)
+    int s_layout_es = 0;                // element size the slot matrix `s` was last laid out for (its pad columns are zeroed per layout)
     bool taps_on = false;
     DevBuf taps;                        // f32 [(L + 1)][B*T, D4]
     int taps_B = 0;
@@ -561,30 +540,58 @@ static int build_weight_table(vitdet_handle* h) {
 }
 
 // ------------------------------------------------------------------------------------------------
+// arithmetic forms
+// ------------------------------------------------------------------------------------------------
+// Bf16:  bf16 operands and stored activations, one tcgen05 pass per Dense (VITDET_MODE_BF16).
+// Split: the fp32 mode on the tensor cores (north_star: <= 1e-3 against the float32 reference).  Every float32 activation
+//        that feeds a Dense layer or the attention core travels as two bf16 planes (hi = bf16(x), lo = bf16(x - hi)) and
+//        every Dense is three tcgen05 passes (hi*hi + hi*lo + lo*hi, float32 accumulation in TMEM) through the same two
+//        GEMM kernels as Bf16, with exact expf-based activations in the epilogue; attention is attention_tcs.cu.  The
+//        residual stream, LayerNorm, the head's slot projection and last Dense stay IEEE float32.  Buffers are sized
+//        as the fp32 mode's (4 bytes per element): the hi plane in the first half, the lo plane in the second (planes_of).
+// Ieee:  the fp32 mode on IEEE float32 CUDA-core kernels (gemm_simt.cu, attn_f32): "fp32_tc" = 0, or heads wider than
+//        the split attention kernel takes (it holds hi and lo tiles: one 64-column box per head).
+enum class Form { Bf16, Split, Ieee };
+
+static Form pick_form(int mode, const Options& o, int key_dim) {
+    if (mode == VITDET_MODE_BF16) return Form::Bf16;
+    return o.fp32_tc && key_dim <= kMaxKeyDimSplit ? Form::Split : Form::Ieee;
+}
+
+struct Planes { __nv_bfloat16* hi; __nv_bfloat16* lo; };
+static Planes planes_of(const DevBuf& b) {
+    return Planes{b.as<__nv_bfloat16>(), reinterpret_cast<__nv_bfloat16*>(b.as<char>() + (b.bytes / 2 & ~static_cast<size_t>(255)))};
+}
+
+// ------------------------------------------------------------------------------------------------
 // Dense dispatch
 // ------------------------------------------------------------------------------------------------
+// One activation matrix as a GEMM operand: bf16 or f32 rows, or the Split form's (hi, lo) planes (lo != nullptr).
+struct Operand { void* p = nullptr; void* lo = nullptr; int ld = 0; };
+
 struct DenseCall {
-    const void* A; int lda;
+    Operand A;
     const DenseW* w;
+    int M;
     const float* pos = nullptr; int pos_period = 1;
     const float* resid = nullptr; int ldr = 0;
-    void* out; int ldc; int out_f32; int act;
-    int M;
-    // optional fused LayerNorm of the output row (bf16 mode, N <= 32): see GemmDesc
+    Operand out; int out_f32 = 0; int act = ACT_NONE;     // out.lo: the result is stored as (hi, lo) planes
+    // optional fused LayerNorm of the output row (Bf16, N <= 32): see GemmDesc
     const float* ln_gamma = nullptr; const float* ln_beta = nullptr; void* ln_out = nullptr; int ln_ld = 0; float ln_eps = 1e-3f;
 };
 
-static GemmDesc make_desc(const DenseCall& c, int mode) {
+static GemmDesc make_desc(const DenseCall& c, Form f) {
     GemmDesc g;
-    g.A = c.A; g.lda = c.lda;
-    g.W = mode == VITDET_MODE_BF16 ? c.w->w16.p : c.w->w32.p;
-    g.ldw = mode == VITDET_MODE_BF16 ? c.w->ld16 : c.w->ld32;
+    g.A = c.A.p; g.A_lo = c.A.lo; g.lda = c.A.ld;
+    g.W = f == Form::Ieee ? c.w->w32.p : c.w->w16.p;
+    g.ldw = f == Form::Ieee ? c.w->ld32 : c.w->ld16;
     g.M = c.M; g.N = c.w->N; g.K = c.w->K;
     g.bias = c.w->bias.as<float>();
     g.pos = c.pos; g.pos_period = c.pos_period;
     g.resid = c.resid; g.ldr = c.ldr;
-    g.out = c.out; g.ldc = c.ldc; g.out_f32 = c.out_f32; g.act = c.act;
+    g.out = c.out.p; g.out_lo = c.out.lo; g.ldc = c.out.ld; g.out_f32 = c.out_f32; g.act = c.act;
     g.ln_gamma = c.ln_gamma; g.ln_beta = c.ln_beta; g.ln_out = c.ln_out; g.ln_ld = c.ln_ld; g.ln_eps = c.ln_eps;
+    if (f == Form::Split) { g.split = 1; g.precise = 1; g.W_lo = c.w->w16_lo(); g.out_split = c.out.lo != nullptr; }
     return g;
 }
 
@@ -601,20 +608,67 @@ static bool use_pair_kernel(int pair_mode, const GemmDesc& g) {
     return pair_mode == 2 || g.K >= 512;
 }
 
-static int make_tc_plan(TcGemmPlan* plan, const GemmDesc& g, int num_sms, int pair_mode) {
+// Tensor-core plan of one Dense (Bf16 / Split)
+static int plan_dense(TcGemmPlan* plan, const DenseCall& c, Form f, int num_sms, int pair_mode) {
+    const GemmDesc g = make_desc(c, f);
     plan->pair = use_pair_kernel(pair_mode, g) ? 1 : 0;
-    return plan->pair ? tc2_gemm_make_plan(plan, g, num_sms) : tc_gemm_make_plan(plan, g, num_sms);
+    const int rc = plan->pair ? tc2_gemm_make_plan(plan, g, num_sms) : tc_gemm_make_plan(plan, g, num_sms);
+    if (rc) return fail(VITDET_E_INVALID, "tensor-core GEMM plan (M=%d N=%d K=%d lda=%d ldc=%d) failed: %d", g.M, g.N, g.K, g.lda, g.ldc, rc);
+    return 0;
+}
+
+static int launch_tc(TcGemmPlan plan /*by value: out / resid are patched per launch*/, void* out, const float* resid,
+                     cudaStream_t st) {
+    plan.desc.out = out;
+    plan.desc.resid = resid;
+    cudaError_t e = plan.pair ? tc2_gemm_launch(plan, st) : tc_gemm_launch(plan, st);
+    if (e != cudaSuccess) return fail(VITDET_E_CUDA, "tc_gemm_launch failed: %s", cudaGetErrorString(e));
+    return 0;
+}
+
+static int launch_simt(const DenseCall& c, cudaStream_t st) {
+    GemmDesc g = make_desc(c, Form::Ieee);
+    cudaError_t e = simt_gemm_launch(g, st);
+    if (e != cudaSuccess) return fail(VITDET_E_CUDA, "simt_gemm_launch(M=%d N=%d K=%d) failed: %s", g.M, g.N, g.K, cudaGetErrorString(e));
+    return 0;
+}
+
+// One Dense launch without a plan cache (operator entry points)
+static int dense_once(const DenseCall& c, Form f, int num_sms, int pair_mode, cudaStream_t st) {
+    if (f == Form::Ieee) return launch_simt(c, st);
+    TcGemmPlan plan;
+    RC_TRY(plan_dense(&plan, c, f, num_sms, pair_mode));
+    return launch_tc(plan, c.out.p, c.resid, st);
 }
 
 // The fused LayerNorm needs the whole residual-stream row in one epilogue thread (D <= 32).
 static bool ln_is_fused(const vitdet_handle* h) { return h->opt.fuse_ln && h->D <= 32; }
 static bool tail_fusion_enabled(const vitdet_handle* h) { return h->opt.fuse_tail != 0; }
 
-static int plan_dense(vitdet_handle* h, const DenseCall& c, TcGemmPlan* plan) {
-    GemmDesc g = make_desc(c, VITDET_MODE_BF16);
-    int rc = make_tc_plan(plan, g, h->num_sms, h->opt.gemm_pair);
-    if (rc) return fail(VITDET_E_INVALID, "tc_gemm_make_plan(M=%d N=%d K=%d lda=%d ldc=%d) failed: %d", g.M, g.N, g.K, g.lda, g.ldc, rc);
+// ------------------------------------------------------------------------------------------------
+// attention dispatch
+// ------------------------------------------------------------------------------------------------
+static AttnDesc attn_desc(const Operand& qkv, const Operand& ctx, int B, int T, int H, int d, int hp) {
+    AttnDesc ad;
+    ad.qkv = qkv.p; ad.ldq = qkv.ld; ad.ctx = ctx.p; ad.ldo = ctx.ld;
+    ad.B = B; ad.T = T; ad.H = H; ad.d = d; ad.hp = hp;
+    ad.scale = 1.f / sqrtf(static_cast<float>(d));
+    return ad;
+}
+
+// Tensor-core attention plan; the Split form also maps the lo plane of qkv (same shape and pitch as the hi plane in `ad`).
+static int attn_plan(AttnTcPlan* p, const AttnDesc& ad, const void* qkv_lo) {
+    int rc = attn_bf16_make_plan(&p->plan, ad);
+    if (!rc && qkv_lo) rc = make_tmap_bf16_2d(&p->lo, qkv_lo, ad.B * ad.T, 3 * ad.H * ad.hp, ad.ldq, 64);
+    if (rc) return fail(VITDET_E_INVALID, "attention plan (B=%d T=%d H=%d d=%d) failed: %d", ad.B, ad.T, ad.H, ad.d, rc);
     return 0;
+}
+
+// ctx_lo: the Split form's lo plane of the context rows; `p` is unused by Ieee
+static cudaError_t attn_launch(Form f, const AttnDesc& ad, const AttnTcPlan* p, void* ctx_lo, cudaStream_t st) {
+    if (f == Form::Bf16) return attn_tc_launch(p->plan, st);
+    if (f == Form::Split) return attn_tcs_launch(p->plan, p->lo, ctx_lo, st);
+    return attn_f32_launch(ad, st);
 }
 
 // ------------------------------------------------------------------------------------------------
@@ -626,14 +680,14 @@ struct Dims {
     int Tp;          // row pitch of the slot matrix s [B*S, T]: T rounded up to a 16-byte multiple (pads stay zero)
 };
 
-static Dims dims_for(const vitdet_handle* h, int mode) {
+static Dims dims_for(const vitdet_handle* h, Form f) {
     Dims m;
     const vitdet_config& c = h->cfg;
-    m.es = mode == VITDET_MODE_BF16 ? 2 : 4;
+    m.es = f == Form::Bf16 ? 2 : 4;
     m.D4 = round_up(h->D, 4);
     m.D8 = round_up(h->D, 8);
     m.Pld = round_up(h->PK, 8);
-    m.Tp = round_up(h->T, mode == VITDET_MODE_BF16 ? 8 : 4);
+    m.Tp = round_up(h->T, f == Form::Bf16 ? 8 : 4);
     m.w_qkv = 3 * h->H * h->hp;
     m.w_ctx = h->H * h->hp;
     // MLP ping-pong: layer j writes buffer j & 1; widest even / odd layer outputs.
@@ -652,142 +706,81 @@ static Dims dims_for(const vitdet_handle* h, int mode) {
 
 static size_t a256(size_t v) { return (v + 255) / 256 * 256; }
 
-static size_t workspace_bytes(const vitdet_handle* h, int B, int mode) {
-    const Dims m = dims_for(h, mode);
-    const size_t bc = static_cast<size_t>(B < h->chunk ? B : h->chunk);
-    const size_t Mc = bc * h->T, R = static_cast<size_t>(B) * h->S;
-    size_t tot = 0;
-    tot += a256(static_cast<size_t>(B) * h->T * m.D4 * 4);
-    tot += a256(Mc * m.Pld * m.es) + a256(Mc * m.D8 * m.es) + a256(Mc * m.w_qkv * m.es) + a256(Mc * m.w_ctx * m.es);
-    tot += a256(Mc * m.w_u0 * m.es) + a256(Mc * m.w_u1 * m.es);
-    tot += a256(R * m.Tp * m.es) + a256(R * m.w_h0 * m.es) + a256(R * m.w_h1 * m.es);
+enum WorkspaceBuf { WS_X, WS_PATCH, WS_Y, WS_QKV, WS_CTX, WS_U0, WS_U1, WS_S, WS_H0, WS_H1, WS_TMP32, WS_COUNT };
+
+// Bytes of every workspace buffer a forward of B images in form f uses.  In the Split form a buffer that holds planes
+// keeps the second one at the 256-byte boundary below the middle of the allocation (planes_of); kPlaneSlack keeps that
+// boundary above the end of the first plane.  tmp32 (Split only) stages the float32 patches / LayerNorm rows before their
+// split, and holds the planes of the slot matrix.
+static void workspace_layout(const vitdet_handle* h, int B, Form f, size_t bytes[WS_COUNT]) {
+    constexpr size_t kPlaneSlack = 1024;
+    const Dims m = dims_for(h, f);
+    const size_t Mc = static_cast<size_t>(B < h->chunk ? B : h->chunk) * h->T, R = static_cast<size_t>(B) * h->S;
+    const size_t slack = f == Form::Split ? kPlaneSlack : 0;
+    bytes[WS_X] = static_cast<size_t>(B) * h->T * m.D4 * 4;
+    bytes[WS_PATCH] = Mc * m.Pld * m.es + slack;
+    bytes[WS_Y] = Mc * m.D8 * m.es + slack;
+    bytes[WS_QKV] = Mc * m.w_qkv * m.es + slack;
+    bytes[WS_CTX] = Mc * m.w_ctx * m.es + slack;
+    bytes[WS_U0] = Mc * m.w_u0 * m.es + slack;
+    bytes[WS_U1] = Mc * m.w_u1 * m.es + slack;
+    bytes[WS_S] = R * m.Tp * m.es;
+    bytes[WS_H0] = R * m.w_h0 * m.es + slack;
+    bytes[WS_H1] = R * m.w_h1 * m.es + slack;
+    bytes[WS_TMP32] = 0;
+    if (f == Form::Split) {
+        const size_t rows = Mc * round_up(h->PK > h->D ? h->PK : h->D, 4) * 4;
+        const size_t slots = R * round_up(h->T, 8) * 4 + kPlaneSlack;
+        bytes[WS_TMP32] = rows > slots ? rows : slots;
+    }
+}
+
+static size_t workspace_bytes(const vitdet_handle* h, int B, Form f) {
+    size_t bytes[WS_COUNT], tot = 0;
+    workspace_layout(h, B, f, bytes);
+    for (size_t b : bytes) tot += a256(b);
     return tot;
 }
 
-static int ensure_workspace(vitdet_handle* h, int B, int mode) {
-    const Dims m = dims_for(h, mode);
-    const size_t bc = static_cast<size_t>(B < h->chunk ? B : h->chunk);
-    const size_t Mc = bc * h->T, R = static_cast<size_t>(B) * h->S;
-    const void* before[10] = {h->x.p, h->patch.p, h->y.p, h->qkv.p, h->ctx.p, h->u0.p, h->u1.p, h->s.p, h->h0.p, h->h1.p};
-    // + kPlaneSlack: in the fp32 tensor-core mode a buffer holds two bf16 planes, the second one at the 256-byte
-    // boundary below the middle of the allocation (planes_of); the slack keeps that boundary above the first plane
-    constexpr size_t kPlaneSlack = 1024;
-    RC_TRY(h->x.ensure(static_cast<size_t>(B) * h->T * m.D4 * 4));
-    RC_TRY(h->patch.ensure(Mc * m.Pld * m.es + kPlaneSlack));
-    RC_TRY(h->y.ensure(Mc * m.D8 * m.es + kPlaneSlack));
-    RC_TRY(h->qkv.ensure(Mc * m.w_qkv * m.es + kPlaneSlack));
-    RC_TRY(h->ctx.ensure(Mc * m.w_ctx * m.es + kPlaneSlack));
-    RC_TRY(h->u0.ensure(Mc * m.w_u0 * m.es + kPlaneSlack));
-    RC_TRY(h->u1.ensure(Mc * m.w_u1 * m.es + kPlaneSlack));
-    {
-        const void* s_before = h->s.p; const size_t s_bytes = h->s.bytes;
-        RC_TRY(h->s.ensure(R * m.Tp * m.es));
-        // the pad columns [T, Tp) of every row are read by the first head GEMM's last k-step and never written
-        if (m.Tp != h->T && (h->s.p != s_before || h->s.bytes != s_bytes || h->s_layout_mode != mode)) { CU_TRY(cudaMemset(h->s.p, 0, h->s.bytes)); CU_TRY(cudaDeviceSynchronize()); }
-        h->s_layout_mode = mode;
-    }
-    RC_TRY(h->h0.ensure(R * m.w_h0 * m.es + kPlaneSlack));
-    RC_TRY(h->h1.ensure(R * m.w_h1 * m.es + kPlaneSlack));
-    const void* after[10] = {h->x.p, h->patch.p, h->y.p, h->qkv.p, h->ctx.p, h->u0.p, h->u1.p, h->s.p, h->h0.p, h->h1.p};
-    for (int i = 0; i < 10; ++i) {
-        if (before[i] != after[i]) {     // a buffer moved: every cached TMA descriptor is stale
-            h->enc_plans.clear();
-            h->head_plans.clear();
-            h->plans32.clear();
-            break;
+static int ensure_workspace(vitdet_handle* h, int B, Form f) {
+    DevBuf* bufs[WS_COUNT] = {&h->x, &h->patch, &h->y, &h->qkv, &h->ctx, &h->u0, &h->u1, &h->s, &h->h0, &h->h1, &h->tmp32};
+    size_t need[WS_COUNT];
+    workspace_layout(h, B, f, need);
+    const Dims m = dims_for(h, f);
+    bool moved = false;
+    for (int i = 0; i < WS_COUNT; ++i) {
+        const void* p = bufs[i]->p;
+        const size_t bytes = bufs[i]->bytes;
+        RC_TRY(bufs[i]->ensure(need[i]));
+        moved = moved || bufs[i]->p != p;
+        if (i == WS_S) {
+            // the pad columns [T, Tp) of every row are read by the first head GEMM's last k-step and never written
+            if (m.Tp != h->T && (h->s.p != p || h->s.bytes != bytes || h->s_layout_es != m.es)) { CU_TRY(cudaMemset(h->s.p, 0, h->s.bytes)); CU_TRY(cudaDeviceSynchronize()); }
+            h->s_layout_es = m.es;
         }
     }
+    if (moved) h->plans.clear();     // a buffer moved: every cached TMA descriptor is stale
     return 0;
 }
 
 // ------------------------------------------------------------------------------------------------
-// plans (bf16 mode): TMA descriptors for every GEMM / attention launch of one encoder chunk
+// plan cache: the tensor-core forms' launch plans of one encoder chunk or of the head, in launch order, recorded by the
+// first forward pass that needs them and replayed afterwards
 // ------------------------------------------------------------------------------------------------
-static int build_enc_plans(vitdet_handle* h, int bc, vitdet_handle::EncPlans* ep) {
-    const Dims m = dims_for(h, VITDET_MODE_BF16);
-    const vitdet_config& c = h->cfg;
-    const int Mc = bc * h->T;
-    const int L = c.repeat_times, q = c.mlp_quantities;
-    float* xdummy = h->x.as<float>();
+enum PlanPart { kEncoderPlans = 0, kHeadPlans = 1 };
 
-    // In bf16 mode with D <= 32 every LayerNorm is fused into the epilogue of the GEMM that produces the residual
-    // stream row (projection -> LN1 of block 0; attention output -> LN2; last MLP layer -> LN1 of the next block).
-    const bool fuse_ln = ln_is_fused(h);
-    auto with_ln = [&](DenseCall c, DevBuf& gamma, DevBuf& beta) {
-        if (fuse_ln) { c.ln_gamma = gamma.as<float>(); c.ln_beta = beta.as<float>(); c.ln_out = h->y.p; c.ln_ld = m.D8; c.ln_eps = h->cfg.ln_epsilon; }
-        return c;
-    };
-    DenseCall pc{h->patch.p, m.Pld, &h->proj, h->pos.as<float>(), h->T, nullptr, 0, xdummy, m.D4, 1, ACT_NONE, Mc};
-    RC_TRY(plan_dense(h, with_ln(pc, h->blocks[0].ln1_g, h->blocks[0].ln1_b), &ep->proj));
+struct PlanCursor {
+    Plans* p;
+    bool record;                   // first pass: make every plan and append it
+    size_t gemm = 0, attn = 0, tail = 0;
+};
 
-    ep->qkv.resize(L); ep->out.resize(L); ep->attn.resize(L); ep->mlp.assign(L, std::vector<TcGemmPlan>(q));
-    for (int i = 0; i < L; ++i) {
-        BlockW& b = h->blocks[i];
-        DenseCall qc{h->y.p, m.D8, &b.qkv, nullptr, 1, nullptr, 0, h->qkv.p, m.w_qkv, 0, ACT_NONE, Mc};
-        RC_TRY(plan_dense(h, qc, &ep->qkv[i]));
-        AttnDesc ad;
-        ad.qkv = h->qkv.p; ad.ldq = m.w_qkv; ad.ctx = h->ctx.p; ad.ldo = m.w_ctx;
-        ad.B = bc; ad.T = h->T; ad.H = h->H; ad.d = h->d; ad.hp = h->hp;
-        ad.scale = 1.f / sqrtf(static_cast<float>(h->d));
-        int rc = attn_bf16_make_plan(&ep->attn[i], ad);
-        if (rc) return fail(VITDET_E_INVALID, "attn_bf16_make_plan failed: %d", rc);
-        DenseCall oc{h->ctx.p, m.w_ctx, &b.out, nullptr, 1, xdummy, m.D4, xdummy, m.D4, 1, ACT_NONE, Mc};
-        RC_TRY(plan_dense(h, with_ln(oc, b.ln2_g, b.ln2_b), &ep->out[i]));
-        // The last three layers fuse into one kernel when their widths fit it (default model: 224 -> 112 -> 56 -> 28).
-        bool tail = false;
-        if (fuse_ln && tail_fusion_enabled(h) && q >= 4) {
-            const int N3[3] = {b.mlp[q - 3].N, b.mlp[q - 2].N, b.mlp[q - 1].N};
-            const int K3[3] = {b.mlp[q - 3].K, b.mlp[q - 2].K, b.mlp[q - 1].K};
-            tail = mlp_tail_supported(N3, K3);
-        }
-        if (i == 0) { ep->tail_fused = tail; ep->tail.assign(tail ? L : 0, MlpTailPlan()); }
-        const void* a = h->y.p; int lda = m.D8;
-        for (int j = 0; j < q; ++j) {
-            if (tail && j == q - 3) {
-                MlpTailDesc td;
-                td.A = a; td.lda = lda; td.M = Mc;
-                for (int l = 0; l < 3; ++l) {
-                    DenseW& w = b.mlp[q - 3 + l];
-                    td.N[l] = w.N; td.K[l] = w.K; td.W[l] = w.w16.p; td.ldw[l] = w.ld16; td.bias[l] = w.bias.as<float>();
-                }
-                td.x = xdummy; td.ldx = m.D4; td.act = h->act;
-                if (i + 1 < L) {
-                    td.ln_gamma = h->blocks[i + 1].ln1_g.as<float>(); td.ln_beta = h->blocks[i + 1].ln1_b.as<float>();
-                    td.ln_eps = h->cfg.ln_epsilon; td.ln_out = h->y.p; td.ln_ld = m.D8;
-                }
-                int rc2 = mlp_tail_make_plan(&ep->tail[i], td, h->num_sms);
-                if (rc2) return fail(VITDET_E_INVALID, "mlp_tail_make_plan failed: %d", rc2);
-                ep->tail[i].valid = true;
-                break;
-            }
-            const bool last = j == q - 1;
-            void* o = last ? static_cast<void*>(xdummy) : ((j & 1) ? h->u1.p : h->u0.p);
-            const int ldo = last ? m.D4 : round_up(b.mlp[j].N, 8);
-            DenseCall mc{a, lda, &b.mlp[j], nullptr, 1, last ? xdummy : nullptr, last ? m.D4 : 0, o, ldo, last ? 1 : 0, h->act, Mc};
-            if (last && i + 1 < L) mc = with_ln(mc, h->blocks[i + 1].ln1_g, h->blocks[i + 1].ln1_b);
-            RC_TRY(plan_dense(h, mc, &ep->mlp[i][j]));
-            a = o; lda = ldo;
-        }
-    }
-    ep->valid = true;
-    return 0;
+// part: encoder chunk of n images, or the head of a batch of n
+static PlanCursor plan_cursor(vitdet_handle* h, PlanPart part, Form f, int n) {
+    Plans& p = h->plans[std::make_tuple(static_cast<int>(part), static_cast<int>(f), n)];
+    if (!p.complete) p = Plans();       // (an earlier recording stopped at an error)
+    return PlanCursor{&p, !p.complete};
 }
-
-static int build_head_plans(vitdet_handle* h, int B, vitdet_handle::HeadPlans* hp) {
-    const int R = B * h->S;
-    hp->dense.resize(h->head.size());
-    const void* a = h->s.p; int lda = dims_for(h, VITDET_MODE_BF16).Tp;
-    for (size_t i = 0; i < h->head.size(); ++i) {
-        void* o = (i & 1) ? h->h1.p : h->h0.p;
-        const int ldo = round_up(h->head[i].N, 8);
-        DenseCall hc{a, lda, &h->head[i], nullptr, 1, nullptr, 0, o, ldo, 0, h->act, R};
-        RC_TRY(plan_dense(h, hc, &hp->dense[i]));
-        a = o; lda = ldo;
-    }
-    hp->valid = true;
-    return 0;
-}
-
 // ------------------------------------------------------------------------------------------------
 // profiling scopes
 // ------------------------------------------------------------------------------------------------
@@ -837,22 +830,6 @@ static int prof_collect(vitdet_handle* h) {
 // ------------------------------------------------------------------------------------------------
 // forward
 // ------------------------------------------------------------------------------------------------
-static int launch_tc(TcGemmPlan plan /*by value: out / resid are patched per launch*/, void* out, const float* resid,
-                     cudaStream_t st) {
-    plan.desc.out = out;
-    plan.desc.resid = resid;
-    cudaError_t e = plan.pair ? tc2_gemm_launch(plan, st) : tc_gemm_launch(plan, st);
-    if (e != cudaSuccess) return fail(VITDET_E_CUDA, "tc_gemm_launch failed: %s", cudaGetErrorString(e));
-    return 0;
-}
-
-static int launch_simt(const DenseCall& c, cudaStream_t st) {
-    GemmDesc g = make_desc(c, VITDET_MODE_FP32);
-    cudaError_t e = simt_gemm_launch(g, st);
-    if (e != cudaSuccess) return fail(VITDET_E_CUDA, "simt_gemm_launch(M=%d N=%d K=%d) failed: %s", g.M, g.N, g.K, cudaGetErrorString(e));
-    return 0;
-}
-
 // Optional staging information of predict_host: images arrive in sub-chunks of `ready_gran` images,
 // sub-chunk i being complete when ready[i] fires; lead_chunks makes the first encoder chunks small so that
 // compute starts after one sub-chunk and the rest of the copy hides behind it.
@@ -863,168 +840,33 @@ struct ForwardOpts {
     int in_u8 = 0;                    // images are uint8 pixels; the patch kernel normalises them (x / 127.5 - 1)
 };
 
-// ------------------------------------------------------------------------------------------------
-// fp32-accumulate mode on the tensor cores (north_star: <= 1e-3 against the float32 reference).
-// Every float32 activation that feeds a Dense layer travels as two bf16 planes (hi = bf16(x), lo = bf16(x - hi)) and
-// every Dense is three tcgen05 passes (hi*hi + hi*lo + lo*hi, float32 accumulation in TMEM) through the same two GEMM
-// kernels as the bf16 mode, with exact expf-based activations in the epilogue.  The residual stream, LayerNorm, the
-// softmax of the attention core (attn_f32_kernel) and the head's slot projection / last Dense stay in IEEE float32.
-// Buffers are the fp32 mode's (4 bytes per element): the hi plane in the first half, the lo plane in the second.
-// ------------------------------------------------------------------------------------------------
-struct Planes { __nv_bfloat16* hi; __nv_bfloat16* lo; };
-static Planes planes_of(const DevBuf& b) {
-    return Planes{b.as<__nv_bfloat16>(), reinterpret_cast<__nv_bfloat16*>(b.as<char>() + (b.bytes / 2 & ~static_cast<size_t>(255)))};
+// vitdet_decode_params / vitdet_detections -> the decode kernels' arguments (either may be null: defaults / no outputs)
+static void decode_args(const vitdet_decode_params* p, int apply_transform, const vitdet_detections* o, float* logits,
+                        DecodeParams* dp, DecodeOut* out) {
+    out->logits = logits;
+    if (p) {
+        dp->obj_thr = p->objectness_threshold; dp->cls_thr = p->classification_threshold;
+        dp->strict = p->strict; dp->img_h = p->image_h; dp->img_w = p->image_w; dp->classes = p->classes;
+        dp->apply_transform = apply_transform;
+        dp->corner_scale = p->corner_scale > 0.f ? p->corner_scale : 1.f;
+    }
+    if (o) {
+        out->decoded = o->decoded; out->class_id = o->class_id; out->class_conf = o->class_conf;
+        out->keep = o->keep; out->corners = o->corners; out->packed = o->packed;
+    }
 }
 
-static int forward_fp32_tc(vitdet_handle* h, const void* images, int B, float* logits, const vitdet_decode_params* dpar,
-                           const vitdet_detections* det, cudaStream_t st, const ForwardOpts& opts) {
-    const vitdet_config& c = h->cfg;
-    const int mode = VITDET_MODE_FP32;
-    RC_TRY(ensure_workspace(h, B, mode));
-    const Dims m = dims_for(h, mode);
-    const int T = h->T, L = c.repeat_times, q = c.mlp_quantities;
-    const size_t tap_stride = static_cast<size_t>(B) * T * m.D4;
-    if (h->taps_on) { RC_TRY(h->taps.ensure(static_cast<size_t>(L + 1) * tap_stride * 4)); h->taps_B = B; }
-    {
-        const size_t bcmax = static_cast<size_t>(B < h->chunk ? B : h->chunk);
-        size_t need = bcmax * T * round_up(h->PK, 4) * 4;
-        const size_t need_s = static_cast<size_t>(B) * h->S * round_up(T, 8) * 4 + 1024;
-        if (need_s > need) need = need_s;
-        const void* before = h->tmp32.p;
-        RC_TRY(h->tmp32.ensure(need));
-        if (h->tmp32.p != before) h->plans32.clear();
+// One Dense of the forward pass: the tensor-core plan from the cursor (made from `c` on the recording pass), with `out` /
+// `resid` patched because they move with the chunk, or the IEEE CUDA-core GEMM.
+static int dense(vitdet_handle* h, Form f, PlanCursor& pc, int cat, const DenseCall& c, cudaStream_t st) {
+    if (f == Form::Ieee) { ProfScope ps(h, cat, st); return launch_simt(c, st); }
+    if (pc.record) {
+        TcGemmPlan plan;
+        RC_TRY(plan_dense(&plan, c, f, h->num_sms, h->opt.gemm_pair));
+        pc.p->gemm.push_back(plan);
     }
-    std::vector<TcGemmPlan>& cache = h->plans32[(static_cast<long long>(B) << 20) | h->chunk];
-    const bool build = cache.empty();
-    size_t pi = 0;
-    // one Dense: A planes [M, lda] x W planes -> float32 `out` (+ residual / position) or planes `po`
-    auto dense = [&](int cat, Planes A, int lda, const DenseW& w, int M, float* out, int ldc, const Planes* po, int act,
-                     const float* resid, const float* pos) -> int {
-        if (build) {
-            GemmDesc g;
-            g.A = A.hi; g.A_lo = A.lo; g.lda = lda;
-            g.W = w.w16.p; g.W_lo = w.w16_lo(); g.ldw = w.ld16;
-            g.M = M; g.N = w.N; g.K = w.K;
-            g.bias = w.bias.as<float>();
-            g.pos = pos; g.pos_period = T;
-            g.resid = resid; g.ldr = resid ? ldc : 0;
-            g.split = 1; g.precise = 1; g.act = act;
-            if (po) { g.out = po->hi; g.out_lo = po->lo; g.out_split = 1; g.out_f32 = 0; g.ldc = round_up(w.N, 8); }
-            else { g.out = out; g.out_f32 = 1; g.ldc = ldc; }
-            TcGemmPlan plan;
-            int rc = make_tc_plan(&plan, g, h->num_sms, h->opt.gemm_pair);
-            if (rc) return fail(VITDET_E_INVALID, "fp32 tensor-core plan (M=%d N=%d K=%d) failed: %d", g.M, g.N, g.K, rc);
-            cache.push_back(plan);
-        }
-        TcGemmPlan plan = cache[pi++];
-        if (!po) { plan.desc.out = out; plan.desc.resid = resid; }
-        ProfScope ps(h, cat, st);
-        cudaError_t e = plan.pair ? tc2_gemm_launch(plan, st) : tc_gemm_launch(plan, st);
-        if (e != cudaSuccess) return fail(VITDET_E_CUDA, "fp32 tensor-core GEMM launch failed: %s", cudaGetErrorString(e));
-        return 0;
-    };
-    auto split = [&](const float* src, long long rows, int cols, int lds, Planes dst, int ldd) -> int {
-        ++h->launches;
-        split_rows_kernel<<<blocks_for(rows * (ldd >> 3)), 256, 0, st>>>(src, rows, cols, lds, dst.hi, dst.lo, ldd);
-        CU_TRY(cudaGetLastError());
-        return 0;
-    };
-    const Planes p_patch = planes_of(h->patch), p_y = planes_of(h->y), p_u0 = planes_of(h->u0), p_u1 = planes_of(h->u1),
-                 p_qkv = planes_of(h->qkv), p_ctx = planes_of(h->ctx), p_s = planes_of(h->tmp32);
-
-    for (int c0 = 0, bc = 0, ci = 0; c0 < B; c0 += bc, ++ci) {
-        bc = (B - c0) < h->chunk ? (B - c0) : h->chunk;
-        (void)ci;      // no small lead chunks here: the plan cache is keyed by (batch, chunk) only
-        if (opts.ready) CU_TRY(cudaStreamWaitEvent(st, opts.ready[(c0 + bc + opts.ready_gran - 1) / opts.ready_gran - 1], 0));
-        const int Mc = bc * T;
-        float* x = h->x.as<float>() + static_cast<size_t>(c0) * T * m.D4;
-        const char* img = static_cast<const char*>(images) + static_cast<size_t>(c0) * c.image_h * c.image_w * 3 * (opts.in_u8 ? 1 : 4);
-        const int P4 = round_up(h->PK, 4);
-        float* tmp_big = h->tmp32.as<float>();          // [Mc, P4] float32 patches before the split
-        { ProfScope ps(h, PC_PATCHIFY, st);
-        CU_TRY(patchify_launch(img, opts.in_u8, bc, c.image_h, c.image_w, c.patch_size, tmp_big, P4, h->RP, 1, st)); }
-        RC_TRY(split(tmp_big, Mc, h->PK, P4, p_patch, m.Pld));
-        RC_TRY(dense(PC_PROJ, p_patch, m.Pld, h->proj, Mc, x, m.D4, nullptr, ACT_NONE, nullptr, h->pos.as<float>()));
-        if (h->taps_on) CU_TRY(cudaMemcpyAsync(h->taps.as<float>() + static_cast<size_t>(c0) * T * m.D4, x, static_cast<size_t>(Mc) * m.D4 * 4, cudaMemcpyDeviceToDevice, st));
-        float* tmp_ln = h->tmp32.as<float>();           // [Mc, D4] LayerNorm output before the split
-        for (int i = 0; i < L; ++i) {
-            BlockW& b = h->blocks[i];
-            { ProfScope ps(h, PC_LN, st);
-            CU_TRY(layernorm_launch(x, m.D4, b.ln1_g.as<float>(), b.ln1_b.as<float>(), Mc, h->D, c.ln_epsilon, tmp_ln, m.D4, 1, st)); }
-            RC_TRY(split(tmp_ln, Mc, h->D, m.D4, p_y, m.D8));
-            // q | k | v and the context rows stay in the split form end to end: QKV GEMM -> planes -> attention -> planes
-            RC_TRY(dense(PC_QKV, p_y, m.D8, b.qkv, Mc, nullptr, 0, &p_qkv, ACT_NONE, nullptr, nullptr));
-            {
-                AttnDesc ad;
-                ad.qkv = p_qkv.hi; ad.ldq = m.w_qkv; ad.ctx = p_ctx.hi; ad.ldo = m.w_ctx;
-                ad.B = bc; ad.T = T; ad.H = h->H; ad.d = h->d; ad.hp = h->hp;
-                ad.scale = 1.f / sqrtf(static_cast<float>(h->d));
-                AttnPlan ap;
-                CUtensorMap tm_lo;
-                int rc = attn_bf16_make_plan(&ap, ad);
-                if (!rc) rc = make_tmap_bf16_2d(&tm_lo, p_qkv.lo, bc * T, 3 * h->H * h->hp, m.w_qkv, 64);
-                if (rc) return fail(VITDET_E_INVALID, "fp32 tensor-core attention plan failed: %d", rc);
-                ProfScope ps(h, PC_ATTN, st);
-                CU_TRY(attn_tcs_launch(ap, tm_lo, p_ctx.lo, st));
-            }
-            RC_TRY(dense(PC_OUT, p_ctx, m.w_ctx, b.out, Mc, x, m.D4, nullptr, ACT_NONE, x, nullptr));
-            { ProfScope ps(h, PC_LN, st);
-            CU_TRY(layernorm_launch(x, m.D4, b.ln2_g.as<float>(), b.ln2_b.as<float>(), Mc, h->D, c.ln_epsilon, tmp_ln, m.D4, 1, st)); }
-            RC_TRY(split(tmp_ln, Mc, h->D, m.D4, p_y, m.D8));
-            Planes a = p_y; int lda = m.D8;
-            for (int j = 0; j < q; ++j) {
-                const bool last = j == q - 1;
-                if (last) {
-                    RC_TRY(dense(PC_MLP0 + j, a, lda, b.mlp[j], Mc, x, m.D4, nullptr, h->act, x, nullptr));
-                } else {
-                    const Planes o = (j & 1) ? p_u1 : p_u0;
-                    RC_TRY(dense(PC_MLP0 + j, a, lda, b.mlp[j], Mc, nullptr, 0, &o, h->act, nullptr, nullptr));
-                    a = o; lda = round_up(b.mlp[j].N, 8);
-                }
-            }
-            if (h->taps_on) CU_TRY(cudaMemcpyAsync(h->taps.as<float>() + (i + 1) * tap_stride + static_cast<size_t>(c0) * T * m.D4, x, static_cast<size_t>(Mc) * m.D4 * 4, cudaMemcpyDeviceToDevice, st));
-        }
-    }
-
-    // mlp_head over the whole batch (det.py:454-493)
-    const int R = B * h->S;
-    { ProfScope ps(h, PC_HEAD_SLOTS, st);
-    CU_TRY(head_slots_launch(h->x.as<float>(), m.D4, h->head_slot_w.as<float>(), h->head_slot_b.as<float>(), B * T, h->D, h->S, T, m.Tp,
-                             h->s.p, 1, st)); }
-    const int T8 = round_up(T, 8);
-    RC_TRY(split(h->s.as<float>(), R, T, m.Tp, p_s, T8));
-    Planes a = p_s; int lda = T8;
-    const float* last_out = nullptr; int last_ld = 0;
-    for (size_t i = 0; i < h->head.size(); ++i) {
-        const bool last = i + 1 == h->head.size();
-        DevBuf& ob = (i & 1) ? h->h1 : h->h0;
-        if (last) {
-            last_ld = round_up(h->head[i].N, 4);
-            RC_TRY(dense(PC_HEAD_GEMM, a, lda, h->head[i], R, ob.as<float>(), last_ld, nullptr, h->act, nullptr, nullptr));
-            last_out = ob.as<float>();
-        } else {
-            const Planes o = planes_of(ob);
-            RC_TRY(dense(PC_HEAD_GEMM, a, lda, h->head[i], R, nullptr, 0, &o, h->act, nullptr, nullptr));
-            a = o; lda = round_up(h->head[i].N, 8);
-        }
-    }
-    DecodeParams dp;
-    DecodeOut dout;
-    dout.logits = logits;
-    if (dpar) {
-        dp.obj_thr = dpar->objectness_threshold; dp.cls_thr = dpar->classification_threshold;
-        dp.strict = dpar->strict; dp.img_h = dpar->image_h; dp.img_w = dpar->image_w; dp.classes = dpar->classes;
-        dp.apply_transform = 1;
-        dp.corner_scale = dpar->corner_scale > 0.f ? dpar->corner_scale : 1.f;
-    }
-    if (det) {
-        dout.decoded = det->decoded; dout.class_id = det->class_id; dout.class_conf = det->class_conf;
-        dout.keep = det->keep; dout.corners = det->corners; dout.packed = det->packed;
-    }
-    h->head_last = last_out; h->head_last_ld = last_ld; h->head_last_f32 = 1;
-    ProfScope ps(h, PC_HEAD_TAIL, st);
-    CU_TRY(head_tail_launch(last_out, last_ld, 1, h->tail_w.as<float>(), h->tail_b.as<float>(), R, h->tail_U, dp, dout, st));
-    return 0;
+    ProfScope ps(h, cat, st);
+    return launch_tc(pc.p->gemm[pc.gemm++], c.out.p, c.resid, st);
 }
 
 static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, float* logits,
@@ -1042,13 +884,21 @@ static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, f
         if (!s.set) return fail(VITDET_E_UNSET, "forward: weight '%s' has not been set", s.name.c_str());
     if (h->weights_dirty) { CU_TRY(cudaDeviceSynchronize()); h->weights_dirty = false; }
     const vitdet_config& c = h->cfg;
-    const bool bf = mode == VITDET_MODE_BF16;
-    // fp32-accumulate mode on the tensor cores; heads wider than 64 take the IEEE CUDA-core form (the split attention kernel holds hi and lo tiles)
-    if (!bf && h->opt.fp32_tc && h->d <= kMaxKeyDimSplit) return forward_fp32_tc(h, images, B, logits, dpar, det, st, opts);
-    RC_TRY(ensure_workspace(h, B, mode));
-    const Dims m = dims_for(h, mode);
+    const Form f = pick_form(mode, h->opt, h->d);
+    RC_TRY(ensure_workspace(h, B, f));
+    const Dims m = dims_for(h, f);
     const int T = h->T, L = c.repeat_times, q = c.mlp_quantities;
-    const int out_f32_act = bf ? 0 : 1;
+    // Bf16 with D <= 32: every LayerNorm runs in the epilogue of the GEMM that produces the residual-stream row (projection
+    // -> LN1 of block 0; attention output -> LN2; last MLP layer -> LN1 of the next block), and the last three MLP layers
+    // of a block run as one kernel when their widths fit it (default model: 224 -> 112 -> 56 -> 28)
+    const bool fuse_ln = f == Form::Bf16 && ln_is_fused(h);
+    bool fuse_tail = false;
+    if (fuse_ln && tail_fusion_enabled(h) && q >= 4) {
+        const BlockW& b = h->blocks[0];
+        const int N3[3] = {b.mlp[q - 3].N, b.mlp[q - 2].N, b.mlp[q - 1].N};
+        const int K3[3] = {b.mlp[q - 3].K, b.mlp[q - 2].K, b.mlp[q - 1].K};
+        fuse_tail = mlp_tail_supported(N3, K3);
+    }
     const size_t tap_stride = static_cast<size_t>(B) * T * m.D4;      // floats per tap
     if (h->taps_on) { RC_TRY(h->taps.ensure(static_cast<size_t>(L + 1) * tap_stride * 4)); h->taps_B = B; }
     auto tap = [&](int index, const float* xc, int c0, int bc) -> int {
@@ -1057,6 +907,47 @@ static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, f
                                static_cast<size_t>(bc) * T * m.D4 * 4, cudaMemcpyDeviceToDevice, st));
         return 0;
     };
+    // Rows of `cols` values that patchify / LayerNorm / the slot projection write for the next GEMM: into `buf` as bf16
+    // (Bf16) or f32 (Ieee) rows, or (Split) f32 rows at `stage` that operand() splits into the planes of `buf`.
+    struct Rows { void* p; int ld; int f32; };
+    auto rows_out = [&](const DevBuf& buf, const DevBuf& stage, int cols) -> Rows {
+        if (f == Form::Bf16) return Rows{buf.p, round_up(cols, 8), 0};
+        return Rows{f == Form::Split ? stage.p : buf.p, round_up(cols, 4), 1};
+    };
+    // `buf` as rows of pitch ld in the form's operand layout (Split: its planes)
+    auto act_in = [&](const DevBuf& buf, int ld) -> Operand {
+        if (f != Form::Split) return Operand{buf.p, nullptr, ld};
+        const Planes pl = planes_of(buf);
+        return Operand{pl.hi, pl.lo, ld};
+    };
+    auto operand = [&](const Rows& r, const DevBuf& buf, long long rows, int cols, Operand* a) -> int {
+        if (f != Form::Split) { *a = Operand{r.p, nullptr, r.ld}; return 0; }
+        *a = act_in(buf, round_up(cols, 8));
+        ++h->launches;
+        split_rows_kernel<<<blocks_for(rows * (a->ld >> 3)), 256, 0, st>>>(static_cast<const float*>(r.p), rows, cols, r.ld,
+                                                                         static_cast<__nv_bfloat16*>(a->p), static_cast<__nv_bfloat16*>(a->lo), a->ld);
+        CU_TRY(cudaGetLastError());
+        return 0;
+    };
+    auto layernorm = [&](const float* x, const DevBuf& gamma, const DevBuf& beta, int Mc, Operand* a) -> int {
+        const Rows r = rows_out(h->y, h->tmp32, h->D);
+        { ProfScope ps(h, PC_LN, st);
+        CU_TRY(layernorm_launch(x, m.D4, gamma.as<float>(), beta.as<float>(), Mc, h->D, c.ln_epsilon, r.p, r.ld, r.f32, st)); }
+        return operand(r, h->y, Mc, h->D, a);
+    };
+    // Output of a Dense that feeds another GEMM or the attention core: rows of `buf` in the form's operand layout
+    auto to_act = [&](DenseCall& dc, const DevBuf& buf) {
+        dc.out_f32 = f == Form::Ieee;
+        dc.out = act_in(buf, round_up(dc.w->N, dc.out_f32 ? 4 : 8));
+    };
+    // Output into float32 rows [M, ld] (the residual stream, plus itself as the residual when `add`)
+    auto to_f32 = [&](DenseCall& dc, float* o, int ld, bool add) {
+        dc.out = Operand{o, nullptr, ld}; dc.out_f32 = 1;
+        if (add) { dc.resid = o; dc.ldr = ld; }
+    };
+    auto with_ln = [&](DenseCall& dc, const DevBuf& gamma, const DevBuf& beta) {
+        if (fuse_ln) { dc.ln_gamma = gamma.as<float>(); dc.ln_beta = beta.as<float>(); dc.ln_out = h->y.p; dc.ln_ld = m.D8; dc.ln_eps = c.ln_epsilon; }
+    };
 
     for (int c0 = 0, bc = 0, ci = 0; c0 < B; c0 += bc, ++ci) {
         bc = (B - c0) < h->chunk ? (B - c0) : h->chunk;
@@ -1064,111 +955,111 @@ static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, f
         if (opts.ready) CU_TRY(cudaStreamWaitEvent(st, opts.ready[(c0 + bc + opts.ready_gran - 1) / opts.ready_gran - 1], 0));
         const int Mc = bc * T;
         float* x = h->x.as<float>() + static_cast<size_t>(c0) * T * m.D4;
-        vitdet_handle::EncPlans* ep = nullptr;
-        if (bf) {
-            ep = &h->enc_plans[bc];
-            if (!ep->valid) RC_TRY(build_enc_plans(h, bc, ep));
-        }
+        PlanCursor pc = plan_cursor(h, kEncoderPlans, f, bc);
         const char* img = static_cast<const char*>(images) + static_cast<size_t>(c0) * c.image_h * c.image_w * 3 * (opts.in_u8 ? 1 : 4);
+        const Rows pr = rows_out(h->patch, h->tmp32, h->PK);
         { ProfScope ps(h, PC_PATCHIFY, st);
-        CU_TRY(patchify_launch(img, opts.in_u8, bc, c.image_h, c.image_w, c.patch_size, h->patch.p, bf ? m.Pld : round_up(h->PK, 4), h->RP, out_f32_act, st)); }
-        if (bf) {
-            ProfScope ps(h, PC_PROJ, st);
-            RC_TRY(launch_tc(ep->proj, x, nullptr, st));
-        } else {
-            ProfScope ps(h, PC_PROJ, st);
-            DenseCall pc{h->patch.p, round_up(h->PK, 4), &h->proj, h->pos.as<float>(), T, nullptr, 0, x, m.D4, 1, ACT_NONE, Mc};
-            RC_TRY(launch_simt(pc, st));
-        }
+        CU_TRY(patchify_launch(img, opts.in_u8, bc, c.image_h, c.image_w, c.patch_size, pr.p, pr.ld, h->RP, pr.f32, st)); }
+        Operand a;
+        RC_TRY(operand(pr, h->patch, Mc, h->PK, &a));
+        DenseCall pj{a, &h->proj, Mc};
+        pj.pos = h->pos.as<float>(); pj.pos_period = T;
+        to_f32(pj, x, m.D4, false);
+        with_ln(pj, h->blocks[0].ln1_g, h->blocks[0].ln1_b);
+        RC_TRY(dense(h, f, pc, PC_PROJ, pj, st));
         RC_TRY(tap(0, x, c0, bc));
+        const Operand y_fused{h->y.p, nullptr, m.D8};      // LayerNorm output of a fused epilogue
         for (int i = 0; i < L; ++i) {
             BlockW& b = h->blocks[i];
-            const int ldy = bf ? m.D8 : m.D4;
-            if (!(bf && ln_is_fused(h))) { ProfScope ps(h, PC_LN, st);
-            CU_TRY(layernorm_launch(x, m.D4, b.ln1_g.as<float>(), b.ln1_b.as<float>(), Mc, h->D, c.ln_epsilon, h->y.p, ldy, out_f32_act, st)); }
-            if (bf) {
-                { ProfScope ps(h, PC_QKV, st); RC_TRY(launch_tc(ep->qkv[i], h->qkv.p, nullptr, st)); }
-                { ProfScope ps(h, PC_ATTN, st); CU_TRY(attn_launch(h->opt.attention, ep->attn[i], h->num_sms, st)); }
-                { ProfScope ps(h, PC_OUT, st); RC_TRY(launch_tc(ep->out[i], x, x, st)); }
-            } else {
-                DenseCall qc{h->y.p, ldy, &b.qkv, nullptr, 1, nullptr, 0, h->qkv.p, m.w_qkv, 1, ACT_NONE, Mc};
-                { ProfScope ps(h, PC_QKV, st); RC_TRY(launch_simt(qc, st)); }
-                AttnDesc ad;
-                ad.qkv = h->qkv.p; ad.ldq = m.w_qkv; ad.ctx = h->ctx.p; ad.ldo = m.w_ctx;
-                ad.B = bc; ad.T = T; ad.H = h->H; ad.d = h->d; ad.hp = h->hp;
-                ad.scale = 1.f / sqrtf(static_cast<float>(h->d));
-                { ProfScope ps(h, PC_ATTN, st); CU_TRY(attn_f32_launch(ad, st)); }
-                DenseCall oc{h->ctx.p, m.w_ctx, &b.out, nullptr, 1, x, m.D4, x, m.D4, 1, ACT_NONE, Mc};
-                { ProfScope ps(h, PC_OUT, st); RC_TRY(launch_simt(oc, st)); }
+            a = y_fused;
+            if (!fuse_ln) RC_TRY(layernorm(x, b.ln1_g, b.ln1_b, Mc, &a));
+            DenseCall qc{a, &b.qkv, Mc};
+            to_act(qc, h->qkv);
+            RC_TRY(dense(h, f, pc, PC_QKV, qc, st));
+            DenseCall oc{act_in(h->ctx, m.w_ctx), &b.out, Mc};      // the attention output is attention_output's A operand
+            const AttnDesc ad = attn_desc(qc.out, oc.A, bc, T, h->H, h->d, h->hp);
+            if (f != Form::Ieee && pc.record) {
+                AttnTcPlan ap;
+                RC_TRY(attn_plan(&ap, ad, qc.out.lo));
+                pc.p->attn.push_back(ap);
             }
-            if (!(bf && ln_is_fused(h))) { ProfScope ps(h, PC_LN, st);
-            CU_TRY(layernorm_launch(x, m.D4, b.ln2_g.as<float>(), b.ln2_b.as<float>(), Mc, h->D, c.ln_epsilon, h->y.p, ldy, out_f32_act, st)); }
-            const void* a = h->y.p; int lda = ldy;
+            { ProfScope ps(h, PC_ATTN, st);
+            CU_TRY(attn_launch(f, ad, f == Form::Ieee ? nullptr : &pc.p->attn[pc.attn++], oc.A.lo, st)); }
+            to_f32(oc, x, m.D4, true);
+            with_ln(oc, b.ln2_g, b.ln2_b);
+            RC_TRY(dense(h, f, pc, PC_OUT, oc, st));
+            a = y_fused;
+            if (!fuse_ln) RC_TRY(layernorm(x, b.ln2_g, b.ln2_b, Mc, &a));
             for (int j = 0; j < q; ++j) {
-                const bool last = j == q - 1;
-                void* o = last ? static_cast<void*>(x) : ((j & 1) ? h->u1.p : h->u0.p);
-                ProfScope ps(h, PC_MLP0 + j, st);
-                if (bf && ep->tail_fused && j == q - 3) {
-                    MlpTailPlan tp = ep->tail[i];       // by value: the residual-stream pointer is patched per chunk
+                if (fuse_tail && j == q - 3) {
+                    if (pc.record) {
+                        MlpTailDesc td;
+                        td.A = a.p; td.lda = a.ld; td.M = Mc;
+                        for (int l = 0; l < 3; ++l) {
+                            DenseW& w = b.mlp[q - 3 + l];
+                            td.N[l] = w.N; td.K[l] = w.K; td.W[l] = w.w16.p; td.ldw[l] = w.ld16; td.bias[l] = w.bias.as<float>();
+                        }
+                        td.x = x; td.ldx = m.D4; td.act = h->act;
+                        if (i + 1 < L) {
+                            td.ln_gamma = h->blocks[i + 1].ln1_g.as<float>(); td.ln_beta = h->blocks[i + 1].ln1_b.as<float>();
+                            td.ln_eps = c.ln_epsilon; td.ln_out = h->y.p; td.ln_ld = m.D8;
+                        }
+                        MlpTailPlan tp;
+                        const int rc = mlp_tail_make_plan(&tp, td, h->num_sms);
+                        if (rc) return fail(VITDET_E_INVALID, "mlp_tail_make_plan failed: %d", rc);
+                        tp.valid = true;
+                        pc.p->tail.push_back(tp);
+                    }
+                    MlpTailPlan tp = pc.p->tail[pc.tail++];       // by value: the residual-stream pointer is patched per chunk
                     tp.desc.x = x;
-                    cudaError_t te = mlp_tail_launch(tp, st);
+                    ProfScope ps(h, PC_MLP0 + j, st);
+                    const cudaError_t te = mlp_tail_launch(tp, st);
                     if (te != cudaSuccess) return fail(VITDET_E_CUDA, "mlp_tail_launch failed: %s", cudaGetErrorString(te));
                     break;
                 }
-                if (bf) {
-                    RC_TRY(launch_tc(ep->mlp[i][j], o, last ? x : nullptr, st));
+                DenseCall mc{a, &b.mlp[j], Mc};
+                mc.act = h->act;
+                if (j == q - 1) {
+                    to_f32(mc, x, m.D4, true);
+                    if (i + 1 < L) with_ln(mc, h->blocks[i + 1].ln1_g, h->blocks[i + 1].ln1_b);
                 } else {
-                    const int ldo = last ? m.D4 : round_up(b.mlp[j].N, 4);
-                    DenseCall mc{a, lda, &b.mlp[j], nullptr, 1, last ? x : nullptr, last ? m.D4 : 0, o, ldo, 1, h->act, Mc};
-                    RC_TRY(launch_simt(mc, st));
-                    a = o; lda = ldo;
+                    to_act(mc, (j & 1) ? h->u1 : h->u0);
                 }
+                RC_TRY(dense(h, f, pc, PC_MLP0 + j, mc, st));
+                a = mc.out;
             }
             RC_TRY(tap(i + 1, x, c0, bc));
         }
+        pc.p->complete = true;
     }
 
-    // mlp_head over the whole batch (det.py:454-493).
+    // mlp_head over the whole batch (det.py:454-493)
     const int R = B * h->S;
+    PlanCursor pc = plan_cursor(h, kHeadPlans, f, B);
+    const Rows sr{h->s.p, m.Tp, f != Form::Bf16};        // the Split form splits the slot matrix into tmp32's planes
     { ProfScope ps(h, PC_HEAD_SLOTS, st);
     CU_TRY(head_slots_launch(h->x.as<float>(), m.D4, h->head_slot_w.as<float>(), h->head_slot_b.as<float>(), B * T, h->D, h->S,
-                             T, m.Tp, h->s.p, out_f32_act, st)); }
-    const void* a = h->s.p; int lda = m.Tp;
-    if (bf) {
-        vitdet_handle::HeadPlans* hp = &h->head_plans[B];
-        if (!hp->valid) RC_TRY(build_head_plans(h, B, hp));
-        for (size_t i = 0; i < h->head.size(); ++i) {
-            void* o = (i & 1) ? h->h1.p : h->h0.p;
-            ProfScope ps(h, PC_HEAD_GEMM, st);
-            RC_TRY(launch_tc(hp->dense[i], o, nullptr, st));
-            a = o; lda = round_up(h->head[i].N, 8);
-        }
-    } else {
-        for (size_t i = 0; i < h->head.size(); ++i) {
-            void* o = (i & 1) ? h->h1.p : h->h0.p;
-            const int ldo = round_up(h->head[i].N, 4);
-            DenseCall hc{a, lda, &h->head[i], nullptr, 1, nullptr, 0, o, ldo, 1, h->act, R};
-            ProfScope ps(h, PC_HEAD_GEMM, st);
-            RC_TRY(launch_simt(hc, st));
-            a = o; lda = ldo;
-        }
+                             T, sr.ld, sr.p, sr.f32, st)); }
+    Operand a;
+    RC_TRY(operand(sr, h->tmp32, R, T, &a));
+    for (size_t i = 0; i < h->head.size(); ++i) {
+        DenseCall hc{a, &h->head[i], R};
+        hc.act = h->act;
+        DevBuf& ob = (i & 1) ? h->h1 : h->h0;
+        // the final Dense(6) reads float32 rows in the Split form
+        if (f == Form::Split && i + 1 == h->head.size()) to_f32(hc, ob.as<float>(), round_up(h->head[i].N, 4), false);
+        else to_act(hc, ob);
+        RC_TRY(dense(h, f, pc, PC_HEAD_GEMM, hc, st));
+        a = hc.out;
     }
+    pc.p->complete = true;
     DecodeParams dp;
     DecodeOut dout;
-    dout.logits = logits;
-    if (dpar) {
-        dp.obj_thr = dpar->objectness_threshold; dp.cls_thr = dpar->classification_threshold;
-        dp.strict = dpar->strict; dp.img_h = dpar->image_h; dp.img_w = dpar->image_w; dp.classes = dpar->classes;
-        dp.apply_transform = 1;   // the head emits raw logits
-        dp.corner_scale = dpar->corner_scale > 0.f ? dpar->corner_scale : 1.f;
-    }
-    if (det) {
-        dout.decoded = det->decoded; dout.class_id = det->class_id; dout.class_conf = det->class_conf;
-        dout.keep = det->keep; dout.corners = det->corners; dout.packed = det->packed;
-    }
-    h->head_last = a; h->head_last_ld = lda; h->head_last_f32 = out_f32_act;
+    decode_args(dpar, 1 /*the head emits raw logits*/, det, logits, &dp, &dout);
+    const int in_f32 = f != Form::Bf16;
+    h->head_last = a.p; h->head_last_ld = a.ld; h->head_last_f32 = in_f32;
     ProfScope ps(h, PC_HEAD_TAIL, st);
-    CU_TRY(head_tail_launch(a, lda, out_f32_act, h->tail_w.as<float>(), h->tail_b.as<float>(), R, h->tail_U, dp, dout, st));
+    CU_TRY(head_tail_launch(a.p, a.ld, in_f32, h->tail_w.as<float>(), h->tail_b.as<float>(), R, h->tail_U, dp, dout, st));
     return 0;
 }
 
@@ -1350,18 +1241,8 @@ int vitdet_set_option(vitdet_handle* h, const char* key, int value) {
     else if (k == "fuse_tail") h->opt.fuse_tail = value != 0;
     else if (k == "gemm_pair") { if (value < 0 || value > 2) return fail(VITDET_E_INVALID, "set_option(gemm_pair): 0, 1 or 2"); h->opt.gemm_pair = value; }
     else if (k == "fp32_tc") h->opt.fp32_tc = value != 0;
-    else if (k == "attention") {
-#ifdef VITDET_EXPERIMENTS
-        if (value != 1 && value != 2 && value != 3 && value != 4 && value != 8 && value != 40 && value != 80) return fail(VITDET_E_INVALID, "set_option(attention): 1, 2, 3, 4, 8, 40 or 80");
-#else
-        if (value != 4) return fail(VITDET_E_INVALID, "set_option(attention): this build only holds the product kernel (4); VITDET_BUILD_EXPERIMENTS=1 adds the others");
-#endif
-        h->opt.attention = value;
-    }
     else return fail(VITDET_E_NOT_FOUND, "set_option: unknown option '%s'", key);
-    h->enc_plans.clear();
-    h->head_plans.clear();
-    h->plans32.clear();
+    h->plans.clear();
     return 0;
 }
 
@@ -1371,7 +1252,6 @@ int vitdet_get_option(const vitdet_handle* h, const char* key, int* value) {
     if (k == "fuse_ln") *value = h->opt.fuse_ln;
     else if (k == "fuse_tail") *value = h->opt.fuse_tail;
     else if (k == "gemm_pair") *value = h->opt.gemm_pair;
-    else if (k == "attention") *value = h->opt.attention;
     else if (k == "fp32_tc") *value = h->opt.fp32_tc;
     else return fail(VITDET_E_NOT_FOUND, "get_option: unknown option '%s'", key);
     return 0;
@@ -1425,7 +1305,7 @@ int vitdet_set_chunk(vitdet_handle* h, int n) {
 
 size_t vitdet_workspace_bytes(const vitdet_handle* h, int B, int mode) {
     if (!h || B <= 0) return 0;
-    return workspace_bytes(h, B, mode);
+    return workspace_bytes(h, B, pick_form(mode, h->opt, h->d));
 }
 
 int vitdet_forward(vitdet_handle* h, const float* images_dev, int B, float* logits_dev, int mode, void* stream) {
@@ -1452,13 +1332,8 @@ int vitdet_decode(const float* logits_dev, int R, const vitdet_decode_params* p,
     if (!logits_dev || !p || !out || R < 0) return fail(VITDET_E_INVALID, "decode: bad arguments");
     if (R == 0) return 0;
     DecodeParams dp;
-    dp.obj_thr = p->objectness_threshold; dp.cls_thr = p->classification_threshold; dp.strict = p->strict;
-    dp.img_h = p->image_h; dp.img_w = p->image_w; dp.classes = p->classes;
-    dp.apply_transform = p->use_transform_predictions ? 1 : 0;
-    dp.corner_scale = p->corner_scale > 0.f ? p->corner_scale : 1.f;
     DecodeOut o;
-    o.decoded = out->decoded; o.class_id = out->class_id; o.class_conf = out->class_conf; o.keep = out->keep; o.corners = out->corners;
-    o.packed = out->packed;
+    decode_args(p, p->use_transform_predictions ? 1 : 0, out, nullptr, &dp, &o);
     CU_TRY(decode_launch(logits_dev, R, dp, o, static_cast<cudaStream_t>(stream)));
     return 0;
 }
@@ -1577,6 +1452,9 @@ static int submit_host_impl(vitdet_handle* h, const void* images_host, int in_u8
     if (in_u8) { kGran = 16; lead0 = 16; lead1 = 0; }       // a quarter of the bytes per image: same 0.3 ms lead-in with 16 images
     // with the previous submission still computing, this one's copy has a whole forward pass to finish: no small lead chunks
     if (h->host_slots[(h->next_slot + vitdet_handle::kHostSlots - 1) % vitdet_handle::kHostSlots].busy) { lead0 = 0; lead1 = 0; }
+    // nor in the split fp32 form: its three-pass GEMMs lose more on 4- and 12-image chunks than the early start gains
+    // (B = 64 on a B200 at 1000 W: 48.5 ms with lead chunks 4, 12 against 45.1 ms without)
+    if (pick_form(mode, h->opt, h->d) == Form::Split) { lead0 = 0; lead1 = 0; }
     if (const char* e = getenv("VITDET_E2E_LEAD")) sscanf(e, "%d,%d,%d", &kGran, &lead0, &lead1);
     if (kGran < 1) kGran = 8;
     const int n_sub = (B + kGran - 1) / kGran;
@@ -1711,43 +1589,31 @@ int vitdet_op_dense(const float* A, const float* kernel, const float* bias, cons
         pad_rows_f32_kernel<<<blocks_for(static_cast<long long>(M) * N4), 256, 0, st>>>(resid, M, N, N, r_buf.as<float>(), N4);
         rp = r_buf.as<float>();
     }
-    int rc = 0;
-    if (mode == VITDET_MODE_BF16) {
-        const int K8 = round_up(K, 8);
-        RC_TRY(a_buf.ensure(static_cast<size_t>(M) * K8 * 2));
-        f32_to_bf16_kernel<<<blocks_for(static_cast<long long>(M) * K8), 256, 0, st>>>(A, M, K, K, a_buf.as<__nv_bfloat16>(), K8);
-        DenseCall c{a_buf.p, K8, &w, nullptr, 1, rp, N4, o_buf.p, N4, 1, act, M};
-        TcGemmPlan plan;
-        GemmDesc g = make_desc(c, VITDET_MODE_BF16);
-        rc = make_tc_plan(&plan, g, sms, env_options().gemm_pair);
-        if (rc) return fail(VITDET_E_INVALID, "op_dense: tc_gemm_make_plan failed: %d", rc);
-        RC_TRY(launch_tc(plan, o_buf.p, rp, st));
-    } else if (env_options().fp32_tc) {
-        // fp32-accumulate mode on the tensor cores: split (hi, lo) bf16 planes, three passes, exact activation
-        const int K8 = round_up(K, 8);
-        RC_TRY(a_buf.ensure(static_cast<size_t>(M) * K8 * 2 * 2));
-        __nv_bfloat16* a_hi = a_buf.as<__nv_bfloat16>();
-        __nv_bfloat16* a_lo = a_hi + static_cast<size_t>(M) * K8;
-        split_rows_kernel<<<blocks_for(static_cast<long long>(M) * (K8 >> 3)), 256, 0, st>>>(A, M, K, K, a_hi, a_lo, K8);
-        GemmDesc g;
-        g.A = a_hi; g.A_lo = a_lo; g.lda = K8;
-        g.W = w.w16.p; g.W_lo = w.w16_lo(); g.ldw = w.ld16;
-        g.M = M; g.N = N; g.K = K;
-        g.bias = w.bias.as<float>();
-        g.resid = rp; g.ldr = N4;
-        g.out = o_buf.p; g.ldc = N4; g.out_f32 = 1; g.act = act;
-        g.split = 1; g.precise = 1;
-        TcGemmPlan plan;
-        rc = make_tc_plan(&plan, g, sms, env_options().gemm_pair);
-        if (rc) return fail(VITDET_E_INVALID, "op_dense: fp32 tensor-core plan failed: %d", rc);
-        RC_TRY(launch_tc(plan, o_buf.p, rp, st));
+    // A in the form's operand layout: bf16 rows, (hi, lo) planes, or f32 rows
+    const Form f = pick_form(mode, env_options(), 0 /*no attention*/);
+    Operand a;
+    if (f == Form::Ieee) {
+        a = Operand{nullptr, nullptr, round_up(K, 4)};
+        RC_TRY(a_buf.ensure(static_cast<size_t>(M) * a.ld * 4));
+        a.p = a_buf.p;
+        pad_rows_f32_kernel<<<blocks_for(static_cast<long long>(M) * a.ld), 256, 0, st>>>(A, M, K, K, a_buf.as<float>(), a.ld);
     } else {
-        const int K4 = round_up(K, 4);
-        RC_TRY(a_buf.ensure(static_cast<size_t>(M) * K4 * 4));
-        pad_rows_f32_kernel<<<blocks_for(static_cast<long long>(M) * K4), 256, 0, st>>>(A, M, K, K, a_buf.as<float>(), K4);
-        DenseCall c{a_buf.p, K4, &w, nullptr, 1, rp, N4, o_buf.p, N4, 1, act, M};
-        RC_TRY(launch_simt(c, st));
+        a = Operand{nullptr, nullptr, round_up(K, 8)};
+        const size_t plane = static_cast<size_t>(M) * a.ld;
+        RC_TRY(a_buf.ensure(plane * 2 * (f == Form::Split ? 2 : 1)));
+        a.p = a_buf.p;
+        if (f == Form::Bf16) {
+            f32_to_bf16_kernel<<<blocks_for(static_cast<long long>(plane)), 256, 0, st>>>(A, M, K, K, a_buf.as<__nv_bfloat16>(), a.ld);
+        } else {
+            a.lo = a_buf.as<__nv_bfloat16>() + plane;
+            split_rows_kernel<<<blocks_for(static_cast<long long>(M) * (a.ld >> 3)), 256, 0, st>>>(A, M, K, K, a_buf.as<__nv_bfloat16>(),
+                                                                                                 static_cast<__nv_bfloat16*>(a.lo), a.ld);
+        }
     }
+    DenseCall c{a, &w, M};
+    c.resid = rp; c.ldr = N4;
+    c.out = Operand{o_buf.p, nullptr, N4}; c.out_f32 = 1; c.act = act;
+    RC_TRY(dense_once(c, f, sms, env_options().gemm_pair, st));
     unpad_rows_f32_kernel<<<blocks_for(static_cast<long long>(M) * N), 256, 0, st>>>(o_buf.as<float>(), M, N, N4, out);
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaStreamSynchronize(st));
@@ -1780,49 +1646,31 @@ int vitdet_op_attention(const float* q, const float* k, const float* v, float* o
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     const int hp = head_pitch(d);
     const long long rows = static_cast<long long>(B) * T;
-    const int es = mode == VITDET_MODE_BF16 ? 2 : 4;
-    DevBuf qkv, ctx;
-    RC_TRY(qkv.ensure(static_cast<size_t>(rows) * 3 * H * hp * es));
+    const Form f = pick_form(mode, env_options(), d);
+    const int ld = 3 * H * hp;
+    // q | k | v as bf16 or f32 rows; the Split form's (hi, lo) planes of them in `planes`, of the context rows in `ctx`
+    DevBuf qkv, ctx, planes;
+    const size_t es = f == Form::Bf16 ? 2 : 4;
+    RC_TRY(qkv.ensure(static_cast<size_t>(rows) * ld * es));
     RC_TRY(ctx.ensure(static_cast<size_t>(rows) * H * hp * es));
-    AttnDesc ad;
-    ad.qkv = qkv.p; ad.ldq = 3 * H * hp; ad.ctx = ctx.p; ad.ldo = H * hp;
-    ad.B = B; ad.T = T; ad.H = H; ad.d = d; ad.hp = hp; ad.scale = 1.f / sqrtf(static_cast<float>(d));
-    if (mode == VITDET_MODE_BF16) {
-        pack_qkv_kernel<__nv_bfloat16><<<blocks_for(rows * 3 * H * hp), 256, 0, st>>>(q, k, v, rows, H, d, hp, qkv.as<__nv_bfloat16>());
-        AttnPlan plan;
-        int rc = attn_bf16_make_plan(&plan, ad);
-        if (rc) return fail(VITDET_E_INVALID, "op_attention: attn_bf16_make_plan failed: %d", rc);
-        { int dev2 = 0, sms2 = 148; CU_TRY(cudaGetDevice(&dev2)); CU_TRY(cudaDeviceGetAttribute(&sms2, cudaDevAttrMultiProcessorCount, dev2));
-          CU_TRY(attn_launch(env_options().attention, plan, sms2, st)); }
-        unpack_ctx_kernel<__nv_bfloat16><<<blocks_for(rows * H * d), 256, 0, st>>>(ctx.as<__nv_bfloat16>(), rows, H, d, hp, out);
-    } else if (env_options().fp32_tc && d <= kMaxKeyDimSplit) {
-        // fp32-accumulate mode on the tensor cores: q | k | v as (hi, lo) planes, three-pass products (attention_tcs.cu)
-        const int ld = 3 * H * hp;
-        DevBuf planes, cplanes;
+    if (f == Form::Bf16) pack_qkv_kernel<__nv_bfloat16><<<blocks_for(rows * ld), 256, 0, st>>>(q, k, v, rows, H, d, hp, qkv.as<__nv_bfloat16>());
+    else pack_qkv_kernel<float><<<blocks_for(rows * ld), 256, 0, st>>>(q, k, v, rows, H, d, hp, qkv.as<float>());
+    Operand a{qkv.p, nullptr, ld}, o{ctx.p, nullptr, H * hp};
+    if (f == Form::Split) {
         RC_TRY(planes.ensure(static_cast<size_t>(rows) * ld * 2 * 2));
-        RC_TRY(cplanes.ensure(static_cast<size_t>(rows) * H * hp * 2 * 2));
-        pack_qkv_kernel<float><<<blocks_for(rows * ld), 256, 0, st>>>(q, k, v, rows, H, d, hp, qkv.as<float>());
-        __nv_bfloat16* q_hi = planes.as<__nv_bfloat16>();
-        __nv_bfloat16* q_lo = q_hi + static_cast<size_t>(rows) * ld;
-        __nv_bfloat16* c_hi = cplanes.as<__nv_bfloat16>();
-        __nv_bfloat16* c_lo = c_hi + static_cast<size_t>(rows) * H * hp;
-        split_rows_kernel<<<blocks_for(rows * (ld >> 3)), 256, 0, st>>>(qkv.as<float>(), rows, ld, ld, q_hi, q_lo, ld);
-        ad.qkv = q_hi; ad.ctx = c_hi;
-        AttnPlan plan;
-        CUtensorMap tm_lo;
-        int rc = attn_bf16_make_plan(&plan, ad);
-        if (!rc) rc = make_tmap_bf16_2d(&tm_lo, q_lo, static_cast<int>(rows), ld, ld, 64);
-        if (rc) return fail(VITDET_E_INVALID, "op_attention: fp32 tensor-core plan failed: %d", rc);
-        CU_TRY(attn_tcs_launch(plan, tm_lo, c_lo, st));
-        unpack_ctx_planes_kernel<<<blocks_for(rows * H * d), 256, 0, st>>>(c_hi, c_lo, rows, H, d, hp, out);
-        CU_TRY(cudaGetLastError());
-        CU_TRY(cudaStreamSynchronize(st));
-        return 0;
-    } else {
-        pack_qkv_kernel<float><<<blocks_for(rows * 3 * H * hp), 256, 0, st>>>(q, k, v, rows, H, d, hp, qkv.as<float>());
-        CU_TRY(attn_f32_launch(ad, st));
-        unpack_ctx_kernel<float><<<blocks_for(rows * H * d), 256, 0, st>>>(ctx.as<float>(), rows, H, d, hp, out);
+        a = Operand{planes.p, planes.as<__nv_bfloat16>() + static_cast<size_t>(rows) * ld, ld};
+        o.lo = ctx.as<__nv_bfloat16>() + static_cast<size_t>(rows) * H * hp;
+        split_rows_kernel<<<blocks_for(rows * (ld >> 3)), 256, 0, st>>>(qkv.as<float>(), rows, ld, ld, planes.as<__nv_bfloat16>(),
+                                                                       static_cast<__nv_bfloat16*>(a.lo), ld);
     }
+    const AttnDesc ad = attn_desc(a, o, B, T, H, d, hp);
+    AttnTcPlan plan;
+    if (f != Form::Ieee) RC_TRY(attn_plan(&plan, ad, a.lo));
+    CU_TRY(attn_launch(f, ad, &plan, o.lo, st));
+    if (f == Form::Bf16) unpack_ctx_kernel<__nv_bfloat16><<<blocks_for(rows * H * d), 256, 0, st>>>(ctx.as<__nv_bfloat16>(), rows, H, d, hp, out);
+    else if (f == Form::Split)
+        unpack_ctx_planes_kernel<<<blocks_for(rows * H * d), 256, 0, st>>>(ctx.as<__nv_bfloat16>(), static_cast<const __nv_bfloat16*>(o.lo), rows, H, d, hp, out);
+    else unpack_ctx_kernel<float><<<blocks_for(rows * H * d), 256, 0, st>>>(ctx.as<float>(), rows, H, d, hp, out);
     CU_TRY(cudaGetLastError());
     CU_TRY(cudaStreamSynchronize(st));
     return 0;
@@ -1861,17 +1709,17 @@ int vitdet_op_dense_ex(const float* A, const float* kernel, const float* bias, c
     }
     const int ldc = ex->store_bf16 ? N8 : N4;
     RC_TRY(o_buf.ensure(static_cast<size_t>(M) * ldc * (ex->store_bf16 ? 2 : 4)));
-    DenseCall c{a_buf.p, K8, &w, ex->pos, ex->pos_period > 0 ? ex->pos_period : 1, rp, N4, o_buf.p, ldc, ex->store_bf16 ? 0 : 1, act, M};
+    DenseCall c{Operand{a_buf.p, nullptr, K8}, &w, M};
+    c.pos = ex->pos; c.pos_period = ex->pos_period > 0 ? ex->pos_period : 1;
+    c.resid = rp; c.ldr = N4;
+    c.out = Operand{o_buf.p, nullptr, ldc}; c.out_f32 = ex->store_bf16 ? 0 : 1; c.act = act;
     if (ex->ln_out) {
         RC_TRY(ln_buf.ensure(static_cast<size_t>(M) * N8 * 2));
         c.ln_gamma = ex->ln_gamma; c.ln_beta = ex->ln_beta; c.ln_eps = ex->ln_eps; c.ln_out = ln_buf.p; c.ln_ld = N8;
     }
-    TcGemmPlan plan;
-    GemmDesc g = make_desc(c, VITDET_MODE_BF16);
-    if (ex->pair > 0 && !pair_kernel_legal(g)) return fail(VITDET_E_INVALID, "op_dense_ex: the CTA-pair kernel needs M >= 1024, N >= 128 and no fused LayerNorm");
-    int rc = make_tc_plan(&plan, g, sms, ex->pair < 0 ? env_options().gemm_pair : (ex->pair ? 2 : 0));
-    if (rc) return fail(VITDET_E_INVALID, "op_dense_ex: tc_gemm_make_plan failed: %d", rc);
-    RC_TRY(launch_tc(plan, o_buf.p, rp, st));
+    if (ex->pair > 0 && !pair_kernel_legal(make_desc(c, Form::Bf16)))
+        return fail(VITDET_E_INVALID, "op_dense_ex: the CTA-pair kernel needs M >= 1024, N >= 128 and no fused LayerNorm");
+    RC_TRY(dense_once(c, Form::Bf16, sms, ex->pair < 0 ? env_options().gemm_pair : (ex->pair ? 2 : 0), st));
     if (ex->store_bf16) bf16_rows_to_f32_kernel<<<blocks_for(static_cast<long long>(M) * N), 256, 0, st>>>(o_buf.as<__nv_bfloat16>(), M, N, N8, out);
     else unpad_rows_f32_kernel<<<blocks_for(static_cast<long long>(M) * N), 256, 0, st>>>(o_buf.as<float>(), M, N, N4, out);
     if (ex->ln_out) bf16_rows_to_f32_kernel<<<blocks_for(static_cast<long long>(M) * N), 256, 0, st>>>(ln_buf.as<__nv_bfloat16>(), M, N, N8, ex->ln_out);

@@ -633,7 +633,7 @@ class VisionTransformerDetector:
 
     # -- run-time switches and debug taps (parity tests, A/B measurements) ---------------------------
     def set_option(self, key: str, value: int) -> None:
-        """'fuse_ln', 'fuse_tail', 'gemm_pair' (0/1/2), 'attention' (4/8) — see include/vitdet_b200.h."""
+        """'fuse_ln', 'fuse_tail', 'gemm_pair' (0/1/2), 'fp32_tc' — see include/vitdet_b200.h."""
         _capi.check(self._lib.vitdet_set_option(self._h, key.encode(), int(value)))
 
     def get_option(self, key: str) -> int:
