@@ -31,6 +31,6 @@ echo "ncu rowops rc=$?"
 BENCH32="python bench.py --mode fp32 --steps 1 --warmup 3 --no-cpu-baseline --no-e2e --no-variants"
 timeout 600 $BENCH32 > $O/plain32.log 2>&1 &&
 timeout 900 ncu --set full --clock-control none -k regex:"gemm_tc2_kernel" -s 0 -c 1 -f -o $O/prof_fp32_gemm $BENCH32 > $O/ncu_fp32_gemm.log 2>&1
-timeout 900 ncu --set full --clock-control none -k regex:"attn_tcs_kernel" -s 1 -c 1 -f -o $O/prof_fp32_attn $BENCH32 > $O/ncu_fp32_attn.log 2>&1
+timeout 900 ncu --set full --clock-control none -k regex:attn_tc_kernel -s 1 -c 1 -f -o $O/prof_fp32_attn $BENCH32 > $O/ncu_fp32_attn.log 2>&1
 echo "ncu fp32 rc=$?"
 ls -la $O/*.ncu-rep

@@ -546,9 +546,10 @@ static int build_weight_table(vitdet_handle* h) {
 // Split: the fp32 mode on the tensor cores (north_star: <= 1e-3 against the float32 reference).  Every float32 activation
 //        that feeds a Dense layer or the attention core travels as two bf16 planes (hi = bf16(x), lo = bf16(x - hi)) and
 //        every Dense is three tcgen05 passes (hi*hi + hi*lo + lo*hi, float32 accumulation in TMEM) through the same two
-//        GEMM kernels as Bf16, with exact expf-based activations in the epilogue; attention is attention_tcs.cu.  The
-//        residual stream, LayerNorm, the head's slot projection and last Dense stay IEEE float32.  Buffers are sized
-//        as the fp32 mode's (4 bytes per element): the hi plane in the first half, the lo plane in the second (planes_of).
+//        GEMM kernels as Bf16, with exact expf-based activations in the epilogue; attention is the split instance of
+//        attention_tc.cu.  The residual stream, LayerNorm, the head's slot projection and last Dense stay IEEE float32.
+//        Buffers are sized as the fp32 mode's (4 bytes per element): the hi plane in the first half, the lo plane in the
+//        second (planes_of).
 // Ieee:  the fp32 mode on IEEE float32 CUDA-core kernels (gemm_simt.cu, attn_f32): "fp32_tc" = 0, or heads wider than
 //        the split attention kernel takes (it holds hi and lo tiles: one 64-column box per head).
 enum class Form { Bf16, Split, Ieee };
