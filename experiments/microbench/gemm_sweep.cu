@@ -17,11 +17,11 @@ static void* dalloc(size_t bytes, int fill) {
 
 struct Case { const char* name; int M, K, N, act, out_f32, resid, ln, pair, block_n; int ld = 0; };
 
-static float time_plan(const TcGemmPlan& plan, bool pair, int reps) {
+static float time_plan(const TcGemmPlan& plan, int reps) {
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
-    for (int i = 0; i < 3; ++i) pair ? tc2_gemm_launch(plan, 0) : tc_gemm_launch(plan, 0);
+    for (int i = 0; i < 3; ++i) tc_gemm_launch(plan, 0);
     cudaEventRecord(e0);
-    for (int i = 0; i < reps; ++i) pair ? tc2_gemm_launch(plan, 0) : tc_gemm_launch(plan, 0);
+    for (int i = 0; i < reps; ++i) tc_gemm_launch(plan, 0);
     cudaEventRecord(e1);
     cudaError_t err = cudaDeviceSynchronize();
     if (err != cudaSuccess) { printf("error %s\n", cudaGetErrorString(err)); exit(1); }
@@ -78,9 +78,9 @@ int main() {
             d.out = out; d.ldc = (c.N + 7) / 8 * 8;
         }
         TcGemmPlan plan;
-        int r = c.pair ? tc2_gemm_make_plan(&plan, d, 148) : tc_gemm_make_plan(&plan, d, 148);
+        int r = tc_gemm_make_plan(&plan, d, 148, c.pair);
         if (r) { printf("%-28s plan error %d\n", c.name, r); continue; }
-        const float us = time_plan(plan, c.pair, 20);
+        const float us = time_plan(plan, 20);
         printf("%-28s M %6d K %4d N %4d bn %3d stages %d tiles %5d (%.1f / CTA): %7.1f us  %6.0f clk/tile@1.8GHz\n", c.name, c.M, c.K, c.N,
                plan.block_n, plan.num_stages, plan.num_tiles, plan.num_tiles / double(plan.grid), us,
                us * 1800.0 / (plan.num_tiles / double(plan.grid)));

@@ -35,14 +35,14 @@ int main(int argc, char** argv) {
     else { printf("unknown case\n"); return 1; }
     d.lda = (d.K + 7) / 8 * 8; d.ldw = d.lda; d.ldc = d.N;
     TcGemmPlan plan;
-    int r = pair ? tc2_gemm_make_plan(&plan, d, 148) : tc_gemm_make_plan(&plan, d, 148);
+    int r = tc_gemm_make_plan(&plan, d, 148, pair);
     if (r) { printf("plan error %d\n", r); return 1; }
     cudaEvent_t e0, e1; cudaEventCreate(&e0); cudaEventCreate(&e1);
     auto t0 = std::chrono::steady_clock::now();
     long launches = 0; float ms_total = 0.f;
     while (std::chrono::duration<double>(std::chrono::steady_clock::now() - t0).count() < seconds) {
         cudaEventRecord(e0);
-        for (int i = 0; i < 50; ++i) pair ? tc2_gemm_launch(plan, 0) : tc_gemm_launch(plan, 0);
+        for (int i = 0; i < 50; ++i) tc_gemm_launch(plan, 0);
         cudaEventRecord(e1);
         if (cudaDeviceSynchronize() != cudaSuccess) { printf("launch failed\n"); return 1; }
         float ms; cudaEventElapsedTime(&ms, e0, e1); ms_total += ms; launches += 50;

@@ -94,10 +94,10 @@ def traffic(tag):
     out = {"kernel": row[hdr.index("Kernel Name")][:80], "dram_bytes_read": val("dram__bytes_read.sum"),
            "dram_bytes_write": val("dram__bytes_write.sum"), "source": f"profiles/{tag}_ncu_gemm.md (ncu --set full, B = 64)"}
     out["traffic_bytes_per_launch"] = out["dram_bytes_read"] + out["dram_bytes_write"]
-    # stamp: bench.py quotes the figure only for the source tree and launch size it was captured on
+    # stamp: bench.py quotes the figure only for the machine code and launch size it was captured on
     hp = os.path.join(OUT, "kernel_hash.txt")
     out["kernel_hash"] = open(hp).read().strip() if os.path.exists(hp) else None
-    out["kernel_hash_of"] = "gemm_tc2.cu common.cuh kernels.h launch.h + nvcc flags (vision_transformer_detector_b200.build.kernel_hash)"
+    out["kernel_hash_of"] = "sha256 of the SASS of gemm_tc_kernel<ACT_MISH, 0, false, true> (vision_transformer_detector_b200.build.kernel_hash)"
     out["rows_per_launch"] = 64 * 1296
     with open(os.path.join(PROF, "gemm_mlp_2_traffic.json"), "w") as f:
         json.dump(out, f, indent=1)

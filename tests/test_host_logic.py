@@ -131,15 +131,15 @@ def test_category_names_match_the_reference_table():
 
 def test_traffic_capture_is_stamped_for_the_current_kernel_sources():
     """bench.py quotes roofline.traffic from profiles/gemm_mlp_2_traffic.json only while the capture's stamp equals the hash
-    of the dominant kernel's sources (gemm_tc2.cu + the headers it includes + the nvcc flags).  A change to those files
-    needs a new `ncu --set full` capture (scripts/gpu_round2.sh + scripts/summarize_profiles.py), otherwise the bench line
-    silently carries `traffic: null`."""
+    of the dominant kernel's SASS (gemm_tc_kernel<ACT_MISH, 0, false, true>, the CTA-pair bf16 Mish instance, compiled
+    with the library's nvcc flags).  A change to its machine code needs a new `ncu --set full` capture
+    (scripts/gpu_round2.sh + scripts/summarize_profiles.py), otherwise the bench line silently carries `traffic: null`."""
     import json
     import os
     from vision_transformer_detector_b200 import build
     path = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "profiles", "gemm_mlp_2_traffic.json")
     t = json.load(open(path))
-    assert t["kernel_hash"] == build.kernel_hash(), "re-capture the dominant GEMM under ncu: its sources changed"
+    assert t["kernel_hash"] == build.kernel_hash(), "re-capture the dominant GEMM under ncu: its machine code changed"
     assert t["rows_per_launch"] == 64 * 1296
     # no re-reads: measured DRAM traffic within 5 % of the algorithmic bytes 2 (M (K + N) + K N)
     algorithmic = 2.0 * (82944 * (3584 + 1792) + 3584 * 1792)

@@ -596,9 +596,10 @@ static GemmDesc make_desc(const DenseCall& c, Form f) {
     return g;
 }
 
-// The CTA-pair kernel (gemm_tc2.cu) serves the layers with enough rows, columns and depth to fill 256 x BN
-// cluster tiles; VITDET_GEMM_PAIR=0 forces the single-CTA kernel everywhere, =all the pair kernel wherever it
-// is legal (A/B measurements and tests).
+// The CTA-pair form of the GEMM (gemm_tc.cu) serves the layers with enough rows, columns and depth to fill 256 x BN
+// cluster tiles; VITDET_GEMM_PAIR=0 forces the single-CTA form everywhere, =all the pair form wherever it
+// is legal (A/B measurements and tests).  The pair form has no fused LayerNorm, and no narrow float32 epilogue
+// (its float32 layers take the wide one, OUT = 3).
 // Measured (B = 64): 3 % faster on the MMA-bound layers (3584 -> 1792 -> 896 -> 448), slower on the K = 28
 // layers whose time is the epilogue (the pair couples both CTAs' epilogues), hence the K threshold.
 static bool pair_kernel_legal(const GemmDesc& g) { return g.M >= 1024 && g.N >= 128 && !g.ln_out; }
@@ -612,8 +613,7 @@ static bool use_pair_kernel(int pair_mode, const GemmDesc& g) {
 // Tensor-core plan of one Dense (Bf16 / Split)
 static int plan_dense(TcGemmPlan* plan, const DenseCall& c, Form f, int num_sms, int pair_mode) {
     const GemmDesc g = make_desc(c, f);
-    plan->pair = use_pair_kernel(pair_mode, g) ? 1 : 0;
-    const int rc = plan->pair ? tc2_gemm_make_plan(plan, g, num_sms) : tc_gemm_make_plan(plan, g, num_sms);
+    const int rc = tc_gemm_make_plan(plan, g, num_sms, use_pair_kernel(pair_mode, g) ? 1 : 0);
     if (rc) return fail(VITDET_E_INVALID, "tensor-core GEMM plan (M=%d N=%d K=%d lda=%d ldc=%d) failed: %d", g.M, g.N, g.K, g.lda, g.ldc, rc);
     return 0;
 }
@@ -622,7 +622,7 @@ static int launch_tc(TcGemmPlan plan /*by value: out / resid are patched per lau
                      cudaStream_t st) {
     plan.desc.out = out;
     plan.desc.resid = resid;
-    cudaError_t e = plan.pair ? tc2_gemm_launch(plan, st) : tc_gemm_launch(plan, st);
+    cudaError_t e = tc_gemm_launch(plan, st);
     if (e != cudaSuccess) return fail(VITDET_E_CUDA, "tc_gemm_launch failed: %s", cudaGetErrorString(e));
     return 0;
 }

@@ -20,6 +20,18 @@
 // Two TMEM accumulator stages (2 x 256 columns) let the MMA of tile i+1 overlap the epilogue of
 // tile i.  BN and the ring depth are run-time values (N lives in the instruction descriptor), so one
 // binary serves every layer width of the model.
+//
+// CTA-pair form (PAIR, cta_group::2) for the large layers (the 3584 -> 1792 MLP layer is 37 % of the forward):
+// two CTAs on the two SMs of a TPC form a cluster and compute one 256 x BN tile.  Each CTA stages ITS 128 rows
+// of A and HALF of the BN rows of W per k-block; the producers' loads complete on the LEADER's full barrier, the
+// leader's MMA warp issues tcgen05.mma.cta_group::2 (M = 256) and commits with multicast so that both CTAs'
+// "stage empty" / "accumulator full" barriers fire, each CTA's TMEM receives the accumulator of its own 128 rows,
+// and both CTAs' epilogue warps arrive on the leader's "accumulator drained" barrier.  Per SM and per MMA the
+// tensor core then reads 4 KB (A) + 4 KB (half of B) of shared memory instead of 4 + 8 KB, and TMA fills 32 KB
+// per k-block instead of 48 KB: the single-CTA kernel sat at 81 % tensor-pipe activity with the shared-memory
+// operand pipe at 75 % of its rate (profiles/r01b_ncu_gemm.md).
+#include <type_traits>
+
 #include "common.cuh"
 #include "kernels.h"
 #include "launch.h"
@@ -31,7 +43,21 @@ namespace {
 template <int ACT, bool F32ACC>
 __device__ __forceinline__ float act_out(float x) { return F32ACC ? apply_act_f32acc<ACT>(x) : apply_act<ACT, false>(x); }
 
-constexpr int kBM = 128;              // UMMA M (cta_group::1)
+// The cta_group::1 / cta_group::2 forms of the TMA load, the MMA and its commit
+template <bool PAIR>
+__device__ __forceinline__ void tma_load(uint32_t smem_dst, const CUtensorMap* map, uint32_t bar, int c0, int c1) {
+    if constexpr (PAIR) tma_load_2d_2sm(smem_dst, map, bar, c0, c1); else tma_load_2d(smem_dst, map, bar, c0, c1);
+}
+template <bool PAIR>
+__device__ __forceinline__ void umma(uint32_t tmem_d, uint64_t desc_a, uint64_t desc_b, uint32_t idesc, uint32_t accumulate) {
+    if constexpr (PAIR) umma_bf16_ss_2sm(tmem_d, desc_a, desc_b, idesc, accumulate); else umma_bf16_ss(tmem_d, desc_a, desc_b, idesc, accumulate);
+}
+template <bool PAIR>
+__device__ __forceinline__ void commit(uint32_t bar) {
+    if constexpr (PAIR) umma_commit_2sm(bar, 3); else umma_commit(bar);      // pair: the barrier at `bar` in both CTAs
+}
+
+constexpr int kBM = 128;              // rows of A per CTA (UMMA M of cta_group::1; the pair's M is 256)
 constexpr int kBK = 64;               // one 128-byte swizzle row of bf16
 constexpr int kUK = 16;               // UMMA K for 16-bit inputs
 constexpr int kMaxBN = 256;
@@ -68,7 +94,12 @@ struct TcGemmArgs {
     int ldc;
     int n_store;   // round_up(N, store vector): columns [N, n_store) are written as zero
     int split;     // 1: A and W are (hi, lo) bf16 planes; three passes over K (hi*hi, hi*lo, lo*hi)
-    const float* ln_gamma;      // fused LayerNorm of the output row (f32 output, N <= 32), or nullptr
+};
+// The single-CTA form's arguments add the fused LayerNorm of the output row (f32 output, N <= 32).  The pair form has none, so
+// its kernel parameters end with TcGemmArgs: a parameter block of more than 128 bytes changes how the compiler loads the
+// fields, and with it the machine code of the pair instances.
+struct TcGemmLnArgs : TcGemmArgs {
+    const float* ln_gamma;      // or nullptr
     const float* ln_beta;
     float ln_eps;
     __nv_bfloat16* ln_out;
@@ -78,13 +109,16 @@ struct TcGemmArgs {
 // OUT: 0 bf16 (TMA store), 1 float32 rows of <= 32 columns (direct stores, residual, fused LayerNorm), 2 split bf16 planes (hi, lo),
 //      3 float32 rows wider than 32 columns (coalesced stores through the staging tile, residual prefetched)
 // PRECISE: exact activations (the fp32-accumulate mode)
-template <int ACT, int OUT, bool PRECISE>
+// PAIR: CTA-pair form, launched as clusters of two CTAs (no fused LayerNorm)
+template <int ACT, int OUT, bool PRECISE, bool PAIR>
 __global__ void __launch_bounds__(kThreads, 1)   // 96 registers is the most 576 threads can be granted (104 and 112 fail to launch)
 gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmC, const __grid_constant__ CUtensorMap tmA_lo,
-               const __grid_constant__ CUtensorMap tmB_lo, const __grid_constant__ CUtensorMap tmC_lo, const TcGemmArgs p) {
+               const __grid_constant__ CUtensorMap tmB_lo, const __grid_constant__ CUtensorMap tmC_lo,
+               const std::conditional_t<PAIR, TcGemmArgs, TcGemmLnArgs> p) {
     constexpr bool OUT_F32 = OUT == 1 || OUT == 3;
     constexpr bool WIDE_F32 = OUT == 3;      // float32 rows wider than one 32-column chunk: coalesced stores through the staging tile
+    constexpr int kCtas = PAIR ? 2 : 1;      // CTAs per tile
     extern __shared__ __align__(1024) uint8_t smem_raw[];
     __shared__ __align__(8) uint64_t bars[2 * kMaxStages + 4];
     __shared__ uint32_t tmem_base_s;
@@ -98,7 +132,9 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
     // epilogue store staging after the ring: one 2 KB tile per warp, two (hi, lo) in the split-output mode
     constexpr uint32_t kStoreStride = OUT == 2 ? 2 * kStoreTileBytes : kStoreTileBytes;
     const uint32_t s_store0 = smem_base + (OUT == 2 ? kRingBytes - kStoreBytes : kRingBytes);
-    const uint32_t stage_bytes_b = static_cast<uint32_t>(p.block_n) * (kBK * 2);
+    const uint32_t stage_bytes_b = static_cast<uint32_t>(p.block_n / kCtas) * (kBK * 2);      // this CTA's part of the W tile
+    const uint32_t cta_rank = PAIR ? cluster_ctarank() : 0u;
+    const bool leader = cta_rank == 0;
     const uint32_t sA0 = smem_base;
     const uint32_t sB0 = smem_base + static_cast<uint32_t>(p.num_stages) * kStageBytesA;
 
@@ -114,7 +150,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         }
         for (int a = 0; a < 2; ++a) {
             mbar_init(bar_tfull + 8 * a, 1);
-            mbar_init(bar_tempty + 8 * a, kEpiWarps);
+            mbar_init(bar_tempty + 8 * a, kCtas * kEpiWarps);     // pair: the leader's copy collects both CTAs' epilogue warps
         }
         fence_mbar_init();
     }
@@ -126,11 +162,12 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (OUT == 2) tma_prefetch_desc(&tmC_lo);
     }
     if (warp == kMmaWarp) {
-        tmem_alloc(smem_u32(&tmem_base_s), kTmemCols);
-        tmem_relinquish();
+        if constexpr (PAIR) { tmem_alloc_2sm(smem_u32(&tmem_base_s), kTmemCols); tmem_relinquish_2sm(); }
+        else { tmem_alloc(smem_u32(&tmem_base_s), kTmemCols); tmem_relinquish(); }
     }
     tc_fence_before();
-    __syncthreads();
+    if constexpr (PAIR) cluster_sync_all();      // barriers of BOTH CTAs are initialised before any remote arrive / multicast commit
+    else __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = tmem_base_s;
     pdl_wait();       // set-up above overlapped the previous kernel; its outputs are read from here on
@@ -140,56 +177,60 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            const uint32_t tx_bytes = kStageBytesA + stage_bytes_b;
-            for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x) {
-                const int m0 = (tile / p.n_tiles) * kBM;
-                const int n0 = (tile % p.n_tiles) * p.block_n;
+            // pair: this CTA's loads complete on the LEADER's full barrier (same offset, CTA rank 0)
+            const uint32_t bar_full_leader = PAIR ? mapa_shared(bar_full, 0) : bar_full;
+            const uint32_t tx_bytes = kCtas * (kStageBytesA + stage_bytes_b);       // pair: both CTAs' boxes
+            for (int tile = blockIdx.x / kCtas; tile < p.num_tiles; tile += gridDim.x / kCtas) {
+                const int m0 = (tile / p.n_tiles) * (kCtas * kBM) + static_cast<int>(cta_rank) * kBM;
+                const int n0 = (tile % p.n_tiles) * p.block_n + static_cast<int>(cta_rank) * (p.block_n / 2);
                 for (int kb = 0; kb < p.num_kb; ++kb) {
                     // split mode: the k-block is visited three times, with (A, W) = (hi, hi), (hi, lo), (lo, hi)
                     for (int t = 0; t < ((PRECISE && p.split) ? 3 : 1); ++t) {
                         mbar_wait(bar_empty + 8 * stage, phase ^ 1u);
-                        mbar_arrive_expect_tx(bar_full + 8 * stage, tx_bytes);
-                        tma_load_2d(sA0 + stage * kStageBytesA, t == 2 ? &tmA_lo : &tmA, bar_full + 8 * stage, kb * kBK, m0);
-                        tma_load_2d(sB0 + stage * stage_bytes_b, t == 1 ? &tmB_lo : &tmB, bar_full + 8 * stage, kb * kBK, n0);
+                        if (leader) mbar_arrive_expect_tx(bar_full + 8 * stage, tx_bytes);
+                        tma_load<PAIR>(sA0 + stage * kStageBytesA, t == 2 ? &tmA_lo : &tmA, bar_full_leader + 8 * stage, kb * kBK, m0);
+                        tma_load<PAIR>(sB0 + stage * stage_bytes_b, t == 1 ? &tmB_lo : &tmB, bar_full_leader + 8 * stage, kb * kBK, n0);
                         if (++stage == p.num_stages) { stage = 0; phase ^= 1u; }
                     }
                 }
             }
         }
     } else if (warp == kMmaWarp) {
-        // ------------------------------ MMA issuer --------------------------------
+        // ------------------------------ MMA issuer (pair: leader CTA only) --------
         // The WHOLE warp runs this loop (warp-uniform control flow keeps the loop state in uniform registers);
         // only the tcgen05 instructions are issued by one elected lane.
-        const uint32_t idesc = umma_idesc_bf16_f32(kBM, p.block_n);
-        const uint64_t da0 = umma_desc_sw128_kmajor(sA0), db0 = umma_desc_sw128_kmajor(sB0);
-        const uint32_t a_step = kStageBytesA >> 4, b_step = stage_bytes_b >> 4;      // descriptor address units (16 B)
-        const int last_steps = (p.K - (p.num_kb - 1) * kBK + kUK - 1) / kUK;         // k-steps of the last k-block (1..4)
-        int stage = 0;
-        uint32_t phase = 0;
-        int it = 0;
-        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
-            const int acc = it & 1;
-            const uint32_t acc_phase = (it >> 1) & 1;
-            mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1u);
-            tc_fence_after();
-            const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(acc * kMaxBN);
-            const int passes = (PRECISE && p.split) ? 3 : 1;      // split planes only exist in the fp32-accumulate mode
-            for (int kb = 0; kb < p.num_kb; ++kb) {
-                const int ksteps = (kb == p.num_kb - 1) ? last_steps : kBK / kUK;
-                for (int t = 0; t < passes; ++t) {
-                    mbar_wait(bar_full + 8 * stage, phase);
-                    tc_fence_after();
-                    if (elect_one()) {
-                        const uint64_t da = da0 + static_cast<uint64_t>(stage * a_step), db = db0 + static_cast<uint64_t>(stage * b_step);
-                        umma_bf16_ss(d_tmem, da, db, idesc, (kb | t) != 0);
-                        if (ksteps > 1) umma_bf16_ss(d_tmem, da + 2u, db + 2u, idesc, 1u);
-                        if (ksteps > 2) umma_bf16_ss(d_tmem, da + 4u, db + 4u, idesc, 1u);
-                        if (ksteps > 3) umma_bf16_ss(d_tmem, da + 6u, db + 6u, idesc, 1u);
-                        umma_commit(bar_empty + 8 * stage);
-                        if (kb == p.num_kb - 1 && t == passes - 1) umma_commit(bar_tfull + 8 * acc);
+        if (leader) {
+            const uint32_t idesc = umma_idesc_bf16_f32(kCtas * kBM, p.block_n);
+            const uint64_t da0 = umma_desc_sw128_kmajor(sA0), db0 = umma_desc_sw128_kmajor(sB0);
+            const uint32_t a_step = kStageBytesA >> 4, b_step = stage_bytes_b >> 4;      // descriptor address units (16 B)
+            const int last_steps = (p.K - (p.num_kb - 1) * kBK + kUK - 1) / kUK;         // k-steps of the last k-block (1..4)
+            int stage = 0;
+            uint32_t phase = 0;
+            int it = 0;
+            for (int tile = blockIdx.x / kCtas; tile < p.num_tiles; tile += gridDim.x / kCtas, ++it) {
+                const int acc = it & 1;
+                const uint32_t acc_phase = (it >> 1) & 1;
+                mbar_wait(bar_tempty + 8 * acc, acc_phase ^ 1u);
+                tc_fence_after();
+                const uint32_t d_tmem = tmem_base + static_cast<uint32_t>(acc * kMaxBN);
+                const int passes = (PRECISE && p.split) ? 3 : 1;      // split planes only exist in the fp32-accumulate mode
+                for (int kb = 0; kb < p.num_kb; ++kb) {
+                    const int ksteps = (kb == p.num_kb - 1) ? last_steps : kBK / kUK;
+                    for (int t = 0; t < passes; ++t) {
+                        mbar_wait(bar_full + 8 * stage, phase);
+                        tc_fence_after();
+                        if (elect_one()) {
+                            const uint64_t da = da0 + static_cast<uint64_t>(stage * a_step), db = db0 + static_cast<uint64_t>(stage * b_step);
+                            umma<PAIR>(d_tmem, da, db, idesc, (kb | t) != 0);
+                            if (ksteps > 1) umma<PAIR>(d_tmem, da + 2u, db + 2u, idesc, 1u);
+                            if (ksteps > 2) umma<PAIR>(d_tmem, da + 4u, db + 4u, idesc, 1u);
+                            if (ksteps > 3) umma<PAIR>(d_tmem, da + 6u, db + 6u, idesc, 1u);
+                            commit<PAIR>(bar_empty + 8 * stage);
+                            if (kb == p.num_kb - 1 && t == passes - 1) commit<PAIR>(bar_tfull + 8 * acc);
+                        }
+                        __syncwarp();
+                        if (++stage == p.num_stages) { stage = 0; phase ^= 1u; }
                     }
-                    __syncwarp();
-                    if (++stage == p.num_stages) { stage = 0; phase ^= 1u; }
                 }
             }
         }
@@ -200,17 +241,21 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         const int quad = warp & 3;                    // TMEM lane quadrant this warp may access
         const int sub = warp >> 2;                    // which chunks of the tile (c0 = 32*sub, +128, ...)
         int it = 0;
-        for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
+        const uint32_t bar_tempty_leader = PAIR ? mapa_shared(bar_tempty, 0) : bar_tempty;
+        for (int tile = blockIdx.x / kCtas; tile < p.num_tiles; tile += gridDim.x / kCtas, ++it) {
             const int acc = it & 1;
             const uint32_t acc_phase = (it >> 1) & 1;
-            const int m0 = (tile / p.n_tiles) * kBM;
+            const int m0 = (tile / p.n_tiles) * (kCtas * kBM) + static_cast<int>(cta_rank) * kBM;   // this CTA's 128 rows
             const int n0 = (tile % p.n_tiles) * p.block_n;
 
             // Bias is read straight from global memory below (a warp-wide broadcast that stays in L1): no staging
             // barrier per tile, so the sixteen epilogue warps drift apart and their SFU phases interleave.
             const float* bs = p.bias + n0;      // valid for columns < N only; the tail path guards its reads
-            const int row = m0 + quad * 32 + lane;
-            const bool row_ok = row < p.M;
+            // The thread's row: the single-CTA form computes it before the wait for the accumulator (the residual prefetch
+            // below needs it), the pair form after the wait, where its instances compile to 16 fewer instructions.
+            int row = 0;
+            bool row_ok = false;
+            if constexpr (!PAIR) { row = m0 + quad * 32 + lane; row_ok = row < p.M; }
             // Narrow float32 rows (the 28-wide residual stream: output projection): the thread's residual row is fetched
             // BEFORE the wait for the accumulator, so that the global-load latency hides behind the tile's MMAs.
             float4 rpre[8];
@@ -225,6 +270,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             }
             mbar_wait(bar_tfull + 8 * acc, acc_phase);
             tc_fence_after();
+            if constexpr (PAIR) { row = m0 + quad * 32 + lane; row_ok = row < p.M; }
             float pos_v = 0.f;
             if (p.pos != nullptr && row_ok) pos_v = __ldg(p.pos + (row % p.pos_period));
             const uint32_t t_row = tmem_base + (static_cast<uint32_t>(quad * 32) << 16) +
@@ -294,7 +340,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
 #pragma unroll
                         for (int j = 0; j < 4; ++j) xr[4 * g + j] = x[j];
                     }
-                    if (p.ln_out != nullptr) {
+                    if constexpr (!PAIR) if (p.ln_out != nullptr) {
                         // keras LayerNormalization(axis=-1) of the row just produced (the host only sets ln_out when
                         // the whole row is this one chunk): biased variance, eps inside the rsqrt, f32 statistics
                         const float inv_n = 1.f / static_cast<float>(p.N);
@@ -390,16 +436,21 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
             }
             tc_fence_before();
             __syncwarp();
-            if (lane == 0) mbar_arrive(bar_tempty + 8 * acc);
+            if (lane == 0) {
+                if constexpr (PAIR) mbar_arrive_cluster(bar_tempty_leader + 8 * acc);
+                else mbar_arrive(bar_tempty + 8 * acc);
+            }
         }
         if (!OUT_F32 && lane == 0) tma_store_wait_all();
     }
 
     tc_fence_before();
-    __syncthreads();
+    if constexpr (PAIR) cluster_sync_all();      // the leader's MMAs touch the peer's smem and TMEM: nobody leaves early
+    else __syncthreads();
     if (warp == kMmaWarp) {
         tc_fence_after();
-        tmem_dealloc(tmem_base, kTmemCols);
+        if constexpr (PAIR) tmem_dealloc_2sm(tmem_base, kTmemCols);
+        else tmem_dealloc(tmem_base, kTmemCols);
     }
 }
 
@@ -424,25 +475,29 @@ EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-template <int ACT, int OUT, bool PRECISE>
-cudaError_t launch_variant(const TcGemmPlan& plan, const TcGemmArgs& a, cudaStream_t stream) {
-    auto kern = gemm_tc_kernel<ACT, OUT, PRECISE>;
+template <int ACT, int OUT, bool PRECISE, bool PAIR>
+cudaError_t launch_variant(const TcGemmPlan& plan, const TcGemmLnArgs& a, cudaStream_t stream) {
+    auto kern = gemm_tc_kernel<ACT, OUT, PRECISE, PAIR>;
     {
         cudaError_t e = ensure_max_dynamic_smem(reinterpret_cast<const void*>(kern), kMaxDynSmem);
         if (e != cudaSuccess) return e;
     }
-    return launch_kernel(kern, dim3(plan.grid), dim3(kThreads), plan.smem_bytes, stream, 1, plan.tmA, plan.tmB, plan.tmC, plan.tmA_lo,
-                         plan.tmB_lo, plan.tmC_lo, a);
+    return launch_kernel(kern, dim3(plan.grid), dim3(kThreads), plan.smem_bytes, stream, PAIR ? 2 : 1, plan.tmA, plan.tmB, plan.tmC,
+                         plan.tmA_lo, plan.tmB_lo, plan.tmC_lo, a);
 }
 
-template <int ACT>
-cudaError_t launch_act(const TcGemmPlan& plan, const TcGemmArgs& a, cudaStream_t stream) {
+template <int ACT, bool PAIR>
+cudaError_t launch_act(const TcGemmPlan& plan, const TcGemmLnArgs& a, cudaStream_t stream) {
     const GemmDesc& d = plan.desc;
-    if (d.out_f32 && d.N > 32 && !d.ln_out)      // wide float32 rows: separate instantiation, so that the narrow (28-wide) epilogue keeps its registers
-        return d.precise ? launch_variant<ACT, 3, true>(plan, a, stream) : launch_variant<ACT, 3, false>(plan, a, stream);
-    if (d.out_f32) return d.precise ? launch_variant<ACT, 1, true>(plan, a, stream) : launch_variant<ACT, 1, false>(plan, a, stream);
-    if (d.out_split) return launch_variant<ACT, 2, true>(plan, a, stream);      // split planes only exist in the fp32-accumulate mode
-    return launch_variant<ACT, 0, false>(plan, a, stream);
+    // Wide float32 rows: separate instantiation, so that the narrow (28-wide) epilogue keeps its registers.  The pair form has
+    // no narrow instantiation: its float32 layers are wide (N >= 128), and OUT = 3 handles a partial chunk as OUT = 1 does.
+    if (d.out_f32 && (PAIR || (d.N > 32 && !d.ln_out)))
+        return d.precise ? launch_variant<ACT, 3, true, PAIR>(plan, a, stream) : launch_variant<ACT, 3, false, PAIR>(plan, a, stream);
+    if constexpr (!PAIR) {
+        if (d.out_f32) return d.precise ? launch_variant<ACT, 1, true, PAIR>(plan, a, stream) : launch_variant<ACT, 1, false, PAIR>(plan, a, stream);
+    }
+    if (d.out_split) return launch_variant<ACT, 2, true, PAIR>(plan, a, stream);      // split planes only exist in the fp32-accumulate mode
+    return launch_variant<ACT, 0, false, PAIR>(plan, a, stream);
 }
 
 }  // namespace
@@ -485,7 +540,8 @@ int make_tmap_bf16_2d(CUtensorMap* map, const void* base, int rows, int cols, in
     return make_tmap_bf16_2d_ex(map, base, rows, cols, ld, kBK, box_rows, 128);
 }
 
-int tc_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms) {
+// pair: tile = 256 rows x BN columns per cluster of two CTAs, W box = BN/2 rows per CTA.
+int tc_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms, int pair) {
     if (d.M <= 0 || d.N <= 0 || d.K <= 0) return -2;
     if ((d.lda % 8) || (d.ldw % 8)) return -3;                        // 16-byte row pitch for TMA
     if ((reinterpret_cast<uintptr_t>(d.A) & 15) || (reinterpret_cast<uintptr_t>(d.W) & 15) ||
@@ -498,32 +554,36 @@ int tc_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms) {
     if (d.split && !d.precise) return -12;      // split planes belong to the fp32-accumulate (precise) instantiations
     if (d.split && (!d.A_lo || !d.W_lo || (reinterpret_cast<uintptr_t>(d.A_lo) & 15) || (reinterpret_cast<uintptr_t>(d.W_lo) & 15))) return -10;
     if (d.out_split && (d.out_f32 || !d.out_lo || (reinterpret_cast<uintptr_t>(d.out_lo) & 15))) return -11;
-    if (d.ln_out && (!d.out_f32 || d.N > 32 || !d.ln_gamma || !d.ln_beta || (d.ln_ld % 8) || d.ln_ld < (d.N + 7) / 8 * 8 || d.ln_ld > 32 ||
-                     (reinterpret_cast<uintptr_t>(d.ln_out) & 15)))
-        return -9;                            // fused LayerNorm needs the whole row in one 32-column chunk
+    if (d.ln_out && (pair || !d.out_f32 || d.N > 32 || !d.ln_gamma || !d.ln_beta || (d.ln_ld % 8) || d.ln_ld < (d.N + 7) / 8 * 8 ||
+                     d.ln_ld > 32 || (reinterpret_cast<uintptr_t>(d.ln_out) & 15)))
+        return -9;                            // fused LayerNorm: single-CTA form only, the whole row in one 32-column chunk
     int bn = d.block_n > 0 ? d.block_n : choose_block_n(d.N);
     if (bn % 32 || bn < 32 || bn > kMaxBN) return -7;
 
+    const int ctas = pair ? 2 : 1;
+    const int box_n = bn / ctas;      // rows of W each CTA stages
     plan->desc = d;
+    plan->pair = pair ? 1 : 0;
     plan->block_n = bn;
-    const int stage = kStageBytesA + bn * kBK * 2;
+    const int stage = kStageBytesA + box_n * kBK * 2;
     const int ring = d.out_split ? kRingBytes - kStoreBytes : kRingBytes;       // split output: two staging tiles per epilogue warp
     int stages = ring / stage;
     if (stages > kMaxStages) stages = kMaxStages;
     plan->num_stages = stages;
     plan->smem_bytes = kMaxDynSmem;    // ring (up to 192 KB) + store staging, fixed layout
-    const int m_tiles = (d.M + kBM - 1) / kBM;
+    const int m_tiles = (d.M + ctas * kBM - 1) / (ctas * kBM);
     const int n_tiles = (d.N + bn - 1) / bn;
     plan->n_tiles = n_tiles;
     plan->num_tiles = m_tiles * n_tiles;
-    plan->grid = plan->num_tiles < num_sms ? plan->num_tiles : num_sms;
+    const int slots = num_sms / ctas;     // tiles in flight: one per CTA, or per cluster of two
+    plan->grid = ctas * (plan->num_tiles < slots ? plan->num_tiles : slots);
     // Inner tensor dimension rounded up to the 16-byte granule (columns [K, K8) are zero in A and in the packed weights by the
     // contract above): with K = 28 the 56-byte rows put the out-of-bounds edge in the middle of a 16-byte chunk and the TMA
     // unit takes a slow path — the 28 -> 960 layer ran 44.5 instead of 35.6 us (experiments/microbench/gemm_sweep.cu).
     const int Kt = ((d.K + 7) / 8 * 8 <= d.lda && (d.K + 7) / 8 * 8 <= d.ldw) ? (d.K + 7) / 8 * 8 : d.K;
     int r = make_tmap_bf16_2d(&plan->tmA, d.A, d.M, Kt, d.lda, kBM);
     if (r) return r;
-    r = make_tmap_bf16_2d(&plan->tmB, d.W, d.N, Kt, d.ldw, bn);
+    r = make_tmap_bf16_2d(&plan->tmB, d.W, d.N, Kt, d.ldw, box_n);
     if (r) return r;
     if (!d.out_f32) {
         // store map: columns [N, round_up(N, 8)) are part of the tensor and receive zeros
@@ -536,7 +596,7 @@ int tc_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms) {
     if (d.split) {
         r = make_tmap_bf16_2d(&plan->tmA_lo, d.A_lo, d.M, Kt, d.lda, kBM);
         if (r) return r;
-        r = make_tmap_bf16_2d(&plan->tmB_lo, d.W_lo, d.N, Kt, d.ldw, bn);
+        r = make_tmap_bf16_2d(&plan->tmB_lo, d.W_lo, d.N, Kt, d.ldw, box_n);
         if (r) return r;
     }
     if (d.out_split) r = make_tmap_bf16_2d_ex(&plan->tmC_lo, d.out_lo, d.M, (d.N + 7) / 8 * 8, d.ldc, 32, 32, 64);
@@ -545,7 +605,7 @@ int tc_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms) {
 
 cudaError_t tc_gemm_launch(const TcGemmPlan& plan, cudaStream_t stream) {
     const GemmDesc& d = plan.desc;
-    TcGemmArgs a;
+    TcGemmLnArgs a;
     a.M = d.M; a.N = d.N; a.K = d.K;
     a.block_n = plan.block_n;
     a.num_stages = plan.num_stages;
@@ -564,9 +624,9 @@ cudaError_t tc_gemm_launch(const TcGemmPlan& plan, cudaStream_t stream) {
     a.ln_out = static_cast<__nv_bfloat16*>(d.ln_out); a.ln_ld = d.ln_ld;
     a.split = d.split;
     switch (d.act) {
-        case ACT_NONE: return launch_act<ACT_NONE>(plan, a, stream);
-        case ACT_MISH: return launch_act<ACT_MISH>(plan, a, stream);
-        case ACT_GELU: return launch_act<ACT_GELU>(plan, a, stream);
+        case ACT_NONE: return plan.pair ? launch_act<ACT_NONE, true>(plan, a, stream) : launch_act<ACT_NONE, false>(plan, a, stream);
+        case ACT_MISH: return plan.pair ? launch_act<ACT_MISH, true>(plan, a, stream) : launch_act<ACT_MISH, false>(plan, a, stream);
+        case ACT_GELU: return plan.pair ? launch_act<ACT_GELU, true>(plan, a, stream) : launch_act<ACT_GELU, false>(plan, a, stream);
     }
     return cudaErrorInvalidValue;
 }

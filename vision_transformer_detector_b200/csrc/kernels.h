@@ -62,17 +62,15 @@ struct TcGemmPlan {
     int num_tiles = 0;
     int grid = 0;
     size_t smem_bytes = 0;
-    int pair = 0;              // 1: built for the CTA-pair kernel
+    int pair = 0;              // 1: built for the CTA-pair form
 };
 
 int choose_block_n(int N);
 int make_tmap_bf16_2d(CUtensorMap* map, const void* base, int rows, int cols, int ld, int box_rows);
 int make_tmap_bf16_2d_ex(CUtensorMap* map, const void* base, int rows, int cols, int ld, int box_cols, int box_rows, int swizzle_bytes);
-int tc_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms);
+// pair = 1: the CTA-pair (cta_group::2) form for the large layers, a 256 x BN tile per 2-CTA cluster (gemm_tc.cu).
+int tc_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms, int pair);
 cudaError_t tc_gemm_launch(const TcGemmPlan& plan, cudaStream_t stream);
-// CTA-pair (cta_group::2) variant for the large layers (gemm_tc2.cu): 256 x BN tile per 2-CTA cluster.
-int tc2_gemm_make_plan(TcGemmPlan* plan, const GemmDesc& d, int num_sms);
-cudaError_t tc2_gemm_launch(const TcGemmPlan& plan, cudaStream_t stream);
 
 // ------------------------------------------------------------------------------------------------
 // Fused tail of the encoder MLP pyramid (mlp_tail.cu): x += act(W2 act(W1 act(W0 A + b0) + b1) + b2) in place on the
@@ -124,16 +122,8 @@ struct AttnPlan {
 };
 int attn_bf16_make_plan(AttnPlan* plan, const AttnDesc& d);
 cudaError_t attn_tc_launch(const AttnPlan& plan, cudaStream_t stream);     // tcgen05 kernel, one softmax thread per query row (attention_tc.cu)
-#ifdef VITDET_EXPERIMENTS      // experiments/attention/: measured and dropped (profiles/r02_attention_analysis.md)
-cudaError_t attn_tc8_launch(const AttnPlan& plan, cudaStream_t stream);
-cudaError_t attn_tc3_launch(const AttnPlan& plan, cudaStream_t stream);
-cudaError_t attn_tcp_launch(const AttnPlan& plan, int num_sms, cudaStream_t stream);
-cudaError_t attn_tc8p_launch(const AttnPlan& plan, int num_sms, cudaStream_t stream);
-cudaError_t attn_pp_launch(const AttnPlan& plan, int num_sms, cudaStream_t stream);
-cudaError_t attn_sw_launch(const AttnPlan& plan, int num_sms, cudaStream_t stream);
-#endif
 cudaError_t attn_f32_launch(const AttnDesc& d, cudaStream_t stream);
-// fp32-accumulate mode on the tensor cores (attention_tcs.cu): plan.desc.qkv / ctx are the hi planes, tm_lo the tensor map
+// fp32-accumulate mode on the tensor cores (attention_tc.cu, split form): plan.desc.qkv / ctx are the hi planes, tm_lo the tensor map
 // of the lo plane of qkv (same shape and pitch), ctx_lo the lo plane of the context rows.
 cudaError_t attn_tcs_launch(const AttnPlan& plan, const CUtensorMap& tm_lo, void* ctx_lo, cudaStream_t stream);
 
