@@ -254,6 +254,30 @@ int vitdet_submit_host(vitdet_handle* h, const void* images_host, int images_are
                        const vitdet_decode_params* params, int want_packed, void* stream, int* ticket);
 int vitdet_collect(vitdet_handle* h, int ticket, float* logits_host, const vitdet_detections* out_host);
 
+/* ---- decoded images of any size ("next" row N4: _get_image_tensor_coco, vision_transformer_utilities.py:418-449) ----
+ * Each image is letterboxed to the model's input size (tf.image.resize_with_pad, bilinear; clip; / 127.5 - 1) inside the
+ * patch kernel, so the float32 image never exists.  Results are bit-identical to preprocessing every image with
+ * vitdet_preprocess_image and running vitdet_forward_decode on the stacked batch.  params->image_h / image_w are the decode
+ * size as elsewhere; boxes_original, when requested, needs them equal to the model's input size.
+ * boxes_original [B * num_slots, 4] f32: x0, y0, x1, y1 of every slot's box on its source image, in source pixels,
+ *   x0 = (cx - w/2 - pad_left) * (width / resized_width) (likewise x1, y0, y1; float32, in this order), clipped to
+ *   [0, width] / [0, height]; computed for every slot whatever `keep` says.
+ * An image list with a null pixel pointer, a non-positive size or a size that resizes to zero rows or columns (e.g.
+ * 1 x 2000 into 608 x 608) fails with VITDET_E_INVALID, naming the image, before anything is launched. */
+typedef struct vitdet_image {
+    const uint8_t* pixels;             /* [height, width, 3] RGB, dense rows */
+    int32_t height, width;
+} vitdet_image;
+/* images: HOST array of B descriptors whose pixels are DEVICE pointers; outputs as vitdet_forward_u8, plus
+ * boxes_original_dev (DEVICE, may be NULL).  Asynchronous on `stream`. */
+int vitdet_forward_images(vitdet_handle* h, const vitdet_image* images, int B, int mode, const vitdet_decode_params* params,
+                          float* logits_dev, const vitdet_detections* out, float* boxes_original_dev, void* stream);
+/* images: HOST descriptors of HOST pixels (page-locked pixels are read directly when every image is page-locked; otherwise
+ * they are staged); the same submission slots as vitdet_submit_host, completed by vitdet_collect, which also fills
+ * boxes_original_host (HOST, may be NULL) if given here. */
+int vitdet_submit_images_host(vitdet_handle* h, const vitdet_image* images, int B, int mode, const vitdet_decode_params* params,
+                              int want_packed, float* boxes_original_host, void* stream, int* ticket);
+
 /* ---- evaluation metric ("next" row N2): MeanAveragePrecision of the reference (det.py:1268-2060) ----
  * The COCO-style AP of the reference: mean over the IoU thresholds tf.linspace(0.5, 0.95, 10) of the mean, over the
  * classes seen so far, of the class AP computed from the latest `latest_related_images` related images per class

@@ -67,6 +67,11 @@ class Detections(C.Structure):
     ]
 
 
+class Image(C.Structure):
+    """struct vitdet_image — one uint8 (height, width, 3) image of a ragged batch (device or host pixels)."""
+    _fields_ = [("pixels", C.c_void_p), ("height", C.c_int32), ("width", C.c_int32)]
+
+
 # every symbol include/vitdet_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -119,6 +124,9 @@ SYMBOLS = {
     "vitdet_op_head_slots": (C.c_int, [_P, _P, _P, _P, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, _P]),
     "vitdet_submit_host": (C.c_int, [_P, _P, C.c_int, C.c_int, C.c_int, C.POINTER(DecodeParams), C.c_int, _P, C.POINTER(C.c_int)]),
     "vitdet_collect": (C.c_int, [_P, C.c_int, _P, C.POINTER(Detections)]),
+    "vitdet_forward_images": (C.c_int, [_P, C.POINTER(Image), C.c_int, C.c_int, C.POINTER(DecodeParams), _P, C.POINTER(Detections), _P, _P]),
+    "vitdet_submit_images_host": (C.c_int, [_P, C.POINTER(Image), C.c_int, C.c_int, C.POINTER(DecodeParams), C.c_int, _P, _P,
+                                            C.POINTER(C.c_int)]),
     "vitdet_gather_detections": (C.c_int, [_P, _P, C.c_int, _P, _P]),
     "vitdet_nccl_unique_id": (C.c_int, [C.c_char_p]),
     "vitdet_nccl_comm_create": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.POINTER(_P)]),

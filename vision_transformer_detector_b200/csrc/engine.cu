@@ -271,12 +271,15 @@ public:
         cv_.notify_all();
         for (auto& t : threads_) t.join();
     }
-    // dst[0, bytes) = src[0, bytes), split over the workers and the calling thread; returns when all of it is done
-    void copy(char* dst, const char* src, size_t bytes) {
+    // Concatenates n pieces into dst: piece k, srcs[k][0, offs[k + 1] - offs[k]), goes to dst + offs[k] - offs[0].  The
+    // bytes are split over the workers and the calling thread; returns when all of it is done.
+    void copy(char* dst, const char* const* srcs, const size_t* offs, int n) {
         const int parts = static_cast<int>(threads_.size()) + 1;
-        if (parts == 1 || bytes < (1u << 20)) { memcpy(dst, src, bytes); return; }
-        const size_t per = ((bytes + parts - 1) / parts + 4095) & ~static_cast<size_t>(4095);
-        { std::lock_guard<std::mutex> g(m_); dst_ = dst; src_ = src; bytes_ = bytes; per_ = per; pending_ = parts - 1; ++gen_; }
+        const size_t bytes = offs[n] - offs[0];
+        const size_t per = parts == 1 || bytes < (1u << 20) ? bytes : ((bytes + parts - 1) / parts + 4095) & ~static_cast<size_t>(4095);
+        { std::lock_guard<std::mutex> g(m_); dst_ = dst; srcs_ = srcs; offs_ = offs; n_ = n; per_ = per; }
+        if (per == bytes) { slice(0); return; }
+        { std::lock_guard<std::mutex> g(m_); pending_ = parts - 1; ++gen_; }
         cv_.notify_all();
         slice(parts - 1);
         std::unique_lock<std::mutex> lk(m_);
@@ -284,8 +287,11 @@ public:
     }
 private:
     void slice(int i) {
-        const size_t lo = per_ * static_cast<size_t>(i);
-        if (lo < bytes_) memcpy(dst_ + lo, src_ + lo, (bytes_ - lo) < per_ ? (bytes_ - lo) : per_);
+        const size_t lo = offs_[0] + per_ * static_cast<size_t>(i), hi = std::min(lo + per_, offs_[n_]);
+        for (int k = 0; k < n_ && lo < hi; ++k) {
+            const size_t a = std::max(lo, offs_[k]), b = std::min(hi, offs_[k + 1]);
+            if (a < b) memcpy(dst_ + (a - offs_[0]), srcs_[k] + (a - offs_[k]), b - a);
+        }
     }
     void run(int i) {
         unsigned long long seen = 0;
@@ -300,24 +306,28 @@ private:
     std::condition_variable cv_, done_;
     unsigned long long gen_ = 0;
     bool stop_ = false;
-    char* dst_ = nullptr; const char* src_ = nullptr; size_t bytes_ = 0, per_ = 0;
+    char* dst_ = nullptr; const char* const* srcs_ = nullptr; const size_t* offs_ = nullptr; int n_ = 0; size_t per_ = 0;
     int pending_ = 0;
 };
 
 // One in-flight host submission (vitdet_submit_host .. vitdet_collect): its own pinned staging, device input and
-// record block, so that the H2D copy of submission i+1 overlaps the compute of submission i.
+// record block, so that the H2D copy of submission i+1 overlaps the compute of submission i.  A submission of separate
+// images (vitdet_submit_images_host) also owns its letterbox table, copied to dev_table on the compute stream.
 struct HostSlot {
     void* pin_in = nullptr; size_t pin_in_bytes = 0;
     void* pin_out = nullptr; size_t pin_out_bytes = 0;
-    DevBuf dev_in, dev_out;
+    LetterboxImage* pin_table = nullptr; size_t pin_table_bytes = 0;
+    DevBuf dev_in, dev_out, dev_table;
     std::vector<cudaEvent_t> copy_events;      // one per staged sub-chunk of images
     cudaEvent_t done = nullptr;                // recorded after the D2H copy of the record block
     bool busy = false;
-    size_t R = 0, o_dec = 0, o_id = 0, o_cc = 0, o_cor = 0, o_keep = 0, o_pk = 0;
+    size_t R = 0, o_dec = 0, o_id = 0, o_cc = 0, o_cor = 0, o_keep = 0, o_pk = 0, o_box = 0;
     bool has_packed = false;
+    float* boxes_host = nullptr;               // where vitdet_collect puts boxes_original, or null
     ~HostSlot() {
         if (pin_in) cudaFreeHost(pin_in);
         if (pin_out) cudaFreeHost(pin_out);
+        if (pin_table) cudaFreeHost(pin_table);
         for (auto e : copy_events) cudaEventDestroy(e);
         if (done) cudaEventDestroy(done);
     }
@@ -392,6 +402,7 @@ struct vitdet_handle {
     HostSlot host_slots[kHostSlots];
     int next_slot = 0;
     StagePool* stage_pool = nullptr;             // created on the first pageable submission
+    DevBuf images_table;                         // letterbox table of vitdet_forward_images, written in stream order
 
     ~vitdet_handle() {
         for (auto& r : prof_pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
@@ -839,6 +850,9 @@ struct ForwardOpts {
     const cudaEvent_t* ready = nullptr;
     int ready_gran = 0;
     int in_u8 = 0;                    // images are uint8 pixels; the patch kernel normalises them (x / 127.5 - 1)
+    // images is a DEVICE table of B LetterboxImage entries: uint8 images of any size, letterboxed inside the patch kernel
+    int letterbox = 0;
+    float* boxes_original = nullptr;  // with letterbox: [B * S, 4] boxes on the source images
 };
 
 // vitdet_decode_params / vitdet_detections -> the decode kernels' arguments (either may be null: defaults / no outputs)
@@ -957,10 +971,16 @@ static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, f
         const int Mc = bc * T;
         float* x = h->x.as<float>() + static_cast<size_t>(c0) * T * m.D4;
         PlanCursor pc = plan_cursor(h, kEncoderPlans, f, bc);
-        const char* img = static_cast<const char*>(images) + static_cast<size_t>(c0) * c.image_h * c.image_w * 3 * (opts.in_u8 ? 1 : 4);
         const Rows pr = rows_out(h->patch, h->tmp32, h->PK);
-        { ProfScope ps(h, PC_PATCHIFY, st);
-        CU_TRY(patchify_launch(img, opts.in_u8, bc, c.image_h, c.image_w, c.patch_size, pr.p, pr.ld, h->RP, pr.f32, st)); }
+        if (opts.letterbox) {
+            ProfScope ps(h, PC_PATCHIFY, st);
+            CU_TRY(letterbox_patchify_launch(static_cast<const LetterboxImage*>(images) + c0, bc, c.image_h, c.image_w, c.patch_size,
+                                             pr.p, pr.ld, h->RP, pr.f32, st));
+        } else {
+            const char* img = static_cast<const char*>(images) + static_cast<size_t>(c0) * c.image_h * c.image_w * 3 * (opts.in_u8 ? 1 : 4);
+            ProfScope ps(h, PC_PATCHIFY, st);
+            CU_TRY(patchify_launch(img, opts.in_u8, bc, c.image_h, c.image_w, c.patch_size, pr.p, pr.ld, h->RP, pr.f32, st));
+        }
         Operand a;
         RC_TRY(operand(pr, h->patch, Mc, h->PK, &a));
         DenseCall pj{a, &h->proj, Mc};
@@ -1057,6 +1077,11 @@ static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, f
     DecodeParams dp;
     DecodeOut dout;
     decode_args(dpar, 1 /*the head emits raw logits*/, det, logits, &dp, &dout);
+    if (opts.letterbox && opts.boxes_original) {
+        dout.boxes_original = opts.boxes_original;
+        dout.letterbox = static_cast<const LetterboxImage*>(images);
+        dout.slots = h->S;
+    }
     const int in_f32 = f != Form::Bf16;
     h->head_last = a.p; h->head_last_ld = a.ld; h->head_last_f32 = in_f32;
     ProfScope ps(h, PC_HEAD_TAIL, st);
@@ -1411,22 +1436,40 @@ int vitdet_decode_host(const float* logits_host, int R, const vitdet_decode_para
 
 }  // extern "C"
 
-static int submit_host_impl(vitdet_handle* h, const void* images_host, int in_u8, int B, int mode, const vitdet_decode_params* params,
-                            int want_packed, void* stream, int* ticket) {
-    if (!h || !images_host || B <= 0 || !params || !ticket) return fail(VITDET_E_INVALID, "submit_host: bad arguments");
+static bool page_locked(const void* p) {
+    cudaPointerAttributes attr;
+    const bool pinned = cudaPointerGetAttributes(&attr, p) == cudaSuccess && attr.type == cudaMemoryTypeHost;
+    cudaGetLastError();
+    return pinned;
+}
+
+// The images of one host submission: image i, src[i][0, offs[i + 1] - offs[i]), goes to byte offs[i] of the slot's device
+// input.  `table` (separate images of any size) holds their letterbox geometry; its pixel pointers are filled in here.
+// Without it the images are one contiguous array of the model's size.
+struct HostImages {
+    std::vector<const char*> src;
+    std::vector<size_t> offs;
+    std::vector<LetterboxImage> table;
+};
+
+static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, int mode, const vitdet_decode_params* params,
+                            int want_packed, float* boxes_host, void* stream, int* ticket) {
     HostSlot& sl = h->host_slots[h->next_slot];
     if (sl.busy) return fail(VITDET_E_INVALID, "submit_host: %d submissions are in flight; collect one first", vitdet_handle::kHostSlots);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const size_t in_bytes = static_cast<size_t>(B) * h->cfg.image_h * h->cfg.image_w * 3 * (in_u8 ? 1 : 4);
+    const bool separate = !in.table.empty();
+    const size_t in_bytes = in.offs[B];
     const size_t R = static_cast<size_t>(B) * h->S;
-    // output record block: logits 24 | decoded 24 | class_id 4 | class_conf 4 | corners 16 | keep 1 | packed 52  bytes per row
-    sl.R = R; sl.has_packed = want_packed != 0;
+    // output record block: logits 24 | decoded 24 | class_id 4 | class_conf 4 | corners 16 | keep 1 | packed 52 | boxes_original 16
+    // bytes per row
+    sl.R = R; sl.has_packed = want_packed != 0; sl.boxes_host = boxes_host;
     sl.o_dec = a256(R * 24); sl.o_id = sl.o_dec + a256(R * 24); sl.o_cc = sl.o_id + a256(R * 4); sl.o_cor = sl.o_cc + a256(R * 4);
     sl.o_keep = sl.o_cor + a256(R * 16); sl.o_pk = sl.o_keep + a256(R);
-    const size_t out_bytes = sl.o_pk + (want_packed ? a256(R * 52) : 0);
-    cudaPointerAttributes attr;
-    const bool pinned = cudaPointerGetAttributes(&attr, images_host) == cudaSuccess && attr.type == cudaMemoryTypeHost;
-    cudaGetLastError();
+    sl.o_box = sl.o_pk + (want_packed ? a256(R * 52) : 0);
+    const size_t out_bytes = sl.o_box + (boxes_host ? a256(R * 16) : 0);
+    // a page-locked source is read directly, otherwise the whole submission is staged
+    bool pinned = page_locked(in.src[0]);
+    for (int i = 1; separate && pinned && i < B; ++i) pinned = page_locked(in.src[i]);
     if (!pinned && sl.pin_in_bytes < in_bytes) {
         if (sl.pin_in) cudaFreeHost(sl.pin_in);
         sl.pin_in = nullptr; sl.pin_in_bytes = 0;
@@ -1479,17 +1522,19 @@ static int submit_host_impl(vitdet_handle* h, const void* images_host, int in_u8
         if (workers < 0) workers = 0;
         h->stage_pool = new StagePool(workers);
     }
-    const size_t img_bytes = in_bytes / static_cast<size_t>(B);
+    char* dev_in = sl.dev_in.as<char>();
     for (int i = 0; i < n_sub; ++i) {
-        const size_t off = static_cast<size_t>(i) * kGran * img_bytes;
-        const int cnt = (B - i * kGran) < kGran ? (B - i * kGran) : kGran;
-        const size_t bytes = static_cast<size_t>(cnt) * img_bytes;
-        const char* src = reinterpret_cast<const char*>(images_host) + off;
+        const int i0 = i * kGran, i1 = std::min(B, i0 + kGran);
+        const size_t off = in.offs[i0], bytes = in.offs[i1] - off;
         if (!pinned) {
-            h->stage_pool->copy(static_cast<char*>(sl.pin_in) + off, src, bytes);
-            src = static_cast<const char*>(sl.pin_in) + off;
+            h->stage_pool->copy(static_cast<char*>(sl.pin_in) + off, in.src.data() + i0, in.offs.data() + i0, i1 - i0);
+            CU_TRY(cudaMemcpyAsync(dev_in + off, static_cast<const char*>(sl.pin_in) + off, bytes, cudaMemcpyHostToDevice, h->copy_stream));
+        } else if (!separate) {
+            CU_TRY(cudaMemcpyAsync(dev_in + off, in.src[i0], bytes, cudaMemcpyHostToDevice, h->copy_stream));
+        } else {
+            for (int k = i0; k < i1; ++k)
+                CU_TRY(cudaMemcpyAsync(dev_in + in.offs[k], in.src[k], in.offs[k + 1] - in.offs[k], cudaMemcpyHostToDevice, h->copy_stream));
         }
-        CU_TRY(cudaMemcpyAsync(sl.dev_in.as<char>() + off, src, bytes, cudaMemcpyHostToDevice, h->copy_stream));
         CU_TRY(cudaEventRecord(sl.copy_events[i], h->copy_stream));
     }
     ForwardOpts opts;
@@ -1498,6 +1543,26 @@ static int submit_host_impl(vitdet_handle* h, const void* images_host, int in_u8
     opts.ready = sl.copy_events.data();
     opts.ready_gran = kGran;
     opts.in_u8 = in_u8;
+    const void* images_dev = dev_in;
+    if (separate) {
+        // the slot's own table: the pinned copy is not touched again before this submission is collected
+        const size_t table_bytes = static_cast<size_t>(B) * sizeof(LetterboxImage);
+        if (sl.pin_table_bytes < table_bytes) {
+            if (sl.pin_table) cudaFreeHost(sl.pin_table);
+            sl.pin_table = nullptr; sl.pin_table_bytes = 0;
+            CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&sl.pin_table), table_bytes, cudaHostAllocDefault));
+            sl.pin_table_bytes = table_bytes;
+        }
+        RC_TRY(sl.dev_table.ensure(table_bytes));
+        for (int k = 0; k < B; ++k) {
+            sl.pin_table[k] = in.table[k];
+            sl.pin_table[k].pixels = reinterpret_cast<const uint8_t*>(dev_in + in.offs[k]);
+        }
+        CU_TRY(cudaMemcpyAsync(sl.dev_table.p, sl.pin_table, table_bytes, cudaMemcpyHostToDevice, st));
+        opts.letterbox = 1;
+        opts.boxes_original = boxes_host ? reinterpret_cast<float*>(sl.dev_out.as<char>() + sl.o_box) : nullptr;
+        images_dev = sl.dev_table.p;
+    }
     char* dbase = sl.dev_out.as<char>();
     vitdet_detections d = {};
     d.decoded = reinterpret_cast<float*>(dbase + sl.o_dec);
@@ -1506,7 +1571,7 @@ static int submit_host_impl(vitdet_handle* h, const void* images_host, int in_u8
     d.corners = reinterpret_cast<int32_t*>(dbase + sl.o_cor);
     d.keep = reinterpret_cast<uint8_t*>(dbase + sl.o_keep);
     if (want_packed) d.packed = reinterpret_cast<float*>(dbase + sl.o_pk);
-    RC_TRY(forward_impl(h, sl.dev_in.p, B, mode, reinterpret_cast<float*>(dbase), params, &d, st, opts));
+    RC_TRY(forward_impl(h, images_dev, B, mode, reinterpret_cast<float*>(dbase), params, &d, st, opts));
     CU_TRY(cudaMemcpyAsync(sl.pin_out, dbase, out_bytes, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaEventRecord(sl.done, st));
     sl.busy = true;
@@ -1535,14 +1600,50 @@ static int collect_impl(vitdet_handle* h, int ticket, float* logits_host, const 
             memcpy(out_host->packed, pb + sl.o_pk, R * 52);
         }
     }
+    if (sl.boxes_host) memcpy(sl.boxes_host, pb + sl.o_box, R * 16);
     return 0;
+}
+
+// A contiguous host array of B images of the model's size
+static int submit_dense_impl(vitdet_handle* h, const void* images_host, int in_u8, int B, int mode, const vitdet_decode_params* params,
+                             int want_packed, void* stream, int* ticket) {
+    if (!h || !images_host || B <= 0 || !params || !ticket) return fail(VITDET_E_INVALID, "submit_host: bad arguments");
+    const size_t img_bytes = static_cast<size_t>(h->cfg.image_h) * h->cfg.image_w * 3 * (in_u8 ? 1 : 4);
+    HostImages in;
+    in.src.resize(B);
+    in.offs.resize(B + 1);
+    for (int i = 0; i <= B; ++i) {
+        in.offs[i] = static_cast<size_t>(i) * img_bytes;
+        if (i < B) in.src[i] = static_cast<const char*>(images_host) + in.offs[i];
+    }
+    return submit_host_impl(h, in, in_u8, B, mode, params, want_packed, nullptr, stream, ticket);
 }
 
 static int predict_host_impl(vitdet_handle* h, const void* images_host, int in_u8, int B, int mode, const vitdet_decode_params* params,
                              float* logits_host, const vitdet_detections* out_host, void* stream) {
     int ticket = -1;
-    RC_TRY(submit_host_impl(h, images_host, in_u8, B, mode, params, (out_host && out_host->packed) ? 1 : 0, stream, &ticket));
+    RC_TRY(submit_dense_impl(h, images_host, in_u8, B, mode, params, (out_host && out_host->packed) ? 1 : 0, stream, &ticket));
     return collect_impl(h, ticket, logits_host, out_host);
+}
+
+// Checks a caller's list of separate images and fills their letterbox table (pixel pointers as given); the message of a
+// rejected list names the first bad image.  boxes: boxes_original is requested, which needs the decode at the model's size.
+static int images_table(const vitdet_handle* h, const char* fn, const vitdet_image* images, int B, const vitdet_decode_params* params,
+                        bool boxes, std::vector<LetterboxImage>* table) {
+    if (!h || !images || B <= 0) return fail(VITDET_E_INVALID, "%s: %s", fn, !h ? "null handle" : (!images ? "images is null" : "B must be positive"));
+    const int th = h->cfg.image_h, tw = h->cfg.image_w;
+    if (boxes && (!params || params->image_h != static_cast<float>(th) || params->image_w != static_cast<float>(tw)))
+        return fail(VITDET_E_INVALID, "%s: boxes_original needs the decode at the model's input size %d x %d (params image_h / image_w)", fn, th, tw);
+    table->resize(B);
+    for (int i = 0; i < B; ++i) {
+        const vitdet_image& im = images[i];
+        if (!im.pixels) return fail(VITDET_E_INVALID, "%s: image %d: null pixel pointer", fn, i);
+        if (im.height <= 0 || im.width <= 0) return fail(VITDET_E_INVALID, "%s: image %d: size %d x %d is not positive", fn, i, im.height, im.width);
+        if (!letterbox_image(im.pixels, im.height, im.width, th, tw, &(*table)[i]))
+            return fail(VITDET_E_INVALID, "%s: image %d: a %d x %d image letterboxed to %d x %d resizes to %d x %d pixels", fn, i, im.height,
+                        im.width, th, tw, (*table)[i].rh, (*table)[i].rw);
+    }
+    return 0;
 }
 
 extern "C" {
@@ -1559,11 +1660,44 @@ int vitdet_predict_host_u8(vitdet_handle* h, const uint8_t* images_host, int B, 
 
 int vitdet_submit_host(vitdet_handle* h, const void* images_host, int images_are_uint8, int B, int mode, const vitdet_decode_params* params,
                        int want_packed, void* stream, int* ticket) {
-    return submit_host_impl(h, images_host, images_are_uint8 ? 1 : 0, B, mode, params, want_packed, stream, ticket);
+    return submit_dense_impl(h, images_host, images_are_uint8 ? 1 : 0, B, mode, params, want_packed, stream, ticket);
 }
 
 int vitdet_collect(vitdet_handle* h, int ticket, float* logits_host, const vitdet_detections* out_host) {
     return collect_impl(h, ticket, logits_host, out_host);
+}
+
+int vitdet_forward_images(vitdet_handle* h, const vitdet_image* images, int B, int mode, const vitdet_decode_params* params,
+                          float* logits_dev, const vitdet_detections* out, float* boxes_original_dev, void* stream) {
+    if (!logits_dev && !(params && out)) return fail(VITDET_E_INVALID, "forward_images: neither logits_dev nor (params, out) given");
+    if ((params == nullptr) != (out == nullptr)) return fail(VITDET_E_INVALID, "forward_images: params and out go together");
+    std::vector<LetterboxImage> table;
+    RC_TRY(images_table(h, "forward_images", images, B, params, boxes_original_dev != nullptr, &table));
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // a pageable source: the copy has taken the table by the time it returns, and it reaches the device in stream order
+    const size_t table_bytes = table.size() * sizeof(LetterboxImage);
+    RC_TRY(h->images_table.ensure(table_bytes));
+    CU_TRY(cudaMemcpyAsync(h->images_table.p, table.data(), table_bytes, cudaMemcpyHostToDevice, st));
+    ForwardOpts opts;
+    opts.in_u8 = 1;
+    opts.letterbox = 1;
+    opts.boxes_original = boxes_original_dev;
+    return forward_impl(h, h->images_table.p, B, mode, logits_dev, params, out, st, opts);
+}
+
+int vitdet_submit_images_host(vitdet_handle* h, const vitdet_image* images, int B, int mode, const vitdet_decode_params* params,
+                              int want_packed, float* boxes_original_host, void* stream, int* ticket) {
+    if (!params || !ticket) return fail(VITDET_E_INVALID, "submit_images_host: params and ticket must not be null");
+    HostImages in;
+    RC_TRY(images_table(h, "submit_images_host", images, B, params, boxes_original_host != nullptr, &in.table));
+    in.src.resize(B);
+    in.offs.resize(B + 1);
+    in.offs[0] = 0;
+    for (int i = 0; i < B; ++i) {
+        in.src[i] = reinterpret_cast<const char*>(images[i].pixels);
+        in.offs[i + 1] = in.offs[i] + static_cast<size_t>(images[i].height) * images[i].width * 3;
+    }
+    return submit_host_impl(h, in, 1, B, mode, params, want_packed, boxes_original_host, stream, ticket);
 }
 
 // ------------------------------------------------------------------------------------------------

@@ -136,6 +136,21 @@ cudaError_t attn_tcs_launch(const AttnPlan& plan, const CUtensorMap& tm_lo, void
 cudaError_t patchify_launch(const void* images, int in_u8 /*1: uint8 pixels, normalised x/127.5-1 on the fly*/, int B, int H, int W, int p,
                             void* patches, int ldp, int rp, int out_f32, cudaStream_t stream);
 
+// One uint8 HWC source image of a ragged batch and how tf.image.resize_with_pad maps it onto the model's input
+// (vision_transformer_utilities.py:435-447): resized to rh x rw, placed at (ph, pw) between bars.
+struct LetterboxImage {
+    const uint8_t* pixels;     // [h, w, 3], dense rows
+    int h, w;
+    int rh, rw, ph, pw;        // resize_with_pad_geometry
+    float hscale, wscale;      // h / rh, w / rw in float32
+};
+// Fills *im for an h x w image letterboxed to th x tw; false when a size is not positive or the resized image is empty.
+bool letterbox_image(const uint8_t* pixels, int h, int w, int th, int tw, LetterboxImage* im);
+// patchify of the letterboxed, normalised images without the float32 images: images is a DEVICE table of B entries,
+// the output the same patch matrix as patchify_launch's (vector layout only: rp and ldp multiples of 4, 16-byte aligned).
+cudaError_t letterbox_patchify_launch(const LetterboxImage* images, int B, int H, int W, int p, void* patches, int ldp, int rp,
+                                      int out_f32, cudaStream_t stream);
+
 // keras LayerNormalization(axis=-1), eps=1e-3, biased variance (det.py:353-357, 375-379).
 cudaError_t layernorm_launch(const float* x, int ldx, const float* gamma, const float* beta, int M, int D,
                              float eps, void* y, int ldy, int out_f32, cudaStream_t stream);
@@ -164,6 +179,10 @@ struct DecodeOut {
     uint8_t* keep = nullptr;    // [R]
     int32_t* corners = nullptr; // [R, 4] x0, y0, x1, y1 (int truncation then clip; det.py:2300-2325), optional
     float* packed = nullptr;    // [R, 13] decoded[6] | class id | class confidence | keep | corners[4], all as float32 (the gather record)
+    // [R, 4] x0, y0, x1, y1 on the source image of row r, letterbox[r / slots] (letterboxed input only), optional
+    float* boxes_original = nullptr;
+    const LetterboxImage* letterbox = nullptr;
+    int slots = 0;
 };
 cudaError_t head_tail_launch(const void* h, int ldh, int in_f32, const float* w /*[6, U] f32*/, const float* bias,
                              int R, int U, const DecodeParams& dp, const DecodeOut& out, cudaStream_t stream);

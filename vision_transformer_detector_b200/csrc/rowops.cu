@@ -156,6 +156,107 @@ patchify_kernel(const IN* __restrict__ img, int H, int W, int p, int gh, int gw,
 }
 
 // ------------------------------------------------------------------------------------------------
+// Input side ("next" row N4): _get_image_tensor_coco of the reference (vision_transformer_utilities.py:418-449) after
+// the file decode: tf.image.resize_with_pad(image, H, W) (bilinear, half-pixel centres, no antialias, zero padding),
+// tf.clip_by_value(0, 255), / 127.5, - 1.  The interpolation follows TF's resize_bilinear CPU kernel term by term, without
+// FMA contraction.  preprocess_kernel and letterbox_patchify_kernel both evaluate a pixel with the two functions below,
+// so the letterboxed patch matrix equals patchify of preprocess_kernel's image bit for bit.
+// ------------------------------------------------------------------------------------------------
+// Value of a letterbox bar pixel: the zero padding of resize_with_pad after clip, / 127.5, - 1.
+constexpr float kLetterboxBar = -1.f;
+
+// Taps of resized coordinate i along one axis: in = (i + 0.5) * scale - 0.5; lower = max(floor(in), 0);
+// upper = min(ceil(in), size - 1); lerp = in - floor(in).
+struct ResizeTap { int lo, hi; float lerp; };
+__device__ __forceinline__ ResizeTap resize_tap(int i, float scale, int size) {
+    const float in = __fsub_rn(__fmul_rn(__fadd_rn(static_cast<float>(i), 0.5f), scale), 0.5f);
+    const float f = floorf(in);
+    return ResizeTap{max(static_cast<int>(f), 0), min(static_cast<int>(ceilf(in)), size - 1), __fsub_rn(in, f)};
+}
+
+// One channel of one resized pixel: r0 / r1 are the source rows of the y taps, x0 / x1 the byte offsets of the channel
+// at the x taps.  Top and bottom lerp in x, then in y; clip to [0, 255]; / 127.5 - 1.
+__device__ __forceinline__ float letterbox_value(const uint8_t* __restrict__ r0, const uint8_t* __restrict__ r1, int x0, int x1,
+                                                 float lx, float ly) {
+    const float tl = __ldg(r0 + x0), tr = __ldg(r0 + x1), bl = __ldg(r1 + x0), br = __ldg(r1 + x1);
+    const float top = __fadd_rn(tl, __fmul_rn(__fsub_rn(tr, tl), lx));
+    const float bot = __fadd_rn(bl, __fmul_rn(__fsub_rn(br, bl), lx));
+    float v = __fadd_rn(top, __fmul_rn(__fsub_rn(bot, top), ly));
+    v = fminf(fmaxf(v, 0.f), 255.f);
+    return __fsub_rn(__fdiv_rn(v, 127.5f), 1.f);
+}
+
+// K1 for a ragged batch of uint8 images: resize_with_pad to the model's H x W fused into patchify (same output layout
+// and work decomposition as the vector form above), so the float32 letterboxed image never exists.  Patch element
+// (y, x, c) of the model image is 0 outside it (extract_patches' SAME padding), kLetterboxBar in resize_with_pad's bars,
+// and the resized pixel otherwise.  images[b] describes image b of the launch.
+// A lane's 4 elements keep their x taps across the patch rows; each row costs one y tap and 16 byte gathers per lane,
+// which L1 serves (a 640 x 480 source is 0.9 MB against the 4.4 MB float32 image patchify reads).
+#ifndef VITDET_LETTERBOX_UNROLL
+#define VITDET_LETTERBOX_UNROLL 4
+#endif
+constexpr int kLetterboxRowUnroll = VITDET_LETTERBOX_UNROLL;
+
+template <typename T>
+__global__ void __launch_bounds__(256)
+letterbox_patchify_kernel(const LetterboxImage* __restrict__ images, int H, int W, int p, int gh, int gw, int pad_top,
+                          int pad_left, T* __restrict__ out, int ldp, int rp) {
+    pdl_launch_dependents();
+    pdl_wait();
+    const int py = blockIdx.x;
+    const int b = blockIdx.y;
+    const LetterboxImage im = images[b];
+    const int run = 3 * p, gpr = rp >> 2;
+    const size_t tok0 = (static_cast<size_t>(b) * gh + py) * gw;
+    const size_t src_pitch = static_cast<size_t>(im.w) * 3;
+    const int y_first = py * p - pad_top;
+    enum { kPad = 0, kBar = 1, kPixel = 2 };
+    const int items = gw * gpr;
+    for (int idx = threadIdx.x; idx < items; idx += 256) {
+        const int px = idx / gpr, q = idx - px * gpr;
+        const int w = 4 * q;
+        T* dst_tok = out + (tok0 + px) * ldp + w;
+        int kind[4], xa[4], xb[4];
+        float lx[4];
+#pragma unroll
+        for (int j = 0; j < 4; ++j) {
+            const int e = w + j, pix = e / 3, ch = e - 3 * pix;
+            const int x = px * p + pix - pad_left, rx = x - im.pw;
+            kind[j] = (e >= run || x < 0 || x >= W) ? kPad : ((rx < 0 || rx >= im.rw) ? kBar : kPixel);
+            const ResizeTap t = resize_tap(kind[j] == kPixel ? rx : 0, im.wscale, im.w);
+            xa[j] = 3 * t.lo + ch; xb[j] = 3 * t.hi + ch; lx[j] = t.lerp;
+        }
+        for (int r0 = 0; r0 < p; r0 += kLetterboxRowUnroll) {
+            float v[kLetterboxRowUnroll][4];
+#pragma unroll
+            for (int u = 0; u < kLetterboxRowUnroll; ++u) {
+                const int y = y_first + r0 + u, ry = y - im.ph;
+                const bool y_ok = (r0 + u < p) && y >= 0 && y < H;
+                const bool in_rows = y_ok && ry >= 0 && ry < im.rh;
+                const ResizeTap t = resize_tap(in_rows ? ry : 0, im.hscale, im.h);
+                const uint8_t* row0 = im.pixels + static_cast<size_t>(t.lo) * src_pitch;
+                const uint8_t* row1 = im.pixels + static_cast<size_t>(t.hi) * src_pitch;
+#pragma unroll
+                for (int j = 0; j < 4; ++j) {
+                    if (!y_ok || kind[j] == kPad) v[u][j] = 0.f;
+                    else if (!in_rows || kind[j] == kBar) v[u][j] = kLetterboxBar;
+                    else v[u][j] = letterbox_value(row0, row1, xa[j], xb[j], lx[j], t.lerp);
+                }
+            }
+#pragma unroll
+            for (int u = 0; u < kLetterboxRowUnroll; ++u)
+                if (r0 + u < p) Vec4Store<T>::st(dst_tok + (r0 + u) * rp, v[u][0], v[u][1], v[u][2], v[u][3]);
+        }
+    }
+    const int P = rp * p;
+    if (ldp > P) {
+        const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, padw = ldp - P;
+        for (int px = warp; px < gw; px += 8)
+            for (int w = lane; w < padw; w += 32) OutT<T>::st(out + (tok0 + px) * ldp + P + w, 0.f);
+    }
+}
+
+// ------------------------------------------------------------------------------------------------
 // K3 LayerNorm over the last axis, eps inside the rsqrt, biased variance, f32 statistics
 // (keras.layers.LayerNormalization defaults; det.py:353-357, 375-379).
 // LPR lanes cooperate on one row (8 for the 28-wide default stream: four rows per warp, each lane
@@ -386,6 +487,18 @@ __device__ __forceinline__ void decode_slot(const float (&l)[6], long long r, co
             pk[9] = static_cast<float>(c0); pk[10] = static_cast<float>(c1); pk[11] = static_cast<float>(c2); pk[12] = static_cast<float>(c3);
         }
     }
+    if (o.boxes_original) {
+        // the box on the source image: undo resize_with_pad (remove the bar, scale by source size / resized size), then clip
+        const LetterboxImage& g = o.letterbox[r / o.slots];
+        const float half_h = __fdiv_rn(dec[4], 2.f), half_w = __fdiv_rn(dec[5], 2.f);
+        const float pw = static_cast<float>(g.pw), ph = static_cast<float>(g.ph);
+        const float sw = static_cast<float>(g.w), sh = static_cast<float>(g.h);
+        float* bo = o.boxes_original + r * 4;
+        bo[0] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fsub_rn(dec[2], half_w), pw), g.wscale), 0.f), sw);
+        bo[1] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fsub_rn(dec[3], half_h), ph), g.hscale), 0.f), sh);
+        bo[2] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fadd_rn(dec[2], half_w), pw), g.wscale), 0.f), sw);
+        bo[3] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fadd_rn(dec[3], half_h), ph), g.hscale), 0.f), sh);
+    }
 }
 
 __device__ __forceinline__ float ld_as_f32(const float* p) { return *p; }
@@ -456,11 +569,7 @@ iou_kernel(const float* __restrict__ label, const float* __restrict__ pred, long
 }
 
 // ------------------------------------------------------------------------------------------------
-// Input side ("next" row N4): _get_image_tensor_coco of the reference (vision_transformer_utilities.py:418-449) after
-// the file decode: tf.image.resize_with_pad(image, H, W) (bilinear, half-pixel centres, no antialias, zero padding),
-// tf.clip_by_value(0, 255), / 127.5, - 1.  uint8 HWC in, float32 HWC in [-1, 1] out.  The interpolation follows TF's
-// resize_bilinear CPU kernel term by term (in = (i + 0.5) * scale - 0.5; lower = max(floor(in), 0); upper =
-// min(ceil(in), size - 1); lerp = in - floor(in); top/bottom lerp in x, then in y), without FMA contraction.
+// Input side, one image: uint8 HWC in, float32 HWC [th, tw, 3] in [-1, 1] out (see resize_tap / letterbox_value).
 // ------------------------------------------------------------------------------------------------
 __global__ void __launch_bounds__(256)
 preprocess_kernel(const uint8_t* __restrict__ img, int h, int w, float* __restrict__ out, int th, int tw, int rh, int rw,
@@ -473,26 +582,14 @@ preprocess_kernel(const uint8_t* __restrict__ img, int h, int w, float* __restri
     float* o = out + (static_cast<size_t>(y) * tw + x) * 3;
     const int ry = y - ph, rx = x - pw;
     if (ry < 0 || ry >= rh || rx < 0 || rx >= rw) {
-        o[0] = -1.f; o[1] = -1.f; o[2] = -1.f;        // zero padding: clip(0) / 127.5 - 1
+        o[0] = kLetterboxBar; o[1] = kLetterboxBar; o[2] = kLetterboxBar;
         return;
     }
-    const float in_y = __fsub_rn(__fmul_rn(__fadd_rn(static_cast<float>(ry), 0.5f), hscale), 0.5f);
-    const float in_x = __fsub_rn(__fmul_rn(__fadd_rn(static_cast<float>(rx), 0.5f), wscale), 0.5f);
-    const float fy = floorf(in_y), fx = floorf(in_x);
-    const int y0 = max(static_cast<int>(fy), 0), y1 = min(static_cast<int>(ceilf(in_y)), h - 1);
-    const int x0 = max(static_cast<int>(fx), 0), x1 = min(static_cast<int>(ceilf(in_x)), w - 1);
-    const float ly = __fsub_rn(in_y, fy), lx = __fsub_rn(in_x, fx);
-    const uint8_t* r0 = img + static_cast<size_t>(y0) * w * 3;
-    const uint8_t* r1 = img + static_cast<size_t>(y1) * w * 3;
+    const ResizeTap ty = resize_tap(ry, hscale, h), tx = resize_tap(rx, wscale, w);
+    const uint8_t* r0 = img + static_cast<size_t>(ty.lo) * w * 3;
+    const uint8_t* r1 = img + static_cast<size_t>(ty.hi) * w * 3;
 #pragma unroll
-    for (int c = 0; c < 3; ++c) {
-        const float tl = r0[x0 * 3 + c], tr = r0[x1 * 3 + c], bl = r1[x0 * 3 + c], br = r1[x1 * 3 + c];
-        const float top = __fadd_rn(tl, __fmul_rn(__fsub_rn(tr, tl), lx));
-        const float bot = __fadd_rn(bl, __fmul_rn(__fsub_rn(br, bl), lx));
-        float v = __fadd_rn(top, __fmul_rn(__fsub_rn(bot, top), ly));
-        v = fminf(fmaxf(v, 0.f), 255.f);
-        o[c] = __fsub_rn(__fdiv_rn(v, 127.5f), 1.f);
-    }
+    for (int c = 0; c < 3; ++c) o[c] = letterbox_value(r0, r1, tx.lo * 3 + c, tx.hi * 3 + c, tx.lerp, ty.lerp);
 }
 
 template <int LPR, typename T>
@@ -604,14 +701,37 @@ void resize_with_pad_geometry(int h, int w, int th, int tw, int* rh, int* rw, in
     *pw = p_w > 0 ? p_w : 0;
 }
 
+bool letterbox_image(const uint8_t* pixels, int h, int w, int th, int tw, LetterboxImage* im) {
+    if (h <= 0 || w <= 0 || th <= 0 || tw <= 0) return false;
+    im->pixels = pixels; im->h = h; im->w = w;
+    resize_with_pad_geometry(h, w, th, tw, &im->rh, &im->rw, &im->ph, &im->pw);
+    if (im->rh <= 0 || im->rw <= 0) return false;
+    im->hscale = static_cast<float>(h) / static_cast<float>(im->rh);
+    im->wscale = static_cast<float>(w) / static_cast<float>(im->rw);
+    return true;
+}
+
 cudaError_t preprocess_launch(const uint8_t* image, int h, int w, float* out, int th, int tw, cudaStream_t stream) {
-    if (h <= 0 || w <= 0 || th <= 0 || tw <= 0) return cudaErrorInvalidValue;
-    int rh, rw, ph, pw;
-    resize_with_pad_geometry(h, w, th, tw, &rh, &rw, &ph, &pw);
-    if (rh <= 0 || rw <= 0) return cudaErrorInvalidValue;
-    const float hscale = static_cast<float>(h) / static_cast<float>(rh), wscale = static_cast<float>(w) / static_cast<float>(rw);
+    LetterboxImage g;
+    if (!letterbox_image(image, h, w, th, tw, &g)) return cudaErrorInvalidValue;
     dim3 grid((tw + 255) / 256, th);
-    return launch_kernel(preprocess_kernel, grid, dim3(256), 0, stream, 1, image, h, w, out, th, tw, rh, rw, ph, pw, hscale, wscale);
+    return launch_kernel(preprocess_kernel, grid, dim3(256), 0, stream, 1, image, h, w, out, th, tw, g.rh, g.rw, g.ph, g.pw,
+                         g.hscale, g.wscale);
+}
+
+cudaError_t letterbox_patchify_launch(const LetterboxImage* images, int B, int H, int W, int p, void* patches, int ldp, int rp,
+                                      int out_f32, cudaStream_t stream) {
+    const int gh = (H + p - 1) / p, gw = (W + p - 1) / p;
+    const int pad_top = (gh * p - H) / 2, pad_left = (gw * p - W) / 2;
+    // the vector stores of the patch runs need every run and token row on a 4-element boundary
+    if (B <= 0 || rp < 3 * p || ldp < rp * p || rp % 4 || ldp % 4 || (reinterpret_cast<uintptr_t>(patches) & 15))
+        return cudaErrorInvalidValue;
+    const dim3 grid(gh, B);
+    if (out_f32)
+        return launch_kernel(letterbox_patchify_kernel<float>, grid, dim3(256), 0, stream, 1, images, H, W, p, gh, gw, pad_top,
+                             pad_left, static_cast<float*>(patches), ldp, rp);
+    return launch_kernel(letterbox_patchify_kernel<__nv_bfloat16>, grid, dim3(256), 0, stream, 1, images, H, W, p, gh, gw, pad_top,
+                         pad_left, static_cast<__nv_bfloat16*>(patches), ldp, rp);
 }
 
 cudaError_t iou_launch(const float* label, const float* pred, long long R, int width, float eps, float* iou,

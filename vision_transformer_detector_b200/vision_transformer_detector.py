@@ -224,6 +224,7 @@ class DetectionRecords:
     keep: Any          # (B,17)   u8  both thresholds passed
     corners: Any       # (B,17,4) i32 x0, y0, x1, y1
     packed: Any = None  # (B*17,13) f32 the same record as one row (what the ranks all-gather); only with packed=True
+    boxes_original: Any = None  # (B,17,4) f32 x0, y0, x1, y1 on each source image; only from detect_images / submit_images
 
     def detections(self) -> list[list[dict]]:
         """Kept slots per image as plain records (what the visualise loop iterates, det.py:2260-2325)."""
@@ -746,7 +747,7 @@ class VisionTransformerDetector:
         _capi.check(self._lib.vitdet_submit_host(self._h, _capi.np_ptr(xi), 1 if u8 else 0, B, self._mode(compute_mode), C.byref(params),
                                                  1 if packed else 0, None, C.byref(ticket)))
         self._inflight = getattr(self, "_inflight", {})
-        self._inflight[ticket.value] = (B, packed, xi)          # xi kept alive: a page-locked buffer is read asynchronously
+        self._inflight[ticket.value] = (B, packed, xi, None)    # xi kept alive: a page-locked buffer is read asynchronously
         return ticket.value
 
     def collect(self, ticket: int) -> DetectionRecords:
@@ -755,13 +756,83 @@ class VisionTransformerDetector:
         if entry is None:
             # not (or no longer) in flight: fail with the library's error type, like vitdet_collect itself does
             raise _capi.VitdetError(_capi.E_INVALID, f"collect: ticket {ticket} is not in flight")
-        B, packed, _ = entry
+        B, packed, _, boxes = entry
         S = Constants.MAX_DETECT_OBJECTS_QUANTITY.value
         logits, dec, cid, cc, keep, cor = _alloc_records_np(B, S)
         pk = np.empty((B * S, 13), np.float32) if packed else None
         st = _records_struct(dec, cid, cc, keep, cor, pk)
         _capi.check(self._lib.vitdet_collect(self._h, int(ticket), _capi.np_ptr(logits), C.byref(st)))
-        return DetectionRecords(logits, dec, cid, cc, keep, cor, pk)
+        return DetectionRecords(logits, dec, cid, cc, keep, cor, pk, boxes)
+
+    # -- decoded images of any size ------------------------------------------------------------------
+    @staticmethod
+    def _image_list(images) -> tuple[list, bool]:
+        """(the images as contiguous uint8 (h, w, 3) arrays or CUDA tensors, whether they are CUDA tensors); ValueError for
+        anything the library would not take as it is."""
+        imgs = list(images)
+        if not imgs:
+            raise ValueError("images must be a non-empty sequence of uint8 (h, w, 3) images")
+        on_gpu = [_is_torch_cuda(im) for im in imgs]
+        if any(on_gpu) and not all(on_gpu):
+            raise ValueError("images mixes host arrays and CUDA tensors; pass one kind")
+        out = []
+        for i, im in enumerate(imgs):
+            im = im if on_gpu[0] else np.asarray(im)
+            if not _is_uint8(im):
+                raise ValueError(f"image {i}: dtype {im.dtype}, expected uint8")
+            if im.ndim != 3 or im.shape[2] != 3:
+                raise ValueError(f"image {i}: shape {tuple(im.shape)}, expected (height, width, 3)")
+            out.append(im.contiguous() if on_gpu[0] else np.ascontiguousarray(im))
+        if on_gpu[0] and len({im.device for im in out}) != 1:
+            raise ValueError("the images are on more than one device")
+        return out, on_gpu[0]
+
+    @staticmethod
+    def _image_table(imgs, ptr) -> C.Array:
+        return (_capi.Image * len(imgs))(*[_capi.Image(ptr(im), int(im.shape[0]), int(im.shape[1])) for im in imgs])
+
+    def detect_images(self, images, objectness_threshold=None, classification_threshold=None, strict=True,
+                      compute_mode: str | None = None, packed: bool = False) -> DetectionRecords:
+        """detect() on decoded images of any size, what _get_image_tensor_coco (vision_transformer_utilities.py:418-449) feeds
+        the model: every image is letterboxed to the model's input size (resize_with_pad, clip, / 127.5 - 1) inside the patch
+        kernel.  images: a sequence of uint8 (h, w, 3) numpy arrays (one synchronous call) or of torch CUDA uint8 tensors on
+        one device (asynchronous on torch's current stream, torch outputs).  Boxes are decoded at the model's input size;
+        `boxes_original` (B, 17, 4) holds x0, y0, x1, y1 of every slot's box on its source image, in source pixels."""
+        imgs, on_gpu = self._image_list(images)
+        if not on_gpu:
+            return self.collect(self.submit_images(imgs, objectness_threshold, classification_threshold, strict, compute_mode, packed))
+        import torch
+        B, S = len(imgs), Constants.MAX_DETECT_OBJECTS_QUANTITY.value
+        params = _decode_params(objectness_threshold, classification_threshold, strict, self.config.input_shape[:2])
+        table = self._image_table(imgs, lambda t: t.data_ptr())
+        dev = imgs[0].device
+        with torch.cuda.device(dev):
+            logits, dec, cid, cc, keep, cor = _alloc_records_torch(B, S, dev)
+            pk = torch.empty((B * S, 13), dtype=torch.float32, device=dev) if packed else None
+            boxes = torch.empty((B, S, 4), dtype=torch.float32, device=dev)
+            st = _records_struct(dec, cid, cc, keep, cor, pk)
+            _capi.check(self._lib.vitdet_forward_images(self._h, table, B, self._mode(compute_mode), C.byref(params),
+                                                        C.c_void_p(logits.data_ptr()), C.byref(st), C.c_void_p(boxes.data_ptr()),
+                                                        _torch_stream_ptr(dev)))
+        return DetectionRecords(logits, dec, cid, cc, keep, cor, pk, boxes)
+
+    def submit_images(self, images, objectness_threshold=None, classification_threshold=None, strict=True,
+                      compute_mode: str | None = None, packed: bool = False) -> int:
+        """Asynchronous detect_images() for host arrays (vitdet_submit_images_host), completed by collect(ticket); shares the
+        two submission slots of submit().  Page-locked arrays must stay alive until their ticket is collected."""
+        imgs, on_gpu = self._image_list(images)
+        if on_gpu:
+            raise ValueError("submit_images takes host arrays; detect_images runs CUDA tensors asynchronously already")
+        B, S = len(imgs), Constants.MAX_DETECT_OBJECTS_QUANTITY.value
+        params = _decode_params(objectness_threshold, classification_threshold, strict, self.config.input_shape[:2])
+        boxes = np.empty((B, S, 4), np.float32)
+        ticket = C.c_int(-1)
+        _capi.check(self._lib.vitdet_submit_images_host(self._h, self._image_table(imgs, lambda a: a.ctypes.data), B,
+                                                        self._mode(compute_mode), C.byref(params), 1 if packed else 0,
+                                                        _capi.np_ptr(boxes), None, C.byref(ticket)))
+        self._inflight = getattr(self, "_inflight", {})
+        self._inflight[ticket.value] = (B, packed, imgs, boxes)
+        return ticket.value
 
     def predict(self, x, batch_size=None, verbose="auto", steps=None, callbacks=None, normalize_uint8: bool = False, **kwargs):
         """keras Model.predict: host array in, numpy (B, 17, 6) raw logits out.  `batch_size` only
