@@ -278,6 +278,36 @@ int vitdet_forward_images(vitdet_handle* h, const vitdet_image* images, int B, i
 int vitdet_submit_images_host(vitdet_handle* h, const vitdet_image* images, int B, int mode, const vitdet_decode_params* params,
                               int want_packed, float* boxes_original_host, void* stream, int* ticket);
 
+/* ---- JPEG files ("next" row N4: tf.io.read_file + tf.image.decode_jpeg, vision_transformer_utilities.py:418-449) ----
+ * Baseline sequential Huffman JPEG decoded on the device, bit-identical to libjpeg-turbo's defaults (ISLOW IDCT, fancy
+ * upsampling), i.e. to PIL's Image.open(f).convert("RGB") and tf.image.decode_jpeg.  Accepted: SOF0 / SOF1, 8-bit;
+ * 1 component (grey, R = G = B) or 3; luma sampling 1x1, 2x1 or 2x2 with chroma 1x1; any size up to 65535 x 65535; restart
+ * intervals; custom Huffman tables; one interleaved scan.  Colour space as libjpeg decides it: JFIF -> YCbCr, else an Adobe
+ * transform flag (0 = RGB), else component ids 'R','G','B' -> RGB, else YCbCr.  APPn / COM / EXIF are skipped; EXIF
+ * orientation is not applied.  Any other file (progressive, lossless, arithmetic, 12-bit, 2 or 4 components, other
+ * sampling, several scans, DNL, a table referenced but not defined, truncated, no EOI, not a JPEG) fails the whole list
+ * with VITDET_E_INVALID, naming the file and the reason, before anything is copied or launched.  Corrupt entropy data
+ * decodes without error (oracle/jpeg_oracle.py states what it decodes to). */
+typedef struct vitdet_jpeg {
+    const uint8_t* data;               /* HOST bytes of one file */
+    int64_t bytes;
+} vitdet_jpeg;
+/* Header check on the host (no device needed): the size and the component count (1 or 3) of an accepted file. */
+int vitdet_jpeg_info(const uint8_t* data, int64_t bytes, int* height, int* width, int* components);
+/* Decodes B files; image i's (height, width, 3) uint8 RGB pixels go to out_dev + out_offsets[i] (DEVICE).  Asynchronous on
+ * `stream`; the files are read before it returns.  The handle's decode buffers are reused by the next call on any stream:
+ * that call first waits on the host for this decode to finish. */
+int vitdet_decode_jpeg(vitdet_handle* h, const vitdet_jpeg* files, int B, uint8_t* out_dev, const int64_t* out_offsets, void* stream);
+/* vitdet_submit_images_host on JPEG files: the files are copied (page-locked bytes read directly when every file is
+ * page-locked, otherwise staged), decoded on the device and letterboxed in the patch kernel.  The same submission slots,
+ * completed by vitdet_collect; page-locked files must stay valid until then. */
+int vitdet_submit_jpeg_host(vitdet_handle* h, const vitdet_jpeg* files, int B, int mode, const vitdet_decode_params* params,
+                            int want_packed, float* boxes_original_host, void* stream, int* ticket);
+/* Counters of the last JPEG decode on this handle (synchronises with it): stats[0] subsequences of the parallel Huffman
+ * decode, stats[1] subsequences re-decoded from a start other than their speculative one (sync passes and repair),
+ * stats[2] symbols re-decoded. */
+int vitdet_jpeg_stats(vitdet_handle* h, int64_t* stats);
+
 /* ---- evaluation metric ("next" row N2): MeanAveragePrecision of the reference (det.py:1268-2060) ----
  * The COCO-style AP of the reference: mean over the IoU thresholds tf.linspace(0.5, 0.95, 10) of the mean, over the
  * classes seen so far, of the class AP computed from the latest `latest_related_images` related images per class

@@ -72,6 +72,11 @@ class Image(C.Structure):
     _fields_ = [("pixels", C.c_void_p), ("height", C.c_int32), ("width", C.c_int32)]
 
 
+class Jpeg(C.Structure):
+    """struct vitdet_jpeg — the host bytes of one JPEG file."""
+    _fields_ = [("data", C.c_void_p), ("bytes", C.c_int64)]
+
+
 # every symbol include/vitdet_b200.h declares: name -> (restype, argtypes)
 _P = C.c_void_p
 SYMBOLS = {
@@ -127,6 +132,11 @@ SYMBOLS = {
     "vitdet_forward_images": (C.c_int, [_P, C.POINTER(Image), C.c_int, C.c_int, C.POINTER(DecodeParams), _P, C.POINTER(Detections), _P, _P]),
     "vitdet_submit_images_host": (C.c_int, [_P, C.POINTER(Image), C.c_int, C.c_int, C.POINTER(DecodeParams), C.c_int, _P, _P,
                                             C.POINTER(C.c_int)]),
+    "vitdet_jpeg_info": (C.c_int, [_P, C.c_int64, C.POINTER(C.c_int), C.POINTER(C.c_int), C.POINTER(C.c_int)]),
+    "vitdet_decode_jpeg": (C.c_int, [_P, C.POINTER(Jpeg), C.c_int, _P, _P, _P]),
+    "vitdet_submit_jpeg_host": (C.c_int, [_P, C.POINTER(Jpeg), C.c_int, C.c_int, C.POINTER(DecodeParams), C.c_int, _P, _P,
+                                          C.POINTER(C.c_int)]),
+    "vitdet_jpeg_stats": (C.c_int, [_P, _P]),
     "vitdet_gather_detections": (C.c_int, [_P, _P, C.c_int, _P, _P]),
     "vitdet_nccl_unique_id": (C.c_int, [C.c_char_p]),
     "vitdet_nccl_comm_create": (C.c_int, [C.c_char_p, C.c_int, C.c_int, C.POINTER(_P)]),

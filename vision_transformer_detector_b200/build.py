@@ -18,7 +18,7 @@ INCLUDE = os.path.join(os.path.dirname(PKG_DIR), "include")
 LIB_PATH = os.path.join(PKG_DIR, "libvitdet_b200.so")
 STAMP_PATH = os.path.join(PKG_DIR, ".libvitdet_b200.stamp")
 
-SOURCES = ["engine.cu", "gemm_tc.cu", "gemm_simt.cu", "attention.cu", "attention_tc.cu", "mlp_tail.cu", "rowops.cu", "metric.cu", "gather.cu"]
+SOURCES = ["engine.cu", "gemm_tc.cu", "gemm_simt.cu", "attention.cu", "attention_tc.cu", "mlp_tail.cu", "rowops.cu", "metric.cu", "gather.cu", "jpeg.cu"]
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",
     "-lineinfo", "-O3", "-std=c++17",

@@ -318,6 +318,9 @@ struct HostSlot {
     void* pin_out = nullptr; size_t pin_out_bytes = 0;
     LetterboxImage* pin_table = nullptr; size_t pin_table_bytes = 0;
     DevBuf dev_in, dev_out, dev_table;
+    // a submission of JPEG files (vitdet_submit_jpeg_host): its descriptor block, decode scratch and decoded pixels
+    char* pin_jpeg = nullptr; size_t pin_jpeg_bytes = 0;
+    DevBuf jpeg_work, jpeg_rgb;
     std::vector<cudaEvent_t> copy_events;      // one per staged sub-chunk of images
     cudaEvent_t done = nullptr;                // recorded after the D2H copy of the record block
     bool busy = false;
@@ -328,6 +331,7 @@ struct HostSlot {
         if (pin_in) cudaFreeHost(pin_in);
         if (pin_out) cudaFreeHost(pin_out);
         if (pin_table) cudaFreeHost(pin_table);
+        if (pin_jpeg) cudaFreeHost(pin_jpeg);
         for (auto e : copy_events) cudaEventDestroy(e);
         if (done) cudaEventDestroy(done);
     }
@@ -403,12 +407,20 @@ struct vitdet_handle {
     int next_slot = 0;
     StagePool* stage_pool = nullptr;             // created on the first pageable submission
     DevBuf images_table;                         // letterbox table of vitdet_forward_images, written in stream order
+    // vitdet_decode_jpeg: descriptor block and files staged in pinned memory, device files and decode scratch; jpeg_done,
+    // recorded after the last decode, orders their reuse whatever stream the next call runs on
+    char* jpeg_pin = nullptr; size_t jpeg_pin_bytes = 0;
+    cudaEvent_t jpeg_done = nullptr;
+    DevBuf jpeg_files, jpeg_work;
+    const long long* jpeg_stats = nullptr;       // repair counters of the last JPEG decode (device)
 
     ~vitdet_handle() {
         for (auto& r : prof_pending) { cudaEventDestroy(r.a); cudaEventDestroy(r.b); }
         for (auto e : prof_pool) cudaEventDestroy(e);
         delete stage_pool;
         if (copy_stream) cudaStreamDestroy(copy_stream);
+        if (jpeg_pin) cudaFreeHost(jpeg_pin);
+        if (jpeg_done) cudaEventDestroy(jpeg_done);
     }
 };
 
@@ -1443,13 +1455,32 @@ static bool page_locked(const void* p) {
     return pinned;
 }
 
+// Creates the handle's staging threads on first use
+static void ensure_stage_pool(vitdet_handle* h) {
+    if (h->stage_pool) return;
+    // staging threads (+ the calling thread): a share of the host's cores, divided among the ranks of this node
+    // (LOCAL_WORLD_SIZE under torchrun); VITDET_STAGE_THREADS overrides the total
+    const int hw = static_cast<int>(std::thread::hardware_concurrency());
+    int local_world = 1;
+    if (const char* e = getenv("LOCAL_WORLD_SIZE")) local_world = atoi(e) > 0 ? atoi(e) : 1;
+    int workers = (hw > 0 ? hw / (2 * local_world) : 6) - 1;
+    if (workers > 11) workers = 11;
+    if (workers < 1) workers = 1;
+    if (const char* e = getenv("VITDET_STAGE_THREADS")) workers = atoi(e) - 1;
+    if (hw > 0 && workers > hw - 1) workers = hw - 1;
+    if (workers < 0) workers = 0;
+    h->stage_pool = new StagePool(workers);
+}
+
 // The images of one host submission: image i, src[i][0, offs[i + 1] - offs[i]), goes to byte offs[i] of the slot's device
 // input.  `table` (separate images of any size) holds their letterbox geometry; its pixel pointers are filled in here.
 // Without it the images are one contiguous array of the model's size.
+// `jpeg`: the sources are JPEG files, decoded on the device into the slot's pixel arena before the forward.
 struct HostImages {
     std::vector<const char*> src;
     std::vector<size_t> offs;
     std::vector<LetterboxImage> table;
+    const JpegBatch* jpeg = nullptr;
 };
 
 static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, int mode, const vitdet_decode_params* params,
@@ -1508,20 +1539,7 @@ static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, 
         CU_TRY(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         sl.copy_events.push_back(e);
     }
-    if (!pinned && !h->stage_pool) {
-        // staging threads (+ the calling thread): a share of the host's cores, divided among the ranks of this node
-        // (LOCAL_WORLD_SIZE under torchrun); VITDET_STAGE_THREADS overrides the total
-        const int hw = static_cast<int>(std::thread::hardware_concurrency());
-        int local_world = 1;
-        if (const char* e = getenv("LOCAL_WORLD_SIZE")) local_world = atoi(e) > 0 ? atoi(e) : 1;
-        int workers = (hw > 0 ? hw / (2 * local_world) : 6) - 1;
-        if (workers > 11) workers = 11;
-        if (workers < 1) workers = 1;
-        if (const char* e = getenv("VITDET_STAGE_THREADS")) workers = atoi(e) - 1;
-        if (hw > 0 && workers > hw - 1) workers = hw - 1;
-        if (workers < 0) workers = 0;
-        h->stage_pool = new StagePool(workers);
-    }
+    if (!pinned) ensure_stage_pool(h);
     char* dev_in = sl.dev_in.as<char>();
     for (int i = 0; i < n_sub; ++i) {
         const int i0 = i * kGran, i1 = std::min(B, i0 + kGran);
@@ -1544,6 +1562,32 @@ static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, 
     opts.ready_gran = kGran;
     opts.in_u8 = in_u8;
     const void* images_dev = dev_in;
+    const char* pixels_dev = dev_in;
+    std::vector<size_t> pixel_offs;
+    if (in.jpeg) {
+        // decode after the last file's copy, on the compute stream, into the slot's arena; the forward then waits for nothing
+        const JpegBatch& jb = *in.jpeg;
+        if (sl.pin_jpeg_bytes < jb.desc.size()) {
+            if (sl.pin_jpeg) cudaFreeHost(sl.pin_jpeg);
+            sl.pin_jpeg = nullptr; sl.pin_jpeg_bytes = 0;
+            CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&sl.pin_jpeg), jb.desc.size(), cudaHostAllocDefault));
+            sl.pin_jpeg_bytes = jb.desc.size();
+        }
+        memcpy(sl.pin_jpeg, jb.desc.data(), jb.desc.size());
+        RC_TRY(sl.jpeg_work.ensure(jb.work_bytes));
+        RC_TRY(sl.jpeg_rgb.ensure(jb.rgb_bytes));
+        CU_TRY(cudaMemcpyAsync(sl.jpeg_work.p, sl.pin_jpeg, jb.desc.size(), cudaMemcpyHostToDevice, st));
+        CU_TRY(cudaStreamWaitEvent(st, sl.copy_events[n_sub - 1], 0));
+        h->launches += kJpegLaunches;
+        CU_TRY(jpeg_decode_launch(jb, dev_in, sl.jpeg_work.p, sl.jpeg_rgb.as<uint8_t>(), st));
+        h->jpeg_stats = reinterpret_cast<const long long*>(sl.jpeg_work.as<char>() + jb.o_stats);
+        opts = ForwardOpts();
+        opts.in_u8 = in_u8;
+        pixels_dev = sl.jpeg_rgb.as<char>();
+        pixel_offs = jb.rgb_off;
+    } else {
+        pixel_offs.assign(in.offs.begin(), in.offs.end() - 1);
+    }
     if (separate) {
         // the slot's own table: the pinned copy is not touched again before this submission is collected
         const size_t table_bytes = static_cast<size_t>(B) * sizeof(LetterboxImage);
@@ -1556,7 +1600,7 @@ static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, 
         RC_TRY(sl.dev_table.ensure(table_bytes));
         for (int k = 0; k < B; ++k) {
             sl.pin_table[k] = in.table[k];
-            sl.pin_table[k].pixels = reinterpret_cast<const uint8_t*>(dev_in + in.offs[k]);
+            sl.pin_table[k].pixels = reinterpret_cast<const uint8_t*>(pixels_dev + pixel_offs[k]);
         }
         CU_TRY(cudaMemcpyAsync(sl.dev_table.p, sl.pin_table, table_bytes, cudaMemcpyHostToDevice, st));
         opts.letterbox = 1;
@@ -1698,6 +1742,90 @@ int vitdet_submit_images_host(vitdet_handle* h, const vitdet_image* images, int 
         in.offs[i + 1] = in.offs[i] + static_cast<size_t>(images[i].height) * images[i].width * 3;
     }
     return submit_host_impl(h, in, 1, B, mode, params, want_packed, boxes_original_host, stream, ticket);
+}
+
+// A caller's list of JPEG files -> the batch plan (every file parsed on the host; a rejected file fails the list, naming it)
+static int jpeg_files_plan(const char* fn, const vitdet_jpeg* files, int B, const int64_t* out_offsets, JpegBatch* jb) {
+    if (!files || B <= 0) return fail(VITDET_E_INVALID, "%s: %s", fn, !files ? "files is null" : "B must be positive");
+    std::vector<const uint8_t*> data(B);
+    std::vector<int64_t> bytes(B);
+    for (int i = 0; i < B; ++i) { data[i] = files[i].data; bytes[i] = files[i].bytes; }
+    return jpeg_plan(fn, data.data(), bytes.data(), B, out_offsets, jb);
+}
+
+int vitdet_jpeg_info(const uint8_t* data, int64_t bytes, int* height, int* width, int* components) {
+    char why[256];
+    if (jpeg_info(data, bytes, height, width, components, why, sizeof(why))) return fail(VITDET_E_INVALID, "jpeg_info: %s", why);
+    return 0;
+}
+
+int vitdet_decode_jpeg(vitdet_handle* h, const vitdet_jpeg* files, int B, uint8_t* out_dev, const int64_t* out_offsets, void* stream) {
+    if (!h || !out_dev || !out_offsets) return fail(VITDET_E_INVALID, "decode_jpeg: null handle, out_dev or out_offsets");
+    int cur = -1;
+    CU_TRY(cudaGetDevice(&cur));
+    if (cur != h->device) return fail(VITDET_E_INVALID, "decode_jpeg: the handle lives on device %d but the current CUDA device is %d", h->device, cur);
+    JpegBatch jb;
+    RC_TRY(jpeg_files_plan("decode_jpeg", files, B, out_offsets, &jb));
+    for (int i = 0; i < B; ++i)
+        if (out_offsets[i] < 0) return fail(VITDET_E_INVALID, "decode_jpeg: image %d: negative output offset", i);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // the previous decode has read the staging and the device buffers before they are reused, on any stream
+    if (h->jpeg_done) CU_TRY(cudaEventSynchronize(h->jpeg_done));
+    else CU_TRY(cudaEventCreateWithFlags(&h->jpeg_done, cudaEventDisableTiming));
+    // descriptors and files in one pinned block, the files concatenated by the staging threads: the caller's bytes are
+    // read before this returns
+    const size_t files_bytes = jb.file_off[B], pin_bytes = jb.desc.size() + files_bytes;
+    if (h->jpeg_pin_bytes < pin_bytes) {
+        if (h->jpeg_pin) cudaFreeHost(h->jpeg_pin);
+        h->jpeg_pin = nullptr; h->jpeg_pin_bytes = 0;
+        CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&h->jpeg_pin), pin_bytes, cudaHostAllocDefault));
+        h->jpeg_pin_bytes = pin_bytes;
+    }
+    memcpy(h->jpeg_pin, jb.desc.data(), jb.desc.size());
+    std::vector<const char*> src(B);
+    for (int i = 0; i < B; ++i) src[i] = reinterpret_cast<const char*>(files[i].data);
+    ensure_stage_pool(h);
+    h->stage_pool->copy(h->jpeg_pin + jb.desc.size(), src.data(), jb.file_off.data(), B);
+    RC_TRY(h->jpeg_work.ensure(jb.work_bytes));
+    RC_TRY(h->jpeg_files.ensure(files_bytes));
+    CU_TRY(cudaMemcpyAsync(h->jpeg_work.p, h->jpeg_pin, jb.desc.size(), cudaMemcpyHostToDevice, st));
+    CU_TRY(cudaMemcpyAsync(h->jpeg_files.p, h->jpeg_pin + jb.desc.size(), files_bytes, cudaMemcpyHostToDevice, st));
+    h->launches += kJpegLaunches;
+    CU_TRY(jpeg_decode_launch(jb, h->jpeg_files.as<char>(), h->jpeg_work.p, out_dev, st));
+    CU_TRY(cudaEventRecord(h->jpeg_done, st));
+    h->jpeg_stats = reinterpret_cast<const long long*>(h->jpeg_work.as<char>() + jb.o_stats);
+    return 0;
+}
+
+int vitdet_submit_jpeg_host(vitdet_handle* h, const vitdet_jpeg* files, int B, int mode, const vitdet_decode_params* params,
+                            int want_packed, float* boxes_original_host, void* stream, int* ticket) {
+    if (!h || !params || !ticket) return fail(VITDET_E_INVALID, "submit_jpeg_host: handle, params and ticket must not be null");
+    const int th = h->cfg.image_h, tw = h->cfg.image_w;
+    if (boxes_original_host && (params->image_h != static_cast<float>(th) || params->image_w != static_cast<float>(tw)))
+        return fail(VITDET_E_INVALID, "submit_jpeg_host: boxes_original needs the decode at the model's input size %d x %d (params image_h / image_w)", th, tw);
+    JpegBatch jb;
+    RC_TRY(jpeg_files_plan("submit_jpeg_host", files, B, nullptr, &jb));
+    HostImages in;
+    in.table.resize(B);
+    in.src.resize(B);
+    in.offs.assign(jb.file_off.begin(), jb.file_off.end());
+    for (int i = 0; i < B; ++i) {
+        in.src[i] = reinterpret_cast<const char*>(files[i].data);
+        if (!letterbox_image(nullptr, jb.height[i], jb.width[i], th, tw, &in.table[i]))
+            return fail(VITDET_E_INVALID, "submit_jpeg_host: image %d: a %d x %d image letterboxed to %d x %d resizes to %d x %d pixels", i,
+                        jb.height[i], jb.width[i], th, tw, in.table[i].rh, in.table[i].rw);
+    }
+    in.jpeg = &jb;
+    return submit_host_impl(h, in, 1, B, mode, params, want_packed, boxes_original_host, stream, ticket);
+}
+
+int vitdet_jpeg_stats(vitdet_handle* h, int64_t* stats) {
+    if (!h || !stats) return fail(VITDET_E_INVALID, "jpeg_stats: null argument");
+    if (!h->jpeg_stats) return fail(VITDET_E_INVALID, "jpeg_stats: no JPEG decode has run on this handle");
+    long long v[3];
+    CU_TRY(cudaMemcpy(v, h->jpeg_stats, sizeof(v), cudaMemcpyDeviceToHost));
+    for (int i = 0; i < 3; ++i) stats[i] = v[i];
+    return 0;
 }
 
 // ------------------------------------------------------------------------------------------------

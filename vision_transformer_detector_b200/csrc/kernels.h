@@ -6,6 +6,8 @@
 #include <stddef.h>
 #include <stdint.h>
 
+#include <vector>
+
 namespace vitdet {
 
 // ------------------------------------------------------------------------------------------------
@@ -197,5 +199,37 @@ cudaError_t iou_launch(const float* label, const float* pred, long long R, int w
 
 // Records the message vitdet_last_error() returns on the calling thread and hands `code` back (engine.cu).
 int fail(int code, const char* fmt, ...);
+
+// ------------------------------------------------------------------------------------------------
+// Baseline JPEG decode (jpeg.cu), bit-exact with libjpeg-turbo's defaults (ISLOW IDCT, fancy upsampling, jdcolor.c).
+// The host parses the headers and cuts the entropy data at RSTn into segments; the device de-stuffs every segment,
+// Huffman-decodes it in subsequences of kJpegSubBits bits (speculative pass, kJpegSyncPasses parallel sync passes, one-warp-per-segment
+// repair, write pass),
+// adds up the DC differences, and runs IDCT, upsampling and colour conversion into dense uint8 (h, w, 3) RGB.
+// ------------------------------------------------------------------------------------------------
+constexpr int kJpegSubBits = 1024;     // L, a multiple of 32: one checkpoint per 32-bit word
+constexpr int kJpegSyncPasses = 8;     // parallel sync passes ahead of the one-warp-per-segment repair
+constexpr int kJpegLaunches = 7 + kJpegSyncPasses;     // kernels of one jpeg_decode, whatever the data
+// Host header check: 0 and the size and component count, or VITDET_E_INVALID with the reason in why.
+int jpeg_info(const uint8_t* data, int64_t bytes, int* height, int* width, int* components, char* why, size_t why_len);
+// The device work of a batch of files, planned on the host.  work_bytes of device scratch hold, at these offsets: the
+// descriptor block `desc` (images, segments, Huffman tables; copied there by the caller), the compact bit streams, the
+// coefficients, the subsequence states, the component planes and three counters (int64: subsequences, subsequences the
+// sync passes and the repair re-decoded, symbols they re-decoded).
+struct JpegBatch {
+    int B = 0, nseg = 0, nsub = 0;
+    long long nblocks = 0, npix = 0;
+    std::vector<char> desc;
+    std::vector<int> height, width;
+    std::vector<size_t> file_off;      // B + 1: file i is bytes [file_off[i], file_off[i + 1]) of the concatenated files
+    std::vector<size_t> rgb_off;       // where image i's pixels go, relative to the output pointer of jpeg_decode
+    size_t rgb_bytes = 0;              // with the default layout (out_offsets null): the output's size
+    size_t o_compact = 0, o_coef = 0, o_spec = 0, o_check = 0, o_sync = 0, o_start = 0, o_planes = 0, o_stats = 0, work_bytes = 0;
+};
+// Parses B files (HOST bytes); out_offsets (may be null: images packed 256-byte aligned) place the outputs.  Fails with
+// VITDET_E_INVALID naming the first rejected file.
+int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, int B, const int64_t* out_offsets, JpegBatch* b);
+// Launches the kJpegLaunches kernels: files_dev holds the concatenated files, work the scratch with b.desc at offset 0.
+cudaError_t jpeg_decode_launch(const JpegBatch& b, const char* files_dev, void* work, uint8_t* out, cudaStream_t stream);
 
 }  // namespace vitdet

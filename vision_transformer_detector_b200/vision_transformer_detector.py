@@ -277,6 +277,37 @@ def _torch_stream_ptr(device) -> C.c_void_p:
     return C.c_void_p(torch.cuda.current_stream(device).cuda_stream)
 
 
+def _jpeg_arrays(files) -> list:
+    """The bytes of every file as a 1-D uint8 numpy array (a view of bytes-like objects, the contents of paths); ValueError
+    for an empty list, an empty file or an item that is neither."""
+    if isinstance(files, (bytes, bytearray, memoryview, str, os.PathLike)):
+        raise ValueError("files must be a sequence of JPEG files, not a single one")
+    items = list(files)
+    if not items:
+        raise ValueError("files must be a non-empty sequence of bytes-like objects or paths")
+    out = []
+    for i, f in enumerate(items):
+        if isinstance(f, (str, os.PathLike)):
+            with open(f, "rb") as fh:
+                a = np.frombuffer(fh.read(), np.uint8)
+        elif isinstance(f, np.ndarray):
+            if f.dtype != np.uint8 or f.ndim != 1 or not f.flags.c_contiguous:
+                raise ValueError(f"file {i}: a numpy array must be 1-D contiguous uint8, got {f.dtype} {f.shape}")
+            a = f
+        elif isinstance(f, (bytes, bytearray, memoryview)):
+            a = np.frombuffer(f, np.uint8)
+        else:
+            raise ValueError(f"file {i}: {type(f).__name__} is neither bytes-like nor a path")
+        if a.size == 0:
+            raise ValueError(f"file {i} is empty")
+        out.append(a)
+    return out
+
+
+def _jpeg_table(arrs) -> C.Array:
+    return (_capi.Jpeg * len(arrs))(*[_capi.Jpeg(a.ctypes.data, int(a.size)) for a in arrs])
+
+
 def _alloc_records_np(B: int, S: int):
     return (np.empty((B, S, 6), np.float32), np.empty((B, S, 6), np.float32), np.empty((B, S), np.int32),
             np.empty((B, S), np.float32), np.empty((B, S), np.uint8), np.empty((B, S, 4), np.int32))
@@ -832,6 +863,30 @@ class VisionTransformerDetector:
                                                         _capi.np_ptr(boxes), None, C.byref(ticket)))
         self._inflight = getattr(self, "_inflight", {})
         self._inflight[ticket.value] = (B, packed, imgs, boxes)
+        return ticket.value
+
+    # -- JPEG files ---------------------------------------------------------------------------------
+    def detect_jpeg(self, files, objectness_threshold=None, classification_threshold=None, strict=True,
+                    compute_mode: str | None = None, packed: bool = False) -> DetectionRecords:
+        """detect_images() on JPEG files, decoded on the GPU bit-identically to PIL's Image.open(f).convert("RGB") (and
+        tf.image.decode_jpeg): the same records, boxes_original included, as detect_images on the PIL-decoded images.
+        files: a sequence of bytes-like objects (bytes, bytearray, memoryview, 1-D uint8 numpy arrays) or paths.  One
+        synchronous call; a file outside baseline JPEG fails the call, naming it (VitdetError E_INVALID)."""
+        return self.collect(self.submit_jpeg(files, objectness_threshold, classification_threshold, strict, compute_mode, packed))
+
+    def submit_jpeg(self, files, objectness_threshold=None, classification_threshold=None, strict=True,
+                    compute_mode: str | None = None, packed: bool = False) -> int:
+        """Asynchronous detect_jpeg() (vitdet_submit_jpeg_host), completed by collect(ticket); shares the two submission
+        slots of submit().  Page-locked files are read directly and must stay alive until their ticket is collected."""
+        arrs = _jpeg_arrays(files)
+        B, S = len(arrs), Constants.MAX_DETECT_OBJECTS_QUANTITY.value
+        params = _decode_params(objectness_threshold, classification_threshold, strict, self.config.input_shape[:2])
+        boxes = np.empty((B, S, 4), np.float32)
+        ticket = C.c_int(-1)
+        _capi.check(self._lib.vitdet_submit_jpeg_host(self._h, _jpeg_table(arrs), B, self._mode(compute_mode), C.byref(params),
+                                                      1 if packed else 0, _capi.np_ptr(boxes), None, C.byref(ticket)))
+        self._inflight = getattr(self, "_inflight", {})
+        self._inflight[ticket.value] = (B, packed, arrs, boxes)
         return ticket.value
 
     def predict(self, x, batch_size=None, verbose="auto", steps=None, callbacks=None, normalize_uint8: bool = False, **kwargs):

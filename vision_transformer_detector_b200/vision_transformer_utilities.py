@@ -4,6 +4,7 @@ the reference module (annotation parsing at import time from hard-coded D:\\ pat
 
     _get_image_tensor_coco(one_image_path)        vision_transformer_utilities.py:418-449
     preprocess_image(image_uint8)                 the arithmetic of that function: resize_with_pad, clip, /127.5 - 1
+    decode_jpeg(files)                            tf.image.decode_jpeg on the GPU, bit-identical to PIL / libjpeg-turbo
 
 The arithmetic runs on the GPU (vitdet_preprocess_image*); only the file decode is host work (PIL)."""
 from __future__ import annotations
@@ -13,7 +14,7 @@ import ctypes as C
 import numpy as np
 
 from . import _capi
-from .vision_transformer_detector import Constants, _is_torch_cuda, _torch_stream_ptr
+from .vision_transformer_detector import Constants, DetectorConfig, _is_torch_cuda, _jpeg_arrays, _jpeg_table, _torch_stream_ptr
 
 MODEL_IMAGE_HEIGHT, MODEL_IMAGE_WIDTH = Constants.MODEL_IMAGE_SIZE.value       # vision_transformer_utilities.py:23-24
 
@@ -56,3 +57,47 @@ def _get_image_tensor_coco(one_image_path):
     with Image.open(one_image_path) as im:
         arr = np.asarray(im.convert("RGB"), dtype=np.uint8)
     return preprocess_image(arr), (int(arr.shape[0]), int(arr.shape[1]))
+
+
+_decoders: dict = {}      # device index -> a handle of a tiny model, whose JPEG decode scratch decode_jpeg uses
+
+
+def _decoder(index: int) -> C.c_void_p:
+    h = _decoders.get(index)
+    if h is None:
+        cfg = DetectorConfig(input_shape=(16, 16, 3), encoder_num_heads=1, encoder_mlp_quantities=1, encoder_repeat_times=1,
+                             mlp_head_last_units=8, mlp_head_dense_layers_quantity=1).to_c()
+        h = C.c_void_p()
+        _capi.check(_capi.load().vitdet_create(C.byref(cfg), C.byref(h)))
+        _decoders[index] = h
+    return h
+
+
+def decode_jpeg(files, device=None) -> list:
+    """Baseline JPEG files -> a list of torch CUDA uint8 (h, w, 3) RGB tensors, decoded on the GPU bit-identically to
+    np.asarray(PIL.Image.open(f).convert("RGB")) (libjpeg-turbo's ISLOW IDCT and fancy upsampling, which
+    tf.image.decode_jpeg also uses).  files: bytes-like objects or paths.  Asynchronous on torch's current stream of
+    `device` (default: the current CUDA device).  A file outside baseline JPEG raises VitdetError (E_INVALID) naming it."""
+    import torch
+    arrs = _jpeg_arrays(files)
+    lib = _capi.load()
+    dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
+    if dev.type != "cuda":
+        raise ValueError(f"device must be a CUDA device, got {dev}")
+    index = dev.index if dev.index is not None else torch.cuda.current_device()
+    shapes, offs, total = [], [], 0
+    for i, a in enumerate(arrs):
+        v = [C.c_int() for _ in range(3)]
+        rc = lib.vitdet_jpeg_info(C.c_void_p(a.ctypes.data), int(a.size), *[C.byref(x) for x in v])
+        if rc:
+            msg = lib.vitdet_last_error()
+            raise _capi.VitdetError(rc, f"file {i}: " + (msg.decode("utf-8", "replace") if msg else ""))
+        shapes.append((v[0].value, v[1].value, 3))
+        offs.append(total)
+        total += (v[0].value * v[1].value * 3 + 255) // 256 * 256
+    with torch.cuda.device(index):
+        buf = torch.empty(total, dtype=torch.uint8, device=dev)
+        off_c = (C.c_int64 * len(arrs))(*offs)
+        _capi.check(lib.vitdet_decode_jpeg(_decoder(index), _jpeg_table(arrs), len(arrs), C.c_void_p(buf.data_ptr()), off_c,
+                                           _torch_stream_ptr(dev)))
+    return [buf[o:o + h * w * 3].view(h, w, 3) for o, (h, w, _) in zip(offs, shapes)]
