@@ -303,6 +303,24 @@ int vitdet_decode_jpeg(vitdet_handle* h, const vitdet_jpeg* files, int B, uint8_
  * completed by vitdet_collect; page-locked files must stay valid until then. */
 int vitdet_submit_jpeg_host(vitdet_handle* h, const vitdet_jpeg* files, int B, int mode, const vitdet_decode_params* params,
                             int want_packed, float* boxes_original_host, void* stream, int* ticket);
+/* Decode at reduced scale in the DCT domain, what tf.image.decode_jpeg(ratio=r) and PIL's Image.draft() return:
+ * ratios[i] (HOST) is 1, 2, 4 or 8, or 0 for auto.  File i then decodes to ceil(height / r) x ceil(width / r), bit-identical
+ * to libjpeg-turbo at scale 1 / r: its reduced IDCTs (jidctred.c 4x4, 2x2, 1x1), each component at its own DCT scaled size
+ * (jdmaster.c; 4:2:0 chroma at r >= 2 needs no upsampling) and fancy upsampling only where the luma's scaled size is above
+ * 1.  Auto is vitdet_jpeg_auto_ratio for the handle's model input size.  Another ratio fails the list with
+ * VITDET_E_INVALID naming the file, before anything is copied or launched; ratio 1 is exactly vitdet_decode_jpeg /
+ * vitdet_submit_jpeg_host.  The same launches whatever the ratios.  boxes_original stays in the file's pixels: the box on
+ * the decoded image, clipped, times float32(width) / float32(decoded width) (height likewise), clipped to [0, width] x
+ * [0, height].  Not supported: EXIF orientation, libjpeg's other N/8 scalings, cropping in the DCT domain. */
+int vitdet_decode_jpeg_scaled(vitdet_handle* h, const vitdet_jpeg* files, const int32_t* ratios, int B, uint8_t* out_dev,
+                              const int64_t* out_offsets, void* stream);
+int vitdet_submit_jpeg_host_scaled(vitdet_handle* h, const vitdet_jpeg* files, const int32_t* ratios, int B, int mode,
+                                   const vitdet_decode_params* params, int want_packed, float* boxes_original_host, void* stream,
+                                   int* ticket);
+/* Host only: the ratio PIL's draft(mode, (rw, rh)) picks for an height x width file letterboxed to target_h x target_w —
+ * the largest of 8, 4, 2, 1 at most min(width / rw, height / rh), (rh, rw) the resized size of
+ * vitdet_resize_with_pad_geometry; 1 when that size is empty.  VITDET_E_INVALID for a size that is not positive. */
+int vitdet_jpeg_auto_ratio(int height, int width, int target_h, int target_w);
 /* Counters of the last JPEG decode on this handle (synchronises with it): stats[0] subsequences of the parallel Huffman
  * decode, stats[1] subsequences re-decoded from a start other than their speculative one (sync passes and repair),
  * stats[2] symbols re-decoded. */

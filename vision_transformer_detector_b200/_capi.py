@@ -136,6 +136,10 @@ SYMBOLS = {
     "vitdet_decode_jpeg": (C.c_int, [_P, C.POINTER(Jpeg), C.c_int, _P, _P, _P]),
     "vitdet_submit_jpeg_host": (C.c_int, [_P, C.POINTER(Jpeg), C.c_int, C.c_int, C.POINTER(DecodeParams), C.c_int, _P, _P,
                                           C.POINTER(C.c_int)]),
+    "vitdet_decode_jpeg_scaled": (C.c_int, [_P, C.POINTER(Jpeg), _P, C.c_int, _P, _P, _P]),
+    "vitdet_submit_jpeg_host_scaled": (C.c_int, [_P, C.POINTER(Jpeg), _P, C.c_int, C.c_int, C.POINTER(DecodeParams), C.c_int, _P,
+                                                 _P, C.POINTER(C.c_int)]),
+    "vitdet_jpeg_auto_ratio": (C.c_int, [C.c_int, C.c_int, C.c_int, C.c_int]),
     "vitdet_jpeg_stats": (C.c_int, [_P, _P]),
     "vitdet_gather_detections": (C.c_int, [_P, _P, C.c_int, _P, _P]),
     "vitdet_nccl_unique_id": (C.c_int, [C.c_char_p]),

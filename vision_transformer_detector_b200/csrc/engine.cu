@@ -1744,13 +1744,15 @@ int vitdet_submit_images_host(vitdet_handle* h, const vitdet_image* images, int 
     return submit_host_impl(h, in, 1, B, mode, params, want_packed, boxes_original_host, stream, ticket);
 }
 
-// A caller's list of JPEG files -> the batch plan (every file parsed on the host; a rejected file fails the list, naming it)
-static int jpeg_files_plan(const char* fn, const vitdet_jpeg* files, int B, const int64_t* out_offsets, JpegBatch* jb) {
+// A caller's list of JPEG files -> the batch plan (every file parsed on the host; a rejected file fails the list, naming it).
+// ratios: null (all 1) or per file 1, 2, 4, 8 or 0 (auto for the model's input size).
+static int jpeg_files_plan(const vitdet_handle* h, const char* fn, const vitdet_jpeg* files, const int32_t* ratios, int B,
+                           const int64_t* out_offsets, JpegBatch* jb) {
     if (!files || B <= 0) return fail(VITDET_E_INVALID, "%s: %s", fn, !files ? "files is null" : "B must be positive");
     std::vector<const uint8_t*> data(B);
     std::vector<int64_t> bytes(B);
     for (int i = 0; i < B; ++i) { data[i] = files[i].data; bytes[i] = files[i].bytes; }
-    return jpeg_plan(fn, data.data(), bytes.data(), B, out_offsets, jb);
+    return jpeg_plan(fn, data.data(), bytes.data(), B, ratios, h->cfg.image_h, h->cfg.image_w, out_offsets, jb);
 }
 
 int vitdet_jpeg_info(const uint8_t* data, int64_t bytes, int* height, int* width, int* components) {
@@ -1759,15 +1761,22 @@ int vitdet_jpeg_info(const uint8_t* data, int64_t bytes, int* height, int* width
     return 0;
 }
 
-int vitdet_decode_jpeg(vitdet_handle* h, const vitdet_jpeg* files, int B, uint8_t* out_dev, const int64_t* out_offsets, void* stream) {
-    if (!h || !out_dev || !out_offsets) return fail(VITDET_E_INVALID, "decode_jpeg: null handle, out_dev or out_offsets");
+int vitdet_jpeg_auto_ratio(int height, int width, int target_h, int target_w) {
+    if (height <= 0 || width <= 0 || target_h <= 0 || target_w <= 0)
+        return fail(VITDET_E_INVALID, "jpeg_auto_ratio: sizes must be positive, got %d x %d to %d x %d", height, width, target_h, target_w);
+    return jpeg_auto_ratio(height, width, target_h, target_w);
+}
+
+static int decode_jpeg_impl(vitdet_handle* h, const char* fn, const vitdet_jpeg* files, const int32_t* ratios, int B, uint8_t* out_dev,
+                            const int64_t* out_offsets, void* stream) {
+    if (!h || !out_dev || !out_offsets) return fail(VITDET_E_INVALID, "%s: null handle, out_dev or out_offsets", fn);
     int cur = -1;
     CU_TRY(cudaGetDevice(&cur));
-    if (cur != h->device) return fail(VITDET_E_INVALID, "decode_jpeg: the handle lives on device %d but the current CUDA device is %d", h->device, cur);
+    if (cur != h->device) return fail(VITDET_E_INVALID, "%s: the handle lives on device %d but the current CUDA device is %d", fn, h->device, cur);
     JpegBatch jb;
-    RC_TRY(jpeg_files_plan("decode_jpeg", files, B, out_offsets, &jb));
+    RC_TRY(jpeg_files_plan(h, fn, files, ratios, B, out_offsets, &jb));
     for (int i = 0; i < B; ++i)
-        if (out_offsets[i] < 0) return fail(VITDET_E_INVALID, "decode_jpeg: image %d: negative output offset", i);
+        if (out_offsets[i] < 0) return fail(VITDET_E_INVALID, "%s: image %d: negative output offset", fn, i);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     // the previous decode has read the staging and the device buffers before they are reused, on any stream
     if (h->jpeg_done) CU_TRY(cudaEventSynchronize(h->jpeg_done));
@@ -1797,26 +1806,54 @@ int vitdet_decode_jpeg(vitdet_handle* h, const vitdet_jpeg* files, int B, uint8_
     return 0;
 }
 
-int vitdet_submit_jpeg_host(vitdet_handle* h, const vitdet_jpeg* files, int B, int mode, const vitdet_decode_params* params,
-                            int want_packed, float* boxes_original_host, void* stream, int* ticket) {
-    if (!h || !params || !ticket) return fail(VITDET_E_INVALID, "submit_jpeg_host: handle, params and ticket must not be null");
+int vitdet_decode_jpeg(vitdet_handle* h, const vitdet_jpeg* files, int B, uint8_t* out_dev, const int64_t* out_offsets, void* stream) {
+    return decode_jpeg_impl(h, "decode_jpeg", files, nullptr, B, out_dev, out_offsets, stream);
+}
+
+int vitdet_decode_jpeg_scaled(vitdet_handle* h, const vitdet_jpeg* files, const int32_t* ratios, int B, uint8_t* out_dev,
+                              const int64_t* out_offsets, void* stream) {
+    if (!ratios) return fail(VITDET_E_INVALID, "decode_jpeg_scaled: ratios is null");
+    return decode_jpeg_impl(h, "decode_jpeg_scaled", files, ratios, B, out_dev, out_offsets, stream);
+}
+
+static int submit_jpeg_impl(vitdet_handle* h, const char* fn, const vitdet_jpeg* files, const int32_t* ratios, int B, int mode,
+                            const vitdet_decode_params* params, int want_packed, float* boxes_original_host, void* stream, int* ticket) {
+    if (!h || !params || !ticket) return fail(VITDET_E_INVALID, "%s: handle, params and ticket must not be null", fn);
     const int th = h->cfg.image_h, tw = h->cfg.image_w;
     if (boxes_original_host && (params->image_h != static_cast<float>(th) || params->image_w != static_cast<float>(tw)))
-        return fail(VITDET_E_INVALID, "submit_jpeg_host: boxes_original needs the decode at the model's input size %d x %d (params image_h / image_w)", th, tw);
+        return fail(VITDET_E_INVALID, "%s: boxes_original needs the decode at the model's input size %d x %d (params image_h / image_w)", fn, th, tw);
     JpegBatch jb;
-    RC_TRY(jpeg_files_plan("submit_jpeg_host", files, B, nullptr, &jb));
+    RC_TRY(jpeg_files_plan(h, fn, files, ratios, B, nullptr, &jb));
     HostImages in;
     in.table.resize(B);
     in.src.resize(B);
     in.offs.assign(jb.file_off.begin(), jb.file_off.end());
     for (int i = 0; i < B; ++i) {
         in.src[i] = reinterpret_cast<const char*>(files[i].data);
-        if (!letterbox_image(nullptr, jb.height[i], jb.width[i], th, tw, &in.table[i]))
-            return fail(VITDET_E_INVALID, "submit_jpeg_host: image %d: a %d x %d image letterboxed to %d x %d resizes to %d x %d pixels", i,
-                        jb.height[i], jb.width[i], th, tw, in.table[i].rh, in.table[i].rw);
+        LetterboxImage& g = in.table[i];
+        if (!letterbox_image(nullptr, jb.height[i], jb.width[i], th, tw, &g))
+            return fail(VITDET_E_INVALID, "%s: image %d: a %d x %d image letterboxed to %d x %d resizes to %d x %d pixels", fn, i,
+                        jb.height[i], jb.width[i], th, tw, g.rh, g.rw);
+        // boxes_original in the file's pixels: the decoded image's box times file size / decoded size (1 at ratio 1)
+        g.file_h = jb.file_height[i];
+        g.file_w = jb.file_width[i];
+        g.file_hscale = static_cast<float>(g.file_h) / static_cast<float>(g.h);
+        g.file_wscale = static_cast<float>(g.file_w) / static_cast<float>(g.w);
     }
     in.jpeg = &jb;
     return submit_host_impl(h, in, 1, B, mode, params, want_packed, boxes_original_host, stream, ticket);
+}
+
+int vitdet_submit_jpeg_host(vitdet_handle* h, const vitdet_jpeg* files, int B, int mode, const vitdet_decode_params* params,
+                            int want_packed, float* boxes_original_host, void* stream, int* ticket) {
+    return submit_jpeg_impl(h, "submit_jpeg_host", files, nullptr, B, mode, params, want_packed, boxes_original_host, stream, ticket);
+}
+
+int vitdet_submit_jpeg_host_scaled(vitdet_handle* h, const vitdet_jpeg* files, const int32_t* ratios, int B, int mode,
+                                   const vitdet_decode_params* params, int want_packed, float* boxes_original_host, void* stream,
+                                   int* ticket) {
+    if (!ratios) return fail(VITDET_E_INVALID, "submit_jpeg_host_scaled: ratios is null");
+    return submit_jpeg_impl(h, "submit_jpeg_host_scaled", files, ratios, B, mode, params, want_packed, boxes_original_host, stream, ticket);
 }
 
 int vitdet_jpeg_stats(vitdet_handle* h, int64_t* stats) {

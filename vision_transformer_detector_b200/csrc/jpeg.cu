@@ -19,6 +19,14 @@
 //   6 dc       one CTA per segment: the DC values, a prefix of the differences per component, reset at every segment
 //   7 idct     one thread per block: dequantisation, jidctint.c ISLOW, jdmaster.c's range-limit table -> component planes
 //   8 colour   one thread per pixel: jdsample.c fancy upsampling and jdcolor.c ycc_rgb_convert -> (h, w, 3) uint8
+// A file may be decoded at 1/2, 1/4 or 1/8 scale in the DCT domain (libjpeg's scale_denom, what PIL's draft() and
+// tf.image.decode_jpeg(ratio=) ask for), mixed freely within a batch and in the same launches.  The output is then
+// ceil(h / ratio) x ceil(w / ratio).  Each component gets its own DCT scaled size as jdmaster.c sets it: the luma's
+// k = 8 / ratio, doubled while both sampling ratios allow, so 4:2:0 chroma keeps 8 x 8 blocks at ratio 2 and is not
+// upsampled.  The idct kernel writes 8 x 8 (ISLOW), 4 x 4, 2 x 2 or 1 x 1 (jidctred.c) blocks.  A block whose IDCT is
+// 1 x 1 reads its DC alone, so the write and DC kernels store one coefficient for it instead of 64.  The Huffman decode
+// is the same at every scale.  The colour kernel upsamples by each component's own expansion factors, fancily only
+// where the luma's scaled size is above 1 (jinit_upsampler).  oracle/jpeg_scaled_oracle.py states the reduced decode.
 // The state at a symbol boundary is (bit offset, block index u within the MCU, coefficient index k); the exact start of
 // subsequence j + 1 is the exit of subsequence j decoded from its exact start, so the result equals a sequential decode by
 // construction.  Every decode loop ends at the end of its subsequence (each symbol consumes at least one bit); corrupt data
@@ -65,13 +73,22 @@ struct JpegHuff {
 enum : int { kSpaceYcc = 0, kSpaceRgb = 1, kSpaceGray = 2 };
 
 struct JpegImage {
-    int32_t h, w, ncomp, space;
+    int32_t h, w, ncomp, space;      // h, w: the output's size, ceil(file size / ratio)
     int32_t hs[3], vs[3], hmax, vmax, mcux, mcuy;
     int32_t bpm;                     // blocks per MCU
     int8_t blk_c[8], blk_x[8], blk_y[8];   // per block of an MCU: component, column and row in its MCU cell
+    int16_t blk_coef[8];             // per block of an MCU: its first coefficient relative to the MCU's
+    // coefficients stored per MCU: 64 per block (starting at a multiple of 8: read as 16-byte words), 1 per block whose
+    // IDCT reads the DC alone; a multiple of 8 when the MCU holds a 64-coefficient block
+    int32_t mcu_coefs;
     int32_t dc[3], ac[3];            // Huffman tables of each component (indices into the batch's table array)
+    // per component at the decode's scale (jdmaster.c jpeg_core_output_dimensions): DCT scaled size (8, 4, 2 or 1), plane
+    // pitch (mcux * hs * size), scaled width and height, expansion factors to the output (1 or 2; jdsample.c)
+    int32_t ks[3], pitch[3], dw[3], dh[3], he[3], ve[3];
+    int32_t fancy;                   // jdsample.c fancy upsampling allowed: the luma's scaled size is above 1
     int64_t block0;                  // first coefficient block of the image
-    int64_t plane[3];                // byte offset of each component plane (pitch mcux * hs * 8)
+    int64_t coef0;                   // first coefficient of the image (a multiple of 8)
+    int64_t plane[3];                // byte offset of each component plane
     int64_t out;                     // byte offset of the image's pixels in the output
     int64_t pix0;                    // first pixel of the image in the batch
     uint16_t q[3][64];               // quantisation tables, natural order
@@ -80,7 +97,7 @@ struct JpegImage {
 struct JpegSegment {
     int64_t src;                     // first byte in the concatenated files
     int64_t dst;                     // first byte of its compact stream (8-byte aligned)
-    int64_t block0;                  // first coefficient block
+    int64_t coef0;                   // first coefficient (its first MCU's)
     int32_t src_len, nbits, nblocks, sub0, image, pad;
 };
 
@@ -385,8 +402,14 @@ __global__ void __launch_bounds__(kDestuffThreads) jpeg_destuff_kernel(JpegBatch
     if (blockIdx.x == 0 && threadIdx.x < 3) stats[threadIdx.x] = threadIdx.x == 0 ? b.nsub : 0;
     for (int si = blockIdx.x; si < b.nseg; si += gridDim.x) {
         const JpegSegment sg = b.seg[si];
-        int4* z = reinterpret_cast<int4*>(coef + sg.block0 * 64);
-        for (int64_t i = threadIdx.x; i < static_cast<int64_t>(sg.nblocks) * 8; i += kDestuffThreads) z[i] = make_int4(0, 0, 0, 0);
+        const JpegImage& im = b.img[sg.image];
+        const int64_t ncoef = static_cast<int64_t>(sg.nblocks / im.bpm) * im.mcu_coefs;
+        if (((sg.coef0 | ncoef) & 7) == 0) {
+            int4* z = reinterpret_cast<int4*>(coef + sg.coef0);
+            for (int64_t i = threadIdx.x; i < ncoef / 8; i += kDestuffThreads) z[i] = make_int4(0, 0, 0, 0);
+        } else {                     // DC-only blocks: a segment's coefficients need not fill whole 16-byte words
+            for (int64_t i = threadIdx.x; i < ncoef; i += kDestuffThreads) coef[sg.coef0 + i] = 0;
+        }
         const uint8_t* src = files + sg.src;
         uint8_t* dst = reinterpret_cast<uint8_t*>(compact + sg.dst);
         if (threadIdx.x == 0) carry = 0;
@@ -584,11 +607,29 @@ __global__ void __launch_bounds__(128) jpeg_write_kernel(JpegBatchDev b, const c
     const int4 a = starts[g];
     DecState st{a.x, a.y, a.z};
     int blk = a.w, idx, val;
-    int16_t* base = coef + sg.block0 * 64;
+    if (im.mcu_coefs == im.bpm * 64) {               // every block keeps 64 coefficients, back to back
+        int16_t* base = coef + sg.coef0;
+        while (st.pos < end && blk < sg.nblocks) {
+            const int b_now = blk;
+            blk += step(im, b.tab, s, st, &idx, &val);
+            if (idx >= 0) base[static_cast<int64_t>(b_now) * 64 + idx] = static_cast<int16_t>(val);
+        }
+        return;
+    }
+    // the current block's coefficients: 64, or the DC alone where the component's IDCT reads nothing else
+    int u = blk % im.bpm;
+    int16_t* mcu = coef + sg.coef0 + static_cast<int64_t>(blk / im.bpm) * im.mcu_coefs;
+    int16_t* p = mcu + im.blk_coef[u];
+    int last = im.ks[im.blk_c[u]] == 1 ? 0 : 63;
     while (st.pos < end && blk < sg.nblocks) {
-        const int b_now = blk;
-        blk += step(im, b.tab, s, st, &idx, &val);
-        if (idx >= 0) base[static_cast<int64_t>(b_now) * 64 + idx] = static_cast<int16_t>(val);
+        const bool done = step(im, b.tab, s, st, &idx, &val);
+        if (idx >= 0 && idx <= last) p[idx] = static_cast<int16_t>(val);
+        if (done) {
+            ++blk;
+            if (++u == im.bpm) { u = 0; mcu += im.mcu_coefs; }
+            p = mcu + im.blk_coef[u];
+            last = im.ks[im.blk_c[u]] == 1 ? 0 : 63;
+        }
     }
 }
 
@@ -607,19 +648,19 @@ __global__ void __launch_bounds__(kDcThreads) jpeg_dc_kernel(JpegBatchDev b, int
         const JpegSegment& sg = b.seg[si];
         const JpegImage& im = b.img[sg.image];
         const int nmcu = sg.nblocks / im.bpm;
-        int16_t* base = coef + sg.block0 * 64;
+        int16_t* base = coef + sg.coef0;
         Dc3 carry{0u, 0u, 0u};
         for (int m0 = 0; m0 < nmcu; m0 += kDcThreads) {
             const int m = m0 + threadIdx.x;
             unsigned sum[3] = {0u, 0u, 0u};
             if (m < nmcu)
-                for (int u = 0; u < im.bpm; ++u) sum[im.blk_c[u]] += static_cast<unsigned>(static_cast<int>(base[(static_cast<int64_t>(m) * im.bpm + u) * 64]));
+                for (int u = 0; u < im.bpm; ++u) sum[im.blk_c[u]] += static_cast<unsigned>(static_cast<int>(base[static_cast<int64_t>(m) * im.mcu_coefs + im.blk_coef[u]]));
             Dc3 pre, tot;
             Scan(tmp).ExclusiveScan(Dc3{sum[0], sum[1], sum[2]}, pre, Dc3{0u, 0u, 0u}, Dc3Add(), tot);
             unsigned run[3] = {carry.a + pre.a, carry.b + pre.b, carry.c + pre.c};
             if (m < nmcu)
                 for (int u = 0; u < im.bpm; ++u) {
-                    int16_t* p = base + (static_cast<int64_t>(m) * im.bpm + u) * 64;
+                    int16_t* p = base + static_cast<int64_t>(m) * im.mcu_coefs + im.blk_coef[u];
                     run[im.blk_c[u]] += static_cast<unsigned>(static_cast<int>(*p));
                     *p = static_cast<int16_t>(run[im.blk_c[u]]);
                 }
@@ -665,17 +706,97 @@ __device__ __forceinline__ int find_image(const JpegImage* img, int B, int64_t v
     return lo;
 }
 
-__global__ void __launch_bounds__(128) jpeg_idct_kernel(JpegBatchDev b, long long nblocks, const int16_t* __restrict__ coef, uint8_t* planes) {
+// jidctred.c jpeg_idct_4x4 / jpeg_idct_2x2 on one column or row (CONST_BITS 13, PASS1_BITS 2): the 4-point form reads
+// inputs 0-3 and 5-7, the 2-point form 0, 1, 3, 5 and 7
+__device__ __forceinline__ void idct4_1d(jlong s0, jlong s1, jlong s2, jlong s3, jlong s5, jlong s6, jlong s7, jlong* o) {
+    const jlong tmp0 = s0 * 16384, tmp2 = s2 * 15137 + s6 * -6270;
+    const jlong t10 = tmp0 + tmp2, t12 = tmp0 - tmp2;
+    const jlong a = s7 * -1730 + s5 * 11893 + s3 * -17799 + s1 * 8697;
+    const jlong c = s7 * -4176 + s5 * -4926 + s3 * 7373 + s1 * 20995;
+    o[0] = t10 + c; o[1] = t12 + a; o[2] = t12 - a; o[3] = t10 - c;
+}
+
+__device__ __forceinline__ void idct2_1d(jlong s0, jlong s1, jlong s3, jlong s5, jlong s7, jlong* o) {
+    const jlong t10 = s0 * 32768, t0 = s7 * -5906 + s5 * 6967 + s3 * -10426 + s1 * 29692;
+    o[0] = t10 + t0; o[1] = t10 - t0;
+}
+
+// 4 x 4 output of one block: x dequantised, natural order
+__device__ __forceinline__ void idct_4x4(const int* x, uint8_t* dst, int pitch) {
+    jlong ws[32], o[4];
+#pragma unroll
+    for (int col = 0; col < 8; ++col) {              // pass 1: columns (column 4 is not read by pass 2)
+        if (col == 4) continue;
+        idct4_1d(x[col], x[8 + col], x[16 + col], x[24 + col], x[40 + col], x[48 + col], x[56 + col], o);
+#pragma unroll
+        for (int r = 0; r < 4; ++r) ws[r * 8 + col] = (o[r] + (1 << 11)) >> 12;
+    }
+#pragma unroll
+    for (int r = 0; r < 4; ++r) {                    // pass 2: rows
+        idct4_1d(ws[r * 8], ws[r * 8 + 1], ws[r * 8 + 2], ws[r * 8 + 3], ws[r * 8 + 5], ws[r * 8 + 6], ws[r * 8 + 7], o);
+        *reinterpret_cast<uint32_t*>(dst + static_cast<int64_t>(r) * pitch) =
+            range_limit((o[0] + (1 << 18)) >> 19) | range_limit((o[1] + (1 << 18)) >> 19) << 8 |
+            range_limit((o[2] + (1 << 18)) >> 19) << 16 | range_limit((o[3] + (1 << 18)) >> 19) << 24;
+    }
+}
+
+// 2 x 2 output of one block
+__device__ __forceinline__ void idct_2x2(const int* x, uint8_t* dst, int pitch) {
+    jlong ws[16], o[2];
+#pragma unroll
+    for (int col = 0; col < 8; ++col) {              // pass 1: columns 0, 1, 3, 5, 7
+        if (col != 0 && !(col & 1)) continue;
+        idct2_1d(x[col], x[8 + col], x[24 + col], x[40 + col], x[56 + col], o);
+        ws[col] = (o[0] + (1 << 12)) >> 13;
+        ws[8 + col] = (o[1] + (1 << 12)) >> 13;
+    }
+#pragma unroll
+    for (int r = 0; r < 2; ++r) {                    // pass 2: rows
+        idct2_1d(ws[r * 8], ws[r * 8 + 1], ws[r * 8 + 3], ws[r * 8 + 5], ws[r * 8 + 7], o);
+        *reinterpret_cast<uint16_t*>(dst + static_cast<int64_t>(r) * pitch) =
+            static_cast<uint16_t>(range_limit((o[0] + (1 << 19)) >> 20) | range_limit((o[1] + (1 << 19)) >> 20) << 8);
+    }
+}
+
+// The 4 x 4 and 2 x 2 blocks of a reduced decode, out of line: the 8 x 8 path of jpeg_idct_kernel keeps its registers
+__device__ __noinline__ void idct_reduced(const int16_t* __restrict__ blk, const uint16_t* q, int k, uint8_t* dst, int pitch) {
+    int x[64];                                       // dequantised as in jpeg_idct_kernel; rows not read stay 0
+#pragma unroll
+    for (int i = 0; i < 64; ++i) x[i] = 0;
+#pragma unroll
+    for (int r = 0; r < 8; ++r) {                    // rows the reduced forms read: 0-3, 5-7 (4 x 4), 0, 1, 3, 5, 7 (2 x 2)
+        if (r == 4 || (k == 2 && r != 0 && !(r & 1))) continue;
+        const int4 v = reinterpret_cast<const int4*>(blk)[r];
+        const int w[4] = {v.x, v.y, v.z, v.w};
+#pragma unroll
+        for (int t = 0; t < 4; ++t) {
+            x[r * 8 + 2 * t] = static_cast<int16_t>(w[t] & 0xFFFF) * static_cast<int>(q[r * 8 + 2 * t]);
+            x[r * 8 + 2 * t + 1] = (w[t] >> 16) * static_cast<int>(q[r * 8 + 2 * t + 1]);
+        }
+    }
+    if (k == 4) idct_4x4(x, dst, pitch);
+    else idct_2x2(x, dst, pitch);
+}
+
+// five CTAs per SM, as the 8 x 8 path alone compiles to (96 registers)
+__global__ void __launch_bounds__(128, 5) jpeg_idct_kernel(JpegBatchDev b, long long nblocks, const int16_t* __restrict__ coef, uint8_t* planes) {
     const long long gb = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
     if (gb >= nblocks) return;
     const JpegImage& im = b.img[find_image(b.img, b.B, gb, false)];
     const long long local = gb - im.block0;
     const int mcu = static_cast<int>(local / im.bpm), u = static_cast<int>(local % im.bpm);
     const int c = im.blk_c[u];
-    const int pitch = im.mcux * im.hs[c] * 8;
-    const int px = ((mcu % im.mcux) * im.hs[c] + im.blk_x[u]) * 8, py = ((mcu / im.mcux) * im.vs[c] + im.blk_y[u]) * 8;
+    const int k = im.ks[c], pitch = im.pitch[c];
+    const int px = ((mcu % im.mcux) * im.hs[c] + im.blk_x[u]) * k, py = ((mcu / im.mcux) * im.vs[c] + im.blk_y[u]) * k;
+    const int16_t* blk = coef + im.coef0 + static_cast<int64_t>(mcu) * im.mcu_coefs + im.blk_coef[u];
+    if (k == 1) {                                    // jidctred.c jpeg_idct_1x1: the DC alone, one coefficient stored
+        planes[im.plane[c] + static_cast<int64_t>(py) * pitch + px] =
+            static_cast<uint8_t>(range_limit((static_cast<jlong>(*blk) * im.q[c][0] + 4) >> 3));
+        return;
+    }
+    if (k < 8) { idct_reduced(blk, im.q[c], k, planes + im.plane[c] + static_cast<int64_t>(py) * pitch + px, pitch); return; }
     int x[64];                                       // dequantised: int16 * uint16 fits 32 bits
-    const int4* src = reinterpret_cast<const int4*>(coef + gb * 64);
+    const int4* src = reinterpret_cast<const int4*>(blk);
 #pragma unroll
     for (int i = 0; i < 8; ++i) {
         const int4 v = src[i];
@@ -709,10 +830,13 @@ __global__ void __launch_bounds__(128) jpeg_idct_kernel(JpegBatchDev b, long lon
 // ------------------------------------------------------------------------------------------------
 // 8 upsampling (jdsample.c) and colour conversion (jdcolor.c)
 // ------------------------------------------------------------------------------------------------
-__device__ __forceinline__ int chroma(const uint8_t* pl, int pitch, int he, int ve, int dw, int dh, int x, int y) {
+// One chroma sample of output pixel (x, y): pl is the component's plane at its DCT scaled size, dw x dh samples, expanded by
+// (he, ve) to the output.  jinit_upsampler replicates when fancy upsampling is off (the luma's scaled size is 1) or the
+// component is at most 2 samples wide.
+__device__ __forceinline__ int chroma(const uint8_t* pl, int pitch, int he, int ve, bool fancy, int dw, int dh, int x, int y) {
     if (he == 1 && ve == 1) return pl[static_cast<int64_t>(y) * pitch + x];
     const int i = x >> 1;
-    if (dw <= 2) return pl[static_cast<int64_t>(y / ve) * pitch + i];     // jinit_upsampler: plain replication
+    if (!fancy || dw <= 2) return pl[static_cast<int64_t>(y / ve) * pitch + i];     // plain replication
     const bool even = (x & 1) == 0;
     const int nb = min(max(even ? i - 1 : i + 1, 0), dw - 1);
     const bool first = even && i == 0, last = !even && i == dw - 1;
@@ -737,15 +861,11 @@ __global__ void __launch_bounds__(256) jpeg_color_kernel(JpegBatchDev b, long lo
     const JpegImage& im = b.img[find_image(b.img, b.B, gp, true)];
     const int64_t local = gp - im.pix0;
     const int y = static_cast<int>(local / im.w), x = static_cast<int>(local % im.w);
-    const int p0 = im.mcux * im.hs[0] * 8;
-    const int Y = planes[im.plane[0] + static_cast<int64_t>(y) * p0 + x];
+    const int Y = planes[im.plane[0] + static_cast<int64_t>(y) * im.pitch[0] + x];
     uint8_t* o = out + im.out + local * 3;
     if (im.space == kSpaceGray) { o[0] = o[1] = o[2] = static_cast<uint8_t>(Y); return; }
-    const int he = im.hmax, ve = im.vmax;
-    const int dw = (im.w + he - 1) / he, dh = (im.h + ve - 1) / ve;
-    const int pc = im.mcux * 8;
-    const int cb = chroma(planes + im.plane[1], pc, he, ve, dw, dh, x, y);
-    const int cr = chroma(planes + im.plane[2], pc, he, ve, dw, dh, x, y);
+    const int cb = chroma(planes + im.plane[1], im.pitch[1], im.he[1], im.ve[1], im.fancy, im.dw[1], im.dh[1], x, y);
+    const int cr = chroma(planes + im.plane[2], im.pitch[2], im.he[2], im.ve[2], im.fancy, im.dw[2], im.dh[2], x, y);
     if (im.space == kSpaceRgb) { o[0] = static_cast<uint8_t>(Y); o[1] = static_cast<uint8_t>(cb); o[2] = static_cast<uint8_t>(cr); return; }
     const int xb = cb - 128, xr = cr - 128;
     const int r = Y + ((91881 * xr + 32768) >> 16);
@@ -770,16 +890,31 @@ int jpeg_info(const uint8_t* data, int64_t bytes, int* height, int* width, int* 
     return 0;
 }
 
-int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, int B, const int64_t* out_offsets, JpegBatch* b) {
+int jpeg_auto_ratio(int h, int w, int th, int tw) {
+    int rh, rw, ph, pw;
+    resize_with_pad_geometry(h, w, th, tw, &rh, &rw, &ph, &pw);
+    if (rh <= 0 || rw <= 0) return 1;
+    const int scale = std::min(w / rw, h / rh);
+    return scale >= 8 ? 8 : scale >= 4 ? 4 : scale >= 2 ? 2 : 1;
+}
+
+int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, int B, const int32_t* ratios, int target_h,
+              int target_w, const int64_t* out_offsets, JpegBatch* b) {
+    for (int i = 0; ratios && i < B; ++i)
+        if (ratios[i] != 0 && ratios[i] != 1 && ratios[i] != 2 && ratios[i] != 4 && ratios[i] != 8)
+            return fail(VITDET_E_INVALID, "%s: file %d: ratio %d (expected 1, 2, 4, 8 or 0 for auto)", fn, i, ratios[i]);
     std::vector<JpegImage> imgs(B);
     std::vector<JpegSegment> segs;
     std::vector<JpegHuff> tabs;
     b->B = B;
     b->height.assign(B, 0);
     b->width.assign(B, 0);
+    b->file_height.assign(B, 0);
+    b->file_width.assign(B, 0);
+    b->ratio.assign(B, 1);
     b->file_off.assign(B + 1, 0);
     b->rgb_off.assign(B, 0);
-    size_t compact = 0, planes = 0, rgb = 0;
+    size_t compact = 0, planes = 0, rgb = 0, coefs = 0;
     long long nblocks = 0, npix = 0;
     int nsub = 0;
     char why[256];
@@ -790,7 +925,11 @@ int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, 
         b->file_off[i + 1] = b->file_off[i] + static_cast<size_t>(bytes[i]);
         JpegImage& im = imgs[i];
         memset(&im, 0, sizeof(im));
-        im.h = P.h; im.w = P.w; im.ncomp = P.ncomp; im.space = P.space;
+        int ratio = ratios ? ratios[i] : 1;
+        if (ratio == 0) ratio = jpeg_auto_ratio(P.h, P.w, target_h, target_w);
+        // the output ceil(h / ratio) x ceil(w / ratio); the luma's DCT scaled size k = 8 / ratio
+        const int k = 8 / ratio;
+        im.h = (P.h + ratio - 1) / ratio; im.w = (P.w + ratio - 1) / ratio; im.ncomp = P.ncomp; im.space = P.space;
         im.hmax = im.vmax = 1;
         for (int c = 0; c < P.ncomp; ++c) {
             im.hs[c] = P.hs[c]; im.vs[c] = P.vs[c];
@@ -805,16 +944,42 @@ int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, 
         for (int c = 0; c < P.ncomp; ++c)
             for (int by = 0; by < im.vs[c]; ++by)
                 for (int bx = 0; bx < im.hs[c]; ++bx) { im.blk_c[im.bpm] = c; im.blk_x[im.bpm] = bx; im.blk_y[im.bpm] = by; ++im.bpm; }
+        // jdmaster.c jpeg_core_output_dimensions: each component's DCT scaled size starts at k and doubles while both
+        // sampling ratios allow it (4:2:0 chroma at ratio 2 takes 8 x 8 blocks and needs no upsampling); its scaled size
+        // is ceil(size * samp * scaled size / (max samp * 8)); jdsample.c expands it by max samp * k / (samp * scaled size)
+        im.fancy = k > 1;
+        for (int c = 0; c < P.ncomp; ++c) {
+            int ss = k;
+            while (ss < 8 && (im.hmax * k) % (im.hs[c] * ss * 2) == 0 && (im.vmax * k) % (im.vs[c] * ss * 2) == 0) ss *= 2;
+            im.ks[c] = ss;
+            im.pitch[c] = im.mcux * im.hs[c] * ss;
+            im.dw[c] = static_cast<int>((static_cast<long long>(P.w) * im.hs[c] * ss + im.hmax * 8 - 1) / (im.hmax * 8));
+            im.dh[c] = static_cast<int>((static_cast<long long>(P.h) * im.vs[c] * ss + im.vmax * 8 - 1) / (im.vmax * 8));
+            im.he[c] = im.hmax * k / (im.hs[c] * ss);
+            im.ve[c] = im.vmax * k / (im.vs[c] * ss);
+        }
+        im.mcu_coefs = 0;
+        bool full = false;
+        for (int u = 0; u < im.bpm; ++u) {
+            const bool dc_only = im.ks[im.blk_c[u]] == 1;
+            if (!dc_only) im.mcu_coefs = (im.mcu_coefs + 7) & ~7;
+            im.blk_coef[u] = static_cast<int16_t>(im.mcu_coefs);
+            im.mcu_coefs += dc_only ? 1 : 64;
+            full |= !dc_only;
+        }
+        if (full) im.mcu_coefs = (im.mcu_coefs + 7) & ~7;
         const long long nmcu = static_cast<long long>(im.mcux) * im.mcuy;
         im.block0 = nblocks;
+        im.coef0 = static_cast<int64_t>(coefs);
+        coefs += (static_cast<size_t>(nmcu) * im.mcu_coefs + 7) & ~static_cast<size_t>(7);
         for (int c = 0; c < P.ncomp; ++c) {
             im.plane[c] = static_cast<int64_t>(planes);
-            planes += a256(static_cast<size_t>(nmcu) * im.hs[c] * im.vs[c] * 64);
+            planes += a256(static_cast<size_t>(nmcu) * im.hs[c] * im.vs[c] * im.ks[c] * im.ks[c]);
         }
         im.pix0 = npix;
         b->rgb_off[i] = out_offsets ? static_cast<size_t>(out_offsets[i]) : rgb;
         im.out = static_cast<int64_t>(b->rgb_off[i]);
-        rgb += a256(static_cast<size_t>(P.h) * P.w * 3);
+        rgb += a256(static_cast<size_t>(im.h) * im.w * 3);
         const long long ri = P.ri ? P.ri : nmcu;
         const long long nseg = (nmcu + ri - 1) / ri;
         for (long long s = 0; s < nseg; ++s) {
@@ -827,7 +992,7 @@ int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, 
             sg.nbits = static_cast<int32_t>(clen * 8);
             sg.dst = static_cast<int64_t>(compact);
             compact += (static_cast<size_t>(clen) + 7) & ~static_cast<size_t>(7);
-            sg.block0 = nblocks + s * ri * im.bpm;
+            sg.coef0 = im.coef0 + s * ri * im.mcu_coefs;
             sg.nblocks = static_cast<int32_t>((std::min(nmcu, (s + 1) * ri) - s * ri) * im.bpm);
             sg.sub0 = nsub;
             sg.image = i;
@@ -835,9 +1000,12 @@ int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, 
             segs.push_back(sg);
         }
         nblocks += nmcu * im.bpm;
-        npix += static_cast<long long>(P.h) * P.w;
-        b->height[i] = P.h;
-        b->width[i] = P.w;
+        npix += static_cast<long long>(im.h) * im.w;
+        b->height[i] = im.h;
+        b->width[i] = im.w;
+        b->file_height[i] = P.h;
+        b->file_width[i] = P.w;
+        b->ratio[i] = ratio;
     }
     b->nseg = static_cast<int>(segs.size());
     b->nsub = nsub;
@@ -852,7 +1020,7 @@ int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, 
     memcpy(b->desc.data() + o_tab, tabs.data(), sizeof(JpegHuff) * tabs.size());
     b->o_compact = a256(desc_bytes);
     b->o_coef = b->o_compact + a256(compact);
-    b->o_spec = b->o_coef + a256(static_cast<size_t>(nblocks) * 128);
+    b->o_spec = b->o_coef + a256(coefs * sizeof(int16_t));
     b->o_check = b->o_spec + a256(sizeof(int2) * nsub);
     b->o_sync = b->o_check + a256(sizeof(int2) * kWordsPerSub * static_cast<size_t>(nsub));
     b->o_start = b->o_sync + 3 * a256(sizeof(int2) * nsub);

@@ -145,8 +145,14 @@ struct LetterboxImage {
     int h, w;
     int rh, rw, ph, pw;        // resize_with_pad_geometry
     float hscale, wscale;      // h / rh, w / rw in float32
+    // boxes_original goes to a file_h x file_w image of which this one is a reduced decode (a JPEG decoded at 1 / ratio):
+    // the box on this image, clipped, times file_h / h (file_w / w) in float32, clipped to the file's size.  Exactly 1
+    // and the image's own size otherwise, where the second step changes nothing.
+    int file_h, file_w;
+    float file_hscale, file_wscale;
 };
-// Fills *im for an h x w image letterboxed to th x tw; false when a size is not positive or the resized image is empty.
+// Fills *im for an h x w image letterboxed to th x tw (file size = image size); false when a size is not positive or the
+// resized image is empty.
 bool letterbox_image(const uint8_t* pixels, int h, int w, int th, int tw, LetterboxImage* im);
 // patchify of the letterboxed, normalised images without the float32 images: images is a DEVICE table of B entries,
 // the output the same patch matrix as patchify_launch's (vector layout only: rp and ldp multiples of 4, 16-byte aligned).
@@ -220,15 +226,21 @@ struct JpegBatch {
     int B = 0, nseg = 0, nsub = 0;
     long long nblocks = 0, npix = 0;
     std::vector<char> desc;
-    std::vector<int> height, width;
+    std::vector<int> height, width;    // of the decoded images: ceil(file size / ratio)
+    std::vector<int> file_height, file_width, ratio;
     std::vector<size_t> file_off;      // B + 1: file i is bytes [file_off[i], file_off[i + 1]) of the concatenated files
     std::vector<size_t> rgb_off;       // where image i's pixels go, relative to the output pointer of jpeg_decode
     size_t rgb_bytes = 0;              // with the default layout (out_offsets null): the output's size
     size_t o_compact = 0, o_coef = 0, o_spec = 0, o_check = 0, o_sync = 0, o_start = 0, o_planes = 0, o_stats = 0, work_bytes = 0;
 };
-// Parses B files (HOST bytes); out_offsets (may be null: images packed 256-byte aligned) place the outputs.  Fails with
-// VITDET_E_INVALID naming the first rejected file.
-int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, int B, const int64_t* out_offsets, JpegBatch* b);
+// Parses B files (HOST bytes); out_offsets (may be null: images packed 256-byte aligned) place the outputs.  ratios (may be
+// null: all 1) decode file i at 1 / ratios[i] scale in the DCT domain (1, 2, 4 or 8; 0: jpeg_auto_ratio for the target
+// size).  Fails with VITDET_E_INVALID naming the first file with an invalid ratio, else the first rejected file.
+int jpeg_plan(const char* fn, const uint8_t* const* data, const int64_t* bytes, int B, const int32_t* ratios, int target_h,
+              int target_w, const int64_t* out_offsets, JpegBatch* b);
+// The ratio PIL's draft() picks for an h x w file letterboxed to th x tw: the largest of 8, 4, 2, 1 at most
+// min(w / rw, h / rh) for the resized size (rh, rw) of resize_with_pad_geometry; 1 when that size is empty.
+int jpeg_auto_ratio(int h, int w, int th, int tw);
 // Launches the kJpegLaunches kernels: files_dev holds the concatenated files, work the scratch with b.desc at offset 0.
 cudaError_t jpeg_decode_launch(const JpegBatch& b, const char* files_dev, void* work, uint8_t* out, cudaStream_t stream);
 

@@ -493,11 +493,17 @@ __device__ __forceinline__ void decode_slot(const float (&l)[6], long long r, co
         const float half_h = __fdiv_rn(dec[4], 2.f), half_w = __fdiv_rn(dec[5], 2.f);
         const float pw = static_cast<float>(g.pw), ph = static_cast<float>(g.ph);
         const float sw = static_cast<float>(g.w), sh = static_cast<float>(g.h);
+        const float x0 = fminf(fmaxf(__fmul_rn(__fsub_rn(__fsub_rn(dec[2], half_w), pw), g.wscale), 0.f), sw);
+        const float y0 = fminf(fmaxf(__fmul_rn(__fsub_rn(__fsub_rn(dec[3], half_h), ph), g.hscale), 0.f), sh);
+        const float x1 = fminf(fmaxf(__fmul_rn(__fsub_rn(__fadd_rn(dec[2], half_w), pw), g.wscale), 0.f), sw);
+        const float y1 = fminf(fmaxf(__fmul_rn(__fsub_rn(__fadd_rn(dec[3], half_h), ph), g.hscale), 0.f), sh);
+        // a reduced decode of a file: on to the file's pixels (a factor of exactly 1 leaves the clipped box as it is)
+        const float fw = static_cast<float>(g.file_w), fh = static_cast<float>(g.file_h);
         float* bo = o.boxes_original + r * 4;
-        bo[0] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fsub_rn(dec[2], half_w), pw), g.wscale), 0.f), sw);
-        bo[1] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fsub_rn(dec[3], half_h), ph), g.hscale), 0.f), sh);
-        bo[2] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fadd_rn(dec[2], half_w), pw), g.wscale), 0.f), sw);
-        bo[3] = fminf(fmaxf(__fmul_rn(__fsub_rn(__fadd_rn(dec[3], half_h), ph), g.hscale), 0.f), sh);
+        bo[0] = fminf(fmaxf(__fmul_rn(x0, g.file_wscale), 0.f), fw);
+        bo[1] = fminf(fmaxf(__fmul_rn(y0, g.file_hscale), 0.f), fh);
+        bo[2] = fminf(fmaxf(__fmul_rn(x1, g.file_wscale), 0.f), fw);
+        bo[3] = fminf(fmaxf(__fmul_rn(y1, g.file_hscale), 0.f), fh);
     }
 }
 
@@ -708,6 +714,8 @@ bool letterbox_image(const uint8_t* pixels, int h, int w, int th, int tw, Letter
     if (im->rh <= 0 || im->rw <= 0) return false;
     im->hscale = static_cast<float>(h) / static_cast<float>(im->rh);
     im->wscale = static_cast<float>(w) / static_cast<float>(im->rw);
+    im->file_h = h; im->file_w = w;
+    im->file_hscale = im->file_wscale = 1.f;
     return true;
 }
 

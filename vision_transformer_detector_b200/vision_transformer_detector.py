@@ -308,6 +308,33 @@ def _jpeg_table(arrs) -> C.Array:
     return (_capi.Jpeg * len(arrs))(*[_capi.Jpeg(a.ctypes.data, int(a.size)) for a in arrs])
 
 
+JPEG_RATIOS = (1, 2, 4, 8)
+
+
+def _jpeg_ratios(ratio, B: int, allow_auto: bool) -> list:
+    """The decode scale of B files as the library's int32 codes: ratio is 1, 2, 4, 8 ("auto", code 0, where allowed) or a
+    sequence of B of them.  ValueError for anything else."""
+    def code(r, where):
+        if allow_auto and isinstance(r, str) and r == "auto":
+            return 0
+        if isinstance(r, (int, np.integer)) and not isinstance(r, (bool, np.bool_)) and int(r) in JPEG_RATIOS:
+            return int(r)
+        allowed = '1, 2, 4, 8 or "auto"' if allow_auto else "1, 2, 4 or 8"
+        raise ValueError(f"{where}ratio must be {allowed}, got {r!r}")
+    if isinstance(ratio, (str, int, np.integer)):
+        return [code(ratio, "")] * B
+    if not isinstance(ratio, (list, tuple, np.ndarray)):
+        raise ValueError(f"ratio must be a ratio or a sequence of one per file, got {type(ratio).__name__}")
+    if len(ratio) != B:
+        raise ValueError(f"ratio holds {len(ratio)} ratios for {B} files")
+    return [code(r, f"file {i}: ") for i, r in enumerate(ratio)]
+
+
+def _full_size(ratio) -> bool:
+    """ratio is the plain default 1: the full-size entry points, exactly as before ratios existed."""
+    return isinstance(ratio, (int, np.integer)) and not isinstance(ratio, (bool, np.bool_)) and int(ratio) == 1
+
+
 def _alloc_records_np(B: int, S: int):
     return (np.empty((B, S, 6), np.float32), np.empty((B, S, 6), np.float32), np.empty((B, S), np.int32),
             np.empty((B, S), np.float32), np.empty((B, S), np.uint8), np.empty((B, S, 4), np.int32))
@@ -867,24 +894,36 @@ class VisionTransformerDetector:
 
     # -- JPEG files ---------------------------------------------------------------------------------
     def detect_jpeg(self, files, objectness_threshold=None, classification_threshold=None, strict=True,
-                    compute_mode: str | None = None, packed: bool = False) -> DetectionRecords:
+                    compute_mode: str | None = None, packed: bool = False, ratio=1) -> DetectionRecords:
         """detect_images() on JPEG files, decoded on the GPU bit-identically to PIL's Image.open(f).convert("RGB") (and
         tf.image.decode_jpeg): the same records, boxes_original included, as detect_images on the PIL-decoded images.
         files: a sequence of bytes-like objects (bytes, bytearray, memoryview, 1-D uint8 numpy arrays) or paths.  One
-        synchronous call; a file outside baseline JPEG fails the call, naming it (VitdetError E_INVALID)."""
-        return self.collect(self.submit_jpeg(files, objectness_threshold, classification_threshold, strict, compute_mode, packed))
+        synchronous call; a file outside baseline JPEG fails the call, naming it (VitdetError E_INVALID).
+        ratio: 1, 2, 4, 8, "auto" or one of them per file: decode at 1 / ratio scale in the DCT domain, as
+        tf.image.decode_jpeg(ratio=) and PIL's draft() do; "auto" picks what draft() picks for the letterbox size
+        (jpeg_auto_ratio; 1 for every image up to about twice the model's input size).  The records are those of
+        detect_images on the reduced decode, except boxes_original, which stays in the file's pixels."""
+        return self.collect(self.submit_jpeg(files, objectness_threshold, classification_threshold, strict, compute_mode, packed,
+                                             ratio))
 
     def submit_jpeg(self, files, objectness_threshold=None, classification_threshold=None, strict=True,
-                    compute_mode: str | None = None, packed: bool = False) -> int:
-        """Asynchronous detect_jpeg() (vitdet_submit_jpeg_host), completed by collect(ticket); shares the two submission
-        slots of submit().  Page-locked files are read directly and must stay alive until their ticket is collected."""
+                    compute_mode: str | None = None, packed: bool = False, ratio=1) -> int:
+        """Asynchronous detect_jpeg() (vitdet_submit_jpeg_host[_scaled]), completed by collect(ticket); shares the two
+        submission slots of submit().  Page-locked files are read directly and must stay alive until their ticket is
+        collected."""
         arrs = _jpeg_arrays(files)
         B, S = len(arrs), Constants.MAX_DETECT_OBJECTS_QUANTITY.value
+        ratios = _jpeg_ratios(ratio, B, allow_auto=True)
         params = _decode_params(objectness_threshold, classification_threshold, strict, self.config.input_shape[:2])
         boxes = np.empty((B, S, 4), np.float32)
         ticket = C.c_int(-1)
-        _capi.check(self._lib.vitdet_submit_jpeg_host(self._h, _jpeg_table(arrs), B, self._mode(compute_mode), C.byref(params),
-                                                      1 if packed else 0, _capi.np_ptr(boxes), None, C.byref(ticket)))
+        if _full_size(ratio):
+            _capi.check(self._lib.vitdet_submit_jpeg_host(self._h, _jpeg_table(arrs), B, self._mode(compute_mode), C.byref(params),
+                                                          1 if packed else 0, _capi.np_ptr(boxes), None, C.byref(ticket)))
+        else:
+            _capi.check(self._lib.vitdet_submit_jpeg_host_scaled(self._h, _jpeg_table(arrs), (C.c_int32 * B)(*ratios), B,
+                                                                 self._mode(compute_mode), C.byref(params), 1 if packed else 0,
+                                                                 _capi.np_ptr(boxes), None, C.byref(ticket)))
         self._inflight = getattr(self, "_inflight", {})
         self._inflight[ticket.value] = (B, packed, arrs, boxes)
         return ticket.value

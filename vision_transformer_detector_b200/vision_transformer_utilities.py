@@ -4,7 +4,8 @@ the reference module (annotation parsing at import time from hard-coded D:\\ pat
 
     _get_image_tensor_coco(one_image_path)        vision_transformer_utilities.py:418-449
     preprocess_image(image_uint8)                 the arithmetic of that function: resize_with_pad, clip, /127.5 - 1
-    decode_jpeg(files)                            tf.image.decode_jpeg on the GPU, bit-identical to PIL / libjpeg-turbo
+    decode_jpeg(files, ratio=1)                   tf.image.decode_jpeg(ratio=) on the GPU, bit-identical to PIL / libjpeg-turbo
+    jpeg_auto_ratio(height, width)                the decode ratio PIL's draft() picks for the model's letterbox
 
 The arithmetic runs on the GPU (vitdet_preprocess_image*); only the file decode is host work (PIL)."""
 from __future__ import annotations
@@ -14,7 +15,8 @@ import ctypes as C
 import numpy as np
 
 from . import _capi
-from .vision_transformer_detector import Constants, DetectorConfig, _is_torch_cuda, _jpeg_arrays, _jpeg_table, _torch_stream_ptr
+from .vision_transformer_detector import (Constants, DetectorConfig, _full_size, _is_torch_cuda, _jpeg_arrays, _jpeg_ratios,
+                                          _jpeg_table, _torch_stream_ptr)
 
 MODEL_IMAGE_HEIGHT, MODEL_IMAGE_WIDTH = Constants.MODEL_IMAGE_SIZE.value       # vision_transformer_utilities.py:23-24
 
@@ -73,13 +75,28 @@ def _decoder(index: int) -> C.c_void_p:
     return h
 
 
-def decode_jpeg(files, device=None) -> list:
+def jpeg_auto_ratio(height: int, width: int, target_size=None) -> int:
+    """The decode ratio detect_jpeg(ratio="auto") uses for a height x width file: what PIL's draft("RGB", (rw, rh)) picks
+    for the size (rh, rw) resize_with_pad gives it at target_size (default: the model's 608 x 608), i.e. the largest of 8,
+    4, 2, 1 that is at most min(width // rw, height // rh)."""
+    th, tw = (MODEL_IMAGE_HEIGHT, MODEL_IMAGE_WIDTH) if target_size is None else (int(target_size[0]), int(target_size[1]))
+    rc = _capi.load().vitdet_jpeg_auto_ratio(int(height), int(width), th, tw)
+    if rc < 0:
+        _capi.check(rc)
+    return rc
+
+
+def decode_jpeg(files, device=None, ratio=1) -> list:
     """Baseline JPEG files -> a list of torch CUDA uint8 (h, w, 3) RGB tensors, decoded on the GPU bit-identically to
     np.asarray(PIL.Image.open(f).convert("RGB")) (libjpeg-turbo's ISLOW IDCT and fancy upsampling, which
     tf.image.decode_jpeg also uses).  files: bytes-like objects or paths.  Asynchronous on torch's current stream of
-    `device` (default: the current CUDA device).  A file outside baseline JPEG raises VitdetError (E_INVALID) naming it."""
+    `device` (default: the current CUDA device).  A file outside baseline JPEG raises VitdetError (E_INVALID) naming it.
+    ratio: 1, 2, 4 or 8, or one of them per file: decode at 1 / ratio scale in the DCT domain, (ceil(h / ratio),
+    ceil(w / ratio), 3), bit-identical to tf.image.decode_jpeg(ratio=) and to PIL after im.draft("RGB", (w // ratio,
+    h // ratio))."""
     import torch
     arrs = _jpeg_arrays(files)
+    ratios = _jpeg_ratios(ratio, len(arrs), allow_auto=False)
     lib = _capi.load()
     dev = torch.device("cuda", torch.cuda.current_device()) if device is None else torch.device(device)
     if dev.type != "cuda":
@@ -92,12 +109,17 @@ def decode_jpeg(files, device=None) -> list:
         if rc:
             msg = lib.vitdet_last_error()
             raise _capi.VitdetError(rc, f"file {i}: " + (msg.decode("utf-8", "replace") if msg else ""))
-        shapes.append((v[0].value, v[1].value, 3))
+        h, w = -(-v[0].value // ratios[i]), -(-v[1].value // ratios[i])
+        shapes.append((h, w, 3))
         offs.append(total)
-        total += (v[0].value * v[1].value * 3 + 255) // 256 * 256
+        total += (h * w * 3 + 255) // 256 * 256
     with torch.cuda.device(index):
         buf = torch.empty(total, dtype=torch.uint8, device=dev)
         off_c = (C.c_int64 * len(arrs))(*offs)
-        _capi.check(lib.vitdet_decode_jpeg(_decoder(index), _jpeg_table(arrs), len(arrs), C.c_void_p(buf.data_ptr()), off_c,
-                                           _torch_stream_ptr(dev)))
+        if _full_size(ratio):
+            _capi.check(lib.vitdet_decode_jpeg(_decoder(index), _jpeg_table(arrs), len(arrs), C.c_void_p(buf.data_ptr()), off_c,
+                                               _torch_stream_ptr(dev)))
+        else:
+            _capi.check(lib.vitdet_decode_jpeg_scaled(_decoder(index), _jpeg_table(arrs), (C.c_int32 * len(arrs))(*ratios),
+                                                      len(arrs), C.c_void_p(buf.data_ptr()), off_c, _torch_stream_ptr(dev)))
     return [buf[o:o + h * w * 3].view(h, w, 3) for o, (h, w, _) in zip(offs, shapes)]
