@@ -1,5 +1,6 @@
 """GPU tests of the JPEG decoder (vitdet_decode_jpeg, vitdet_submit_jpeg_host): decode_jpeg must give PIL's pixels bit for
 bit, and detect_jpeg / submit_jpeg exactly the records of detect_images on the PIL-decoded images."""
+import ctypes as C
 import io
 
 import numpy as np
@@ -11,6 +12,7 @@ import _jpeg_corpus as jc
 import jpeg_oracle as jo
 import vision_transformer_detector_b200 as vd
 from vision_transformer_detector_b200 import _capi
+from vision_transformer_detector_b200.vision_transformer_detector import _jpeg_table
 from vision_transformer_detector_b200.vision_transformer_utilities import decode_jpeg
 
 pytestmark = pytest.mark.gpu
@@ -72,6 +74,17 @@ def test_submit_jpeg_pageable_and_page_locked_in_flight_equal_detect_jpeg():
     got_a = m.collect(ta)
     _assert_same(got_a, m.detect_jpeg(a, packed=True))
     _assert_same(got_b, m.detect_jpeg(b, packed=True))
+    # the full-size entry point gives what submit_jpeg gets from the scaled one at ratio 1
+    lib = _capi.load()
+    S = 17
+    recs, st = vd.vision_transformer_detector._alloc_records(len(a), S, packed=True)
+    recs.boxes_original = np.empty((len(a), S, 4), np.float32)
+    params = vd.vision_transformer_detector._decode_params(None, None, True, cfg.input_shape[:2])
+    ticket = C.c_int(-1)
+    _capi.check(lib.vitdet_submit_jpeg_host(m._h, _jpeg_table([np.frombuffer(d, np.uint8) for d in a]), len(a), _capi.MODE_BF16,
+                                            C.byref(params), 1, _capi.np_ptr(recs.boxes_original), None, C.byref(ticket)))
+    _capi.check(lib.vitdet_collect(m._h, ticket.value, _capi.np_ptr(recs.logits), C.byref(st)))
+    _assert_same(recs, got_a)
     m.close()
 
 

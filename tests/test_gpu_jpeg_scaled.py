@@ -15,7 +15,7 @@ import jpeg_scaled_oracle as js
 import vision_transformer_detector_b200 as vd
 from vision_transformer_detector_b200 import _capi
 from vision_transformer_detector_b200.vision_transformer_detector import _jpeg_table
-from vision_transformer_detector_b200.vision_transformer_utilities import decode_jpeg, jpeg_auto_ratio
+from vision_transformer_detector_b200.vision_transformer_utilities import _decoder, decode_jpeg, jpeg_auto_ratio
 
 pytestmark = pytest.mark.gpu
 
@@ -78,9 +78,19 @@ def test_mixed_ratios_equal_per_ratio_calls():
     got = decode_jpeg(files, ratio=ratios)
     for i, r in enumerate(ratios):
         assert np.array_equal(got[i].cpu().numpy(), per_ratio[r][i].cpu().numpy()), i
-    # ratio 1 through the scaled entry point is today's decode
-    for a, b in zip(decode_jpeg(files, ratio=[1] * len(files)), decode_jpeg(files)):
-        assert np.array_equal(a.cpu().numpy(), b.cpu().numpy())
+    # ratio 1 through the scaled entry point, which decode_jpeg calls, is the full-size entry point's decode
+    import torch
+    full = decode_jpeg(files, ratio=[1] * len(files))
+    offs = [0]
+    for g in full[:-1]:
+        offs.append(offs[-1] + (g.numel() + 255) // 256 * 256)
+    buf = torch.zeros(offs[-1] + full[-1].numel(), dtype=torch.uint8, device="cuda")
+    arrs = [np.frombuffer(d, np.uint8) for d in files]
+    lib = _capi.load()
+    _capi.check(lib.vitdet_decode_jpeg(_decoder(torch.cuda.current_device()), _jpeg_table(arrs), len(files), C.c_void_p(buf.data_ptr()),
+                                       (C.c_int64 * len(files))(*offs), C.c_void_p(torch.cuda.current_stream().cuda_stream)))
+    for o, g in zip(offs, full):
+        assert np.array_equal(buf[o:o + g.numel()].view(g.shape).cpu().numpy(), g.cpu().numpy())
 
 
 def _detect_files(seed):

@@ -57,6 +57,7 @@ int fail(int code, const char* fmt, ...) {
 }
 
 static inline int round_up(int v, int m) { return (v + m - 1) / m * m; }
+static size_t a256(size_t v) { return (v + 255) / 256 * 256; }
 
 constexpr int kMaxKeyDim = 128;   // one or two 64-column (128-byte swizzle row) boxes per head in shared memory
 constexpr int kMaxKeyDimSplit = 64;     // the split (fp32-accumulate) attention kernel keeps hi and lo tiles: one box per head
@@ -310,28 +311,65 @@ private:
     int pending_ = 0;
 };
 
+// The records of R detection rows that a host entry point reads back in one copy, each array 256-byte aligned; bytes
+// per row: logits 24 | decoded 24 | class_id 4 | class_conf 4 | corners 16 | keep 1 | packed 52 | boxes_original 16,
+// the last two only when asked for.
+struct RecordBlock {
+    size_t R = 0, o_dec = 0, o_id = 0, o_cc = 0, o_cor = 0, o_keep = 0, o_pk = 0, o_box = 0, bytes = 0;
+    bool packed = false, boxes = false;
+    RecordBlock() = default;
+    RecordBlock(size_t rows, bool want_packed, bool want_boxes) : R(rows), packed(want_packed), boxes(want_boxes) {
+        o_dec = a256(R * 24); o_id = o_dec + a256(R * 24); o_cc = o_id + a256(R * 4); o_cor = o_cc + a256(R * 4);
+        o_keep = o_cor + a256(R * 16); o_pk = o_keep + a256(R);
+        o_box = o_pk + (packed ? a256(R * 52) : 0);
+        bytes = o_box + (boxes ? a256(R * 16) : 0);
+    }
+    // the decode outputs inside a DEVICE block at base
+    vitdet_detections detections(char* base) const {
+        vitdet_detections d = {};
+        d.decoded = reinterpret_cast<float*>(base + o_dec);
+        d.class_id = reinterpret_cast<int32_t*>(base + o_id);
+        d.class_conf = reinterpret_cast<float*>(base + o_cc);
+        d.corners = reinterpret_cast<int32_t*>(base + o_cor);
+        d.keep = reinterpret_cast<uint8_t*>(base + o_keep);
+        if (packed) d.packed = reinterpret_cast<float*>(base + o_pk);
+        return d;
+    }
+    float* boxes_original(char* base) const { return boxes ? reinterpret_cast<float*>(base + o_box) : nullptr; }
+    // A HOST copy of the block -> the caller's arrays (each may be null)
+    int copy_out(const char* pb, float* logits_host, const vitdet_detections* out_host, float* boxes_host) const {
+        if (logits_host) memcpy(logits_host, pb, R * 24);
+        if (out_host) {
+            if (out_host->decoded) memcpy(out_host->decoded, pb + o_dec, R * 24);
+            if (out_host->class_id) memcpy(out_host->class_id, pb + o_id, R * 4);
+            if (out_host->class_conf) memcpy(out_host->class_conf, pb + o_cc, R * 4);
+            if (out_host->corners) memcpy(out_host->corners, pb + o_cor, R * 16);
+            if (out_host->keep) memcpy(out_host->keep, pb + o_keep, R);
+            if (out_host->packed) {
+                if (!packed) return fail(VITDET_E_INVALID, "collect: the submission did not ask for packed records");
+                memcpy(out_host->packed, pb + o_pk, R * 52);
+            }
+        }
+        if (boxes_host) memcpy(boxes_host, pb + o_box, R * 16);
+        return 0;
+    }
+};
+
 // One in-flight host submission (vitdet_submit_host .. vitdet_collect): its own pinned staging, device input and
 // record block, so that the H2D copy of submission i+1 overlaps the compute of submission i.  A submission of separate
 // images (vitdet_submit_images_host) also owns its letterbox table, copied to dev_table on the compute stream.
 struct HostSlot {
-    void* pin_in = nullptr; size_t pin_in_bytes = 0;
-    void* pin_out = nullptr; size_t pin_out_bytes = 0;
-    LetterboxImage* pin_table = nullptr; size_t pin_table_bytes = 0;
+    PinnedBuf pin_in, pin_out, pin_table;
     DevBuf dev_in, dev_out, dev_table;
     // a submission of JPEG files (vitdet_submit_jpeg_host): its descriptor block, decode scratch and decoded pixels
-    char* pin_jpeg = nullptr; size_t pin_jpeg_bytes = 0;
+    PinnedBuf pin_jpeg;
     DevBuf jpeg_work, jpeg_rgb;
     std::vector<cudaEvent_t> copy_events;      // one per staged sub-chunk of images
     cudaEvent_t done = nullptr;                // recorded after the D2H copy of the record block
     bool busy = false;
-    size_t R = 0, o_dec = 0, o_id = 0, o_cc = 0, o_cor = 0, o_keep = 0, o_pk = 0, o_box = 0;
-    bool has_packed = false;
+    RecordBlock rec;
     float* boxes_host = nullptr;               // where vitdet_collect puts boxes_original, or null
     ~HostSlot() {
-        if (pin_in) cudaFreeHost(pin_in);
-        if (pin_out) cudaFreeHost(pin_out);
-        if (pin_table) cudaFreeHost(pin_table);
-        if (pin_jpeg) cudaFreeHost(pin_jpeg);
         for (auto e : copy_events) cudaEventDestroy(e);
         if (done) cudaEventDestroy(done);
     }
@@ -409,7 +447,7 @@ struct vitdet_handle {
     DevBuf images_table;                         // letterbox table of vitdet_forward_images, written in stream order
     // vitdet_decode_jpeg: descriptor block and files staged in pinned memory, device files and decode scratch; jpeg_done,
     // recorded after the last decode, orders their reuse whatever stream the next call runs on
-    char* jpeg_pin = nullptr; size_t jpeg_pin_bytes = 0;
+    PinnedBuf jpeg_pin;
     cudaEvent_t jpeg_done = nullptr;
     DevBuf jpeg_files, jpeg_work;
     const long long* jpeg_stats = nullptr;       // repair counters of the last JPEG decode (device)
@@ -419,12 +457,19 @@ struct vitdet_handle {
         for (auto e : prof_pool) cudaEventDestroy(e);
         delete stage_pool;
         if (copy_stream) cudaStreamDestroy(copy_stream);
-        if (jpeg_pin) cudaFreeHost(jpeg_pin);
         if (jpeg_done) cudaEventDestroy(jpeg_done);
     }
 };
 
 namespace vitdet {
+
+static int check_device(const vitdet_handle* h, const char* fn) {
+    int cur = -1;
+    CU_TRY(cudaGetDevice(&cur));
+    if (cur != h->device)
+        return fail(VITDET_E_INVALID, "%s: the handle lives on device %d but the current CUDA device is %d", fn, h->device, cur);
+    return 0;
+}
 
 // ------------------------------------------------------------------------------------------------
 // configuration -> weight table (Keras `model.weights` order and names, see SURVEY §8(a))
@@ -728,8 +773,6 @@ static Dims dims_for(const vitdet_handle* h, Form f) {
     return m;
 }
 
-static size_t a256(size_t v) { return (v + 255) / 256 * 256; }
-
 enum WorkspaceBuf { WS_X, WS_PATCH, WS_Y, WS_QKV, WS_CTX, WS_U0, WS_U1, WS_S, WS_H0, WS_H1, WS_TMP32, WS_COUNT };
 
 // Bytes of every workspace buffer a forward of B images in form f uses.  In the Split form a buffer that holds planes
@@ -861,10 +904,16 @@ struct ForwardOpts {
     int lead_chunks[2] = {0, 0};      // sizes of the first two encoder chunks (0 = use the regular chunk)
     const cudaEvent_t* ready = nullptr;
     int ready_gran = 0;
-    int in_u8 = 0;                    // images are uint8 pixels; the patch kernel normalises them (x / 127.5 - 1)
-    // images is a DEVICE table of B LetterboxImage entries: uint8 images of any size, letterboxed inside the patch kernel
-    int letterbox = 0;
-    float* boxes_original = nullptr;  // with letterbox: [B * S, 4] boxes on the source images
+};
+
+// The images of a forward, on the device.  F32 / U8: B images of the model's size, one contiguous array of float32 or
+// uint8 pixels (the patch kernel normalises uint8 ones, x / 127.5 - 1).  Letterbox: a table of B LetterboxImage entries,
+// uint8 images of any size letterboxed inside the patch kernel; boxes_original, if not null, receives the [B * S, 4]
+// boxes on the source images.
+struct Input {
+    enum Kind { F32, U8, Letterbox } kind;
+    const void* p;
+    float* boxes_original = nullptr;
 };
 
 // vitdet_decode_params / vitdet_detections -> the decode kernels' arguments (either may be null: defaults / no outputs)
@@ -896,16 +945,11 @@ static int dense(vitdet_handle* h, Form f, PlanCursor& pc, int cat, const DenseC
     return launch_tc(pc.p->gemm[pc.gemm++], c.out.p, c.resid, st);
 }
 
-static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, float* logits,
+static int forward_impl(vitdet_handle* h, const Input& in, int B, int mode, float* logits,
                         const vitdet_decode_params* dpar, const vitdet_detections* det, cudaStream_t st,
                         const ForwardOpts& opts = ForwardOpts()) {
-    if (!h || !images || B <= 0) return fail(VITDET_E_INVALID, "forward: bad arguments");
-    {
-        int cur = -1;
-        CU_TRY(cudaGetDevice(&cur));
-        if (cur != h->device)
-            return fail(VITDET_E_INVALID, "forward: the handle lives on device %d but the current CUDA device is %d", h->device, cur);
-    }
+    if (!h || !in.p || B <= 0) return fail(VITDET_E_INVALID, "forward: bad arguments");
+    RC_TRY(check_device(h, "forward"));
     if (mode != VITDET_MODE_BF16 && mode != VITDET_MODE_FP32) return fail(VITDET_E_INVALID, "forward: unknown mode %d", mode);
     for (const WeightSlot& s : h->slots)
         if (!s.set) return fail(VITDET_E_UNSET, "forward: weight '%s' has not been set", s.name.c_str());
@@ -984,14 +1028,15 @@ static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, f
         float* x = h->x.as<float>() + static_cast<size_t>(c0) * T * m.D4;
         PlanCursor pc = plan_cursor(h, kEncoderPlans, f, bc);
         const Rows pr = rows_out(h->patch, h->tmp32, h->PK);
-        if (opts.letterbox) {
+        if (in.kind == Input::Letterbox) {
             ProfScope ps(h, PC_PATCHIFY, st);
-            CU_TRY(letterbox_patchify_launch(static_cast<const LetterboxImage*>(images) + c0, bc, c.image_h, c.image_w, c.patch_size,
+            CU_TRY(letterbox_patchify_launch(static_cast<const LetterboxImage*>(in.p) + c0, bc, c.image_h, c.image_w, c.patch_size,
                                              pr.p, pr.ld, h->RP, pr.f32, st));
         } else {
-            const char* img = static_cast<const char*>(images) + static_cast<size_t>(c0) * c.image_h * c.image_w * 3 * (opts.in_u8 ? 1 : 4);
+            const int u8 = in.kind == Input::U8;
+            const char* img = static_cast<const char*>(in.p) + static_cast<size_t>(c0) * c.image_h * c.image_w * 3 * (u8 ? 1 : 4);
             ProfScope ps(h, PC_PATCHIFY, st);
-            CU_TRY(patchify_launch(img, opts.in_u8, bc, c.image_h, c.image_w, c.patch_size, pr.p, pr.ld, h->RP, pr.f32, st));
+            CU_TRY(patchify_launch(img, u8, bc, c.image_h, c.image_w, c.patch_size, pr.p, pr.ld, h->RP, pr.f32, st));
         }
         Operand a;
         RC_TRY(operand(pr, h->patch, Mc, h->PK, &a));
@@ -1089,9 +1134,9 @@ static int forward_impl(vitdet_handle* h, const void* images, int B, int mode, f
     DecodeParams dp;
     DecodeOut dout;
     decode_args(dpar, 1 /*the head emits raw logits*/, det, logits, &dp, &dout);
-    if (opts.letterbox && opts.boxes_original) {
-        dout.boxes_original = opts.boxes_original;
-        dout.letterbox = static_cast<const LetterboxImage*>(images);
+    if (in.kind == Input::Letterbox && in.boxes_original) {
+        dout.boxes_original = in.boxes_original;
+        dout.letterbox = static_cast<const LetterboxImage*>(in.p);
         dout.slots = h->S;
     }
     const int in_f32 = f != Form::Bf16;
@@ -1189,12 +1234,7 @@ int vitdet_weight_info(const vitdet_handle* h, int index, char* name, int cap, i
 
 int vitdet_set_weight(vitdet_handle* h, const char* name_in, const float* data, int ndim, const int64_t* shape) {
     if (!h || !name_in || !data) return fail(VITDET_E_INVALID, "set_weight: null argument");
-    {
-        int cur = -1;
-        CU_TRY(cudaGetDevice(&cur));
-        if (cur != h->device)
-            return fail(VITDET_E_INVALID, "set_weight: the handle lives on device %d but the current CUDA device is %d", h->device, cur);
-    }
+    RC_TRY(check_device(h, "set_weight"));
     std::string name(name_in);
     if (name.size() > 2 && name.compare(name.size() - 2, 2, ":0") == 0) name.resize(name.size() - 2);
     auto it = h->slot_index.find(name);
@@ -1348,22 +1388,20 @@ size_t vitdet_workspace_bytes(const vitdet_handle* h, int B, int mode) {
 
 int vitdet_forward(vitdet_handle* h, const float* images_dev, int B, float* logits_dev, int mode, void* stream) {
     if (!logits_dev) return fail(VITDET_E_INVALID, "forward: logits_dev is null");
-    return forward_impl(h, images_dev, B, mode, logits_dev, nullptr, nullptr, static_cast<cudaStream_t>(stream));
+    return forward_impl(h, Input{Input::F32, images_dev}, B, mode, logits_dev, nullptr, nullptr, static_cast<cudaStream_t>(stream));
 }
 
 int vitdet_forward_u8(vitdet_handle* h, const uint8_t* images_dev, int B, float* logits_dev, int mode, const vitdet_decode_params* params,
                       const vitdet_detections* out, void* stream) {
     if (!logits_dev && !(params && out)) return fail(VITDET_E_INVALID, "forward_u8: neither logits_dev nor (params, out) given");
     if ((params == nullptr) != (out == nullptr)) return fail(VITDET_E_INVALID, "forward_u8: params and out go together");
-    ForwardOpts opts;
-    opts.in_u8 = 1;
-    return forward_impl(h, images_dev, B, mode, logits_dev, params, out, static_cast<cudaStream_t>(stream), opts);
+    return forward_impl(h, Input{Input::U8, images_dev}, B, mode, logits_dev, params, out, static_cast<cudaStream_t>(stream));
 }
 
 int vitdet_forward_decode(vitdet_handle* h, const float* images_dev, int B, int mode, const vitdet_decode_params* params,
                           float* logits_dev, const vitdet_detections* out, void* stream) {
     if (!params || !out) return fail(VITDET_E_INVALID, "forward_decode: null params / out");
-    return forward_impl(h, images_dev, B, mode, logits_dev, params, out, static_cast<cudaStream_t>(stream));
+    return forward_impl(h, Input{Input::F32, images_dev}, B, mode, logits_dev, params, out, static_cast<cudaStream_t>(stream));
 }
 
 int vitdet_decode(const float* logits_dev, int R, const vitdet_decode_params* p, const vitdet_detections* out, void* stream) {
@@ -1421,29 +1459,18 @@ int vitdet_preprocess_image_host(const uint8_t* image_host, int h, int w, float*
 int vitdet_decode_host(const float* logits_host, int R, const vitdet_decode_params* p, const vitdet_detections* out_host) {
     if (!logits_host || !p || !out_host || R < 0) return fail(VITDET_E_INVALID, "decode_host: bad arguments");
     if (R == 0) return 0;
-    const size_t r = static_cast<size_t>(R);
-    const size_t o_dec = a256(r * 24), o_id = o_dec + a256(r * 24), o_cc = o_id + a256(r * 4), o_cor = o_cc + a256(r * 4),
-                 o_keep = o_cor + a256(r * 16), o_pk = o_keep + a256(r), total = o_pk + a256(r * 52);
+    // the logits go into the record block's logits rows; the block comes back in one copy
+    const RecordBlock rb(static_cast<size_t>(R), out_host->packed != nullptr, false);
     DevBuf buf;
-    RC_TRY(buf.ensure(total));
+    RC_TRY(buf.ensure(rb.bytes));
     char* b = buf.as<char>();
-    CU_TRY(cudaMemcpy(b, logits_host, r * 24, cudaMemcpyHostToDevice));
-    vitdet_detections d = {};
-    d.decoded = reinterpret_cast<float*>(b + o_dec);
-    d.class_id = reinterpret_cast<int32_t*>(b + o_id);
-    d.class_conf = reinterpret_cast<float*>(b + o_cc);
-    d.corners = reinterpret_cast<int32_t*>(b + o_cor);
-    d.keep = reinterpret_cast<uint8_t*>(b + o_keep);
-    if (out_host->packed) d.packed = reinterpret_cast<float*>(b + o_pk);
+    CU_TRY(cudaMemcpy(b, logits_host, rb.R * 24, cudaMemcpyHostToDevice));
+    const vitdet_detections d = rb.detections(b);
     RC_TRY(vitdet_decode(reinterpret_cast<const float*>(b), R, p, &d, nullptr));
     CU_TRY(cudaDeviceSynchronize());
-    if (out_host->decoded) CU_TRY(cudaMemcpy(out_host->decoded, d.decoded, r * 24, cudaMemcpyDeviceToHost));
-    if (out_host->class_id) CU_TRY(cudaMemcpy(out_host->class_id, d.class_id, r * 4, cudaMemcpyDeviceToHost));
-    if (out_host->class_conf) CU_TRY(cudaMemcpy(out_host->class_conf, d.class_conf, r * 4, cudaMemcpyDeviceToHost));
-    if (out_host->corners) CU_TRY(cudaMemcpy(out_host->corners, d.corners, r * 16, cudaMemcpyDeviceToHost));
-    if (out_host->keep) CU_TRY(cudaMemcpy(out_host->keep, d.keep, r, cudaMemcpyDeviceToHost));
-    if (out_host->packed) CU_TRY(cudaMemcpy(out_host->packed, d.packed, r * 52, cudaMemcpyDeviceToHost));
-    return 0;
+    std::vector<char> host(rb.bytes);
+    CU_TRY(cudaMemcpy(host.data(), b, rb.bytes, cudaMemcpyDeviceToHost));
+    return rb.copy_out(host.data(), nullptr, out_host, nullptr);
 }
 
 }  // extern "C"
@@ -1473,48 +1500,52 @@ static void ensure_stage_pool(vitdet_handle* h) {
 }
 
 // The images of one host submission: image i, src[i][0, offs[i + 1] - offs[i]), goes to byte offs[i] of the slot's device
-// input.  `table` (separate images of any size) holds their letterbox geometry; its pixel pointers are filled in here.
-// Without it the images are one contiguous array of the model's size.
-// `jpeg`: the sources are JPEG files, decoded on the device into the slot's pixel arena before the forward.
+// input.  F32 / U8: one contiguous array of the model's size.  Letterbox: separate images of any size, whose geometry
+// `table` holds; its pixel pointers are filled in here.  `jpeg`: the sources are JPEG files, decoded on the device into
+// the slot's pixel arena before the forward.
 struct HostImages {
+    Input::Kind kind;
     std::vector<const char*> src;
-    std::vector<size_t> offs;
+    std::vector<size_t> offs{0};
     std::vector<LetterboxImage> table;
     const JpegBatch* jpeg = nullptr;
+    void add(const void* p, size_t bytes) {
+        src.push_back(static_cast<const char*>(p));
+        offs.push_back(offs.back() + bytes);
+    }
 };
 
-static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, int mode, const vitdet_decode_params* params,
+// Enqueues the decode of a planned batch of JPEG files on st: the descriptor block, through `desc_pin` (page-locked, at
+// least jb.desc.size() bytes), to the head of the scratch `work`, then, once files_ready (may be null) has fired, the
+// kernels from the concatenated files at files_dev into out.  Its repair counters become the handle's jpeg_stats.
+static int jpeg_enqueue(vitdet_handle* h, const JpegBatch& jb, char* desc_pin, const char* files_dev, DevBuf& work, uint8_t* out,
+                        cudaEvent_t files_ready, cudaStream_t st) {
+    memcpy(desc_pin, jb.desc.data(), jb.desc.size());
+    RC_TRY(work.ensure(jb.work_bytes));
+    CU_TRY(cudaMemcpyAsync(work.p, desc_pin, jb.desc.size(), cudaMemcpyHostToDevice, st));
+    if (files_ready) CU_TRY(cudaStreamWaitEvent(st, files_ready, 0));
+    h->launches += kJpegLaunches;
+    CU_TRY(jpeg_decode_launch(jb, files_dev, work.p, out, st));
+    h->jpeg_stats = reinterpret_cast<const long long*>(work.as<char>() + jb.o_stats);
+    return 0;
+}
+
+static int submit_host_impl(vitdet_handle* h, HostImages& in, int B, int mode, const vitdet_decode_params* params,
                             int want_packed, float* boxes_host, void* stream, int* ticket) {
     HostSlot& sl = h->host_slots[h->next_slot];
     if (sl.busy) return fail(VITDET_E_INVALID, "submit_host: %d submissions are in flight; collect one first", vitdet_handle::kHostSlots);
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    const bool separate = !in.table.empty();
+    const bool separate = in.kind == Input::Letterbox;
     const size_t in_bytes = in.offs[B];
-    const size_t R = static_cast<size_t>(B) * h->S;
-    // output record block: logits 24 | decoded 24 | class_id 4 | class_conf 4 | corners 16 | keep 1 | packed 52 | boxes_original 16
-    // bytes per row
-    sl.R = R; sl.has_packed = want_packed != 0; sl.boxes_host = boxes_host;
-    sl.o_dec = a256(R * 24); sl.o_id = sl.o_dec + a256(R * 24); sl.o_cc = sl.o_id + a256(R * 4); sl.o_cor = sl.o_cc + a256(R * 4);
-    sl.o_keep = sl.o_cor + a256(R * 16); sl.o_pk = sl.o_keep + a256(R);
-    sl.o_box = sl.o_pk + (want_packed ? a256(R * 52) : 0);
-    const size_t out_bytes = sl.o_box + (boxes_host ? a256(R * 16) : 0);
+    sl.rec = RecordBlock(static_cast<size_t>(B) * h->S, want_packed != 0, boxes_host != nullptr);
+    sl.boxes_host = boxes_host;
     // a page-locked source is read directly, otherwise the whole submission is staged
     bool pinned = page_locked(in.src[0]);
     for (int i = 1; separate && pinned && i < B; ++i) pinned = page_locked(in.src[i]);
-    if (!pinned && sl.pin_in_bytes < in_bytes) {
-        if (sl.pin_in) cudaFreeHost(sl.pin_in);
-        sl.pin_in = nullptr; sl.pin_in_bytes = 0;
-        CU_TRY(cudaHostAlloc(&sl.pin_in, in_bytes, cudaHostAllocDefault));
-        sl.pin_in_bytes = in_bytes;
-    }
-    if (sl.pin_out_bytes < out_bytes) {
-        if (sl.pin_out) cudaFreeHost(sl.pin_out);
-        sl.pin_out = nullptr; sl.pin_out_bytes = 0;
-        CU_TRY(cudaHostAlloc(&sl.pin_out, out_bytes, cudaHostAllocDefault));
-        sl.pin_out_bytes = out_bytes;
-    }
+    if (!pinned) RC_TRY(sl.pin_in.ensure(in_bytes));
+    RC_TRY(sl.pin_out.ensure(sl.rec.bytes));
     RC_TRY(sl.dev_in.ensure(in_bytes));
-    RC_TRY(sl.dev_out.ensure(out_bytes));
+    RC_TRY(sl.dev_out.ensure(sl.rec.bytes));
     if (!sl.done) CU_TRY(cudaEventCreateWithFlags(&sl.done, cudaEventDisableTiming));
     // Images are copied in sub-chunks of kGran images on a dedicated copy stream, one event per sub-chunk; the encoder
     // runs chunks of 4, 12 and then `chunk` images, each waiting only for its own images: at ~12 images/ms of PCIe
@@ -1524,7 +1555,8 @@ static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, 
     // the slot's pinned buffer by the staging threads, sub-chunk by sub-chunk, overlapped with the H2D copies.
     // VITDET_E2E_LEAD="g,a,b" overrides the copy granularity and the two lead chunk sizes (tuning experiments).
     int kGran = 4, lead0 = 4, lead1 = 12;
-    if (in_u8) { kGran = 16; lead0 = 16; lead1 = 0; }       // a quarter of the bytes per image: same 0.3 ms lead-in with 16 images
+    // uint8 pixels, a quarter of the bytes per image: the same 0.3 ms lead-in with 16 images
+    if (in.kind != Input::F32) { kGran = 16; lead0 = 16; lead1 = 0; }
     // with the previous submission still computing, this one's copy has a whole forward pass to finish: no small lead chunks
     if (h->host_slots[(h->next_slot + vitdet_handle::kHostSlots - 1) % vitdet_handle::kHostSlots].busy) { lead0 = 0; lead1 = 0; }
     // nor in the split fp32 form: its three-pass GEMMs lose more on 4- and 12-image chunks than the early start gains
@@ -1545,8 +1577,8 @@ static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, 
         const int i0 = i * kGran, i1 = std::min(B, i0 + kGran);
         const size_t off = in.offs[i0], bytes = in.offs[i1] - off;
         if (!pinned) {
-            h->stage_pool->copy(static_cast<char*>(sl.pin_in) + off, in.src.data() + i0, in.offs.data() + i0, i1 - i0);
-            CU_TRY(cudaMemcpyAsync(dev_in + off, static_cast<const char*>(sl.pin_in) + off, bytes, cudaMemcpyHostToDevice, h->copy_stream));
+            h->stage_pool->copy(sl.pin_in.as<char>() + off, in.src.data() + i0, in.offs.data() + i0, i1 - i0);
+            CU_TRY(cudaMemcpyAsync(dev_in + off, sl.pin_in.as<char>() + off, bytes, cudaMemcpyHostToDevice, h->copy_stream));
         } else if (!separate) {
             CU_TRY(cudaMemcpyAsync(dev_in + off, in.src[i0], bytes, cudaMemcpyHostToDevice, h->copy_stream));
         } else {
@@ -1556,67 +1588,41 @@ static int submit_host_impl(vitdet_handle* h, HostImages& in, int in_u8, int B, 
         CU_TRY(cudaEventRecord(sl.copy_events[i], h->copy_stream));
     }
     ForwardOpts opts;
-    if (lead0 > 0 && B > lead0 + lead1) { opts.lead_chunks[0] = lead0; opts.lead_chunks[1] = lead1; }
-    else if (lead0 > 0 && B > lead0) opts.lead_chunks[0] = lead0;
-    opts.ready = sl.copy_events.data();
-    opts.ready_gran = kGran;
-    opts.in_u8 = in_u8;
-    const void* images_dev = dev_in;
+    Input input{in.kind, dev_in};
     const char* pixels_dev = dev_in;
-    std::vector<size_t> pixel_offs;
+    const size_t* pixel_offs = in.offs.data();
     if (in.jpeg) {
         // decode after the last file's copy, on the compute stream, into the slot's arena; the forward then waits for nothing
         const JpegBatch& jb = *in.jpeg;
-        if (sl.pin_jpeg_bytes < jb.desc.size()) {
-            if (sl.pin_jpeg) cudaFreeHost(sl.pin_jpeg);
-            sl.pin_jpeg = nullptr; sl.pin_jpeg_bytes = 0;
-            CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&sl.pin_jpeg), jb.desc.size(), cudaHostAllocDefault));
-            sl.pin_jpeg_bytes = jb.desc.size();
-        }
-        memcpy(sl.pin_jpeg, jb.desc.data(), jb.desc.size());
-        RC_TRY(sl.jpeg_work.ensure(jb.work_bytes));
+        RC_TRY(sl.pin_jpeg.ensure(jb.desc.size()));
         RC_TRY(sl.jpeg_rgb.ensure(jb.rgb_bytes));
-        CU_TRY(cudaMemcpyAsync(sl.jpeg_work.p, sl.pin_jpeg, jb.desc.size(), cudaMemcpyHostToDevice, st));
-        CU_TRY(cudaStreamWaitEvent(st, sl.copy_events[n_sub - 1], 0));
-        h->launches += kJpegLaunches;
-        CU_TRY(jpeg_decode_launch(jb, dev_in, sl.jpeg_work.p, sl.jpeg_rgb.as<uint8_t>(), st));
-        h->jpeg_stats = reinterpret_cast<const long long*>(sl.jpeg_work.as<char>() + jb.o_stats);
-        opts = ForwardOpts();
-        opts.in_u8 = in_u8;
+        RC_TRY(jpeg_enqueue(h, jb, sl.pin_jpeg.as<char>(), dev_in, sl.jpeg_work, sl.jpeg_rgb.as<uint8_t>(), sl.copy_events[n_sub - 1], st));
         pixels_dev = sl.jpeg_rgb.as<char>();
-        pixel_offs = jb.rgb_off;
+        pixel_offs = jb.rgb_off.data();
     } else {
-        pixel_offs.assign(in.offs.begin(), in.offs.end() - 1);
+        if (lead0 > 0 && B > lead0 + lead1) { opts.lead_chunks[0] = lead0; opts.lead_chunks[1] = lead1; }
+        else if (lead0 > 0 && B > lead0) opts.lead_chunks[0] = lead0;
+        opts.ready = sl.copy_events.data();
+        opts.ready_gran = kGran;
     }
+    char* dbase = sl.dev_out.as<char>();
     if (separate) {
         // the slot's own table: the pinned copy is not touched again before this submission is collected
         const size_t table_bytes = static_cast<size_t>(B) * sizeof(LetterboxImage);
-        if (sl.pin_table_bytes < table_bytes) {
-            if (sl.pin_table) cudaFreeHost(sl.pin_table);
-            sl.pin_table = nullptr; sl.pin_table_bytes = 0;
-            CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&sl.pin_table), table_bytes, cudaHostAllocDefault));
-            sl.pin_table_bytes = table_bytes;
-        }
+        RC_TRY(sl.pin_table.ensure(table_bytes));
         RC_TRY(sl.dev_table.ensure(table_bytes));
+        LetterboxImage* table = sl.pin_table.as<LetterboxImage>();
         for (int k = 0; k < B; ++k) {
-            sl.pin_table[k] = in.table[k];
-            sl.pin_table[k].pixels = reinterpret_cast<const uint8_t*>(pixels_dev + pixel_offs[k]);
+            table[k] = in.table[k];
+            table[k].pixels = reinterpret_cast<const uint8_t*>(pixels_dev + pixel_offs[k]);
         }
-        CU_TRY(cudaMemcpyAsync(sl.dev_table.p, sl.pin_table, table_bytes, cudaMemcpyHostToDevice, st));
-        opts.letterbox = 1;
-        opts.boxes_original = boxes_host ? reinterpret_cast<float*>(sl.dev_out.as<char>() + sl.o_box) : nullptr;
-        images_dev = sl.dev_table.p;
+        CU_TRY(cudaMemcpyAsync(sl.dev_table.p, table, table_bytes, cudaMemcpyHostToDevice, st));
+        input.p = sl.dev_table.p;
+        input.boxes_original = sl.rec.boxes_original(dbase);
     }
-    char* dbase = sl.dev_out.as<char>();
-    vitdet_detections d = {};
-    d.decoded = reinterpret_cast<float*>(dbase + sl.o_dec);
-    d.class_id = reinterpret_cast<int32_t*>(dbase + sl.o_id);
-    d.class_conf = reinterpret_cast<float*>(dbase + sl.o_cc);
-    d.corners = reinterpret_cast<int32_t*>(dbase + sl.o_cor);
-    d.keep = reinterpret_cast<uint8_t*>(dbase + sl.o_keep);
-    if (want_packed) d.packed = reinterpret_cast<float*>(dbase + sl.o_pk);
-    RC_TRY(forward_impl(h, images_dev, B, mode, reinterpret_cast<float*>(dbase), params, &d, st, opts));
-    CU_TRY(cudaMemcpyAsync(sl.pin_out, dbase, out_bytes, cudaMemcpyDeviceToHost, st));
+    const vitdet_detections d = sl.rec.detections(dbase);
+    RC_TRY(forward_impl(h, input, B, mode, reinterpret_cast<float*>(dbase), params, &d, st, opts));
+    CU_TRY(cudaMemcpyAsync(sl.pin_out.p, dbase, sl.rec.bytes, cudaMemcpyDeviceToHost, st));
     CU_TRY(cudaEventRecord(sl.done, st));
     sl.busy = true;
     *ticket = h->next_slot;
@@ -1630,50 +1636,31 @@ static int collect_impl(vitdet_handle* h, int ticket, float* logits_host, const 
     if (!sl.busy) return fail(VITDET_E_INVALID, "collect: ticket %d is not in flight", ticket);
     sl.busy = false;
     CU_TRY(cudaEventSynchronize(sl.done));
-    const char* pb = static_cast<const char*>(sl.pin_out);
-    const size_t R = sl.R;
-    if (logits_host) memcpy(logits_host, pb, R * 24);
-    if (out_host) {
-        if (out_host->decoded) memcpy(out_host->decoded, pb + sl.o_dec, R * 24);
-        if (out_host->class_id) memcpy(out_host->class_id, pb + sl.o_id, R * 4);
-        if (out_host->class_conf) memcpy(out_host->class_conf, pb + sl.o_cc, R * 4);
-        if (out_host->corners) memcpy(out_host->corners, pb + sl.o_cor, R * 16);
-        if (out_host->keep) memcpy(out_host->keep, pb + sl.o_keep, R);
-        if (out_host->packed) {
-            if (!sl.has_packed) return fail(VITDET_E_INVALID, "collect: the submission did not ask for packed records");
-            memcpy(out_host->packed, pb + sl.o_pk, R * 52);
-        }
-    }
-    if (sl.boxes_host) memcpy(sl.boxes_host, pb + sl.o_box, R * 16);
-    return 0;
+    return sl.rec.copy_out(sl.pin_out.as<char>(), logits_host, out_host, sl.boxes_host);
 }
 
 // A contiguous host array of B images of the model's size
-static int submit_dense_impl(vitdet_handle* h, const void* images_host, int in_u8, int B, int mode, const vitdet_decode_params* params,
+static int submit_dense_impl(vitdet_handle* h, const void* images_host, Input::Kind kind, int B, int mode, const vitdet_decode_params* params,
                              int want_packed, void* stream, int* ticket) {
     if (!h || !images_host || B <= 0 || !params || !ticket) return fail(VITDET_E_INVALID, "submit_host: bad arguments");
-    const size_t img_bytes = static_cast<size_t>(h->cfg.image_h) * h->cfg.image_w * 3 * (in_u8 ? 1 : 4);
-    HostImages in;
-    in.src.resize(B);
-    in.offs.resize(B + 1);
-    for (int i = 0; i <= B; ++i) {
-        in.offs[i] = static_cast<size_t>(i) * img_bytes;
-        if (i < B) in.src[i] = static_cast<const char*>(images_host) + in.offs[i];
-    }
-    return submit_host_impl(h, in, in_u8, B, mode, params, want_packed, nullptr, stream, ticket);
+    const size_t img_bytes = static_cast<size_t>(h->cfg.image_h) * h->cfg.image_w * 3 * (kind == Input::U8 ? 1 : 4);
+    HostImages in{kind};
+    for (int i = 0; i < B; ++i) in.add(static_cast<const char*>(images_host) + i * img_bytes, img_bytes);
+    return submit_host_impl(h, in, B, mode, params, want_packed, nullptr, stream, ticket);
 }
 
-static int predict_host_impl(vitdet_handle* h, const void* images_host, int in_u8, int B, int mode, const vitdet_decode_params* params,
+static int predict_host_impl(vitdet_handle* h, const void* images_host, Input::Kind kind, int B, int mode, const vitdet_decode_params* params,
                              float* logits_host, const vitdet_detections* out_host, void* stream) {
     int ticket = -1;
-    RC_TRY(submit_dense_impl(h, images_host, in_u8, B, mode, params, (out_host && out_host->packed) ? 1 : 0, stream, &ticket));
+    RC_TRY(submit_dense_impl(h, images_host, kind, B, mode, params, (out_host && out_host->packed) ? 1 : 0, stream, &ticket));
     return collect_impl(h, ticket, logits_host, out_host);
 }
 
-// Checks a caller's list of separate images and fills their letterbox table (pixel pointers as given); the message of a
-// rejected list names the first bad image.  boxes: boxes_original is requested, which needs the decode at the model's size.
-static int images_table(const vitdet_handle* h, const char* fn, const vitdet_image* images, int B, const vitdet_decode_params* params,
-                        bool boxes, std::vector<LetterboxImage>* table) {
+// Checks a list of B images of any size to be letterboxed to the model's input size and fills their table (pixel
+// pointers as given); the message of a rejected list names the first bad image.  boxes: boxes_original is requested,
+// which needs the decode at the model's size.
+static int letterbox_table(const vitdet_handle* h, const char* fn, const vitdet_image* images, int B, const vitdet_decode_params* params,
+                           bool boxes, std::vector<LetterboxImage>* table) {
     if (!h || !images || B <= 0) return fail(VITDET_E_INVALID, "%s: %s", fn, !h ? "null handle" : (!images ? "images is null" : "B must be positive"));
     const int th = h->cfg.image_h, tw = h->cfg.image_w;
     if (boxes && (!params || params->image_h != static_cast<float>(th) || params->image_w != static_cast<float>(tw)))
@@ -1694,17 +1681,17 @@ extern "C" {
 
 int vitdet_predict_host(vitdet_handle* h, const float* images_host, int B, int mode, const vitdet_decode_params* params,
                         float* logits_host, const vitdet_detections* out_host, void* stream) {
-    return predict_host_impl(h, images_host, 0, B, mode, params, logits_host, out_host, stream);
+    return predict_host_impl(h, images_host, Input::F32, B, mode, params, logits_host, out_host, stream);
 }
 
 int vitdet_predict_host_u8(vitdet_handle* h, const uint8_t* images_host, int B, int mode, const vitdet_decode_params* params,
                            float* logits_host, const vitdet_detections* out_host, void* stream) {
-    return predict_host_impl(h, images_host, 1, B, mode, params, logits_host, out_host, stream);
+    return predict_host_impl(h, images_host, Input::U8, B, mode, params, logits_host, out_host, stream);
 }
 
 int vitdet_submit_host(vitdet_handle* h, const void* images_host, int images_are_uint8, int B, int mode, const vitdet_decode_params* params,
                        int want_packed, void* stream, int* ticket) {
-    return submit_dense_impl(h, images_host, images_are_uint8 ? 1 : 0, B, mode, params, want_packed, stream, ticket);
+    return submit_dense_impl(h, images_host, images_are_uint8 ? Input::U8 : Input::F32, B, mode, params, want_packed, stream, ticket);
 }
 
 int vitdet_collect(vitdet_handle* h, int ticket, float* logits_host, const vitdet_detections* out_host) {
@@ -1716,32 +1703,22 @@ int vitdet_forward_images(vitdet_handle* h, const vitdet_image* images, int B, i
     if (!logits_dev && !(params && out)) return fail(VITDET_E_INVALID, "forward_images: neither logits_dev nor (params, out) given");
     if ((params == nullptr) != (out == nullptr)) return fail(VITDET_E_INVALID, "forward_images: params and out go together");
     std::vector<LetterboxImage> table;
-    RC_TRY(images_table(h, "forward_images", images, B, params, boxes_original_dev != nullptr, &table));
+    RC_TRY(letterbox_table(h, "forward_images", images, B, params, boxes_original_dev != nullptr, &table));
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     // a pageable source: the copy has taken the table by the time it returns, and it reaches the device in stream order
     const size_t table_bytes = table.size() * sizeof(LetterboxImage);
     RC_TRY(h->images_table.ensure(table_bytes));
     CU_TRY(cudaMemcpyAsync(h->images_table.p, table.data(), table_bytes, cudaMemcpyHostToDevice, st));
-    ForwardOpts opts;
-    opts.in_u8 = 1;
-    opts.letterbox = 1;
-    opts.boxes_original = boxes_original_dev;
-    return forward_impl(h, h->images_table.p, B, mode, logits_dev, params, out, st, opts);
+    return forward_impl(h, Input{Input::Letterbox, h->images_table.p, boxes_original_dev}, B, mode, logits_dev, params, out, st);
 }
 
 int vitdet_submit_images_host(vitdet_handle* h, const vitdet_image* images, int B, int mode, const vitdet_decode_params* params,
                               int want_packed, float* boxes_original_host, void* stream, int* ticket) {
     if (!params || !ticket) return fail(VITDET_E_INVALID, "submit_images_host: params and ticket must not be null");
-    HostImages in;
-    RC_TRY(images_table(h, "submit_images_host", images, B, params, boxes_original_host != nullptr, &in.table));
-    in.src.resize(B);
-    in.offs.resize(B + 1);
-    in.offs[0] = 0;
-    for (int i = 0; i < B; ++i) {
-        in.src[i] = reinterpret_cast<const char*>(images[i].pixels);
-        in.offs[i + 1] = in.offs[i] + static_cast<size_t>(images[i].height) * images[i].width * 3;
-    }
-    return submit_host_impl(h, in, 1, B, mode, params, want_packed, boxes_original_host, stream, ticket);
+    HostImages in{Input::Letterbox};
+    RC_TRY(letterbox_table(h, "submit_images_host", images, B, params, boxes_original_host != nullptr, &in.table));
+    for (int i = 0; i < B; ++i) in.add(images[i].pixels, static_cast<size_t>(images[i].height) * images[i].width * 3);
+    return submit_host_impl(h, in, B, mode, params, want_packed, boxes_original_host, stream, ticket);
 }
 
 // A caller's list of JPEG files -> the batch plan (every file parsed on the host; a rejected file fails the list, naming it).
@@ -1770,9 +1747,7 @@ int vitdet_jpeg_auto_ratio(int height, int width, int target_h, int target_w) {
 static int decode_jpeg_impl(vitdet_handle* h, const char* fn, const vitdet_jpeg* files, const int32_t* ratios, int B, uint8_t* out_dev,
                             const int64_t* out_offsets, void* stream) {
     if (!h || !out_dev || !out_offsets) return fail(VITDET_E_INVALID, "%s: null handle, out_dev or out_offsets", fn);
-    int cur = -1;
-    CU_TRY(cudaGetDevice(&cur));
-    if (cur != h->device) return fail(VITDET_E_INVALID, "%s: the handle lives on device %d but the current CUDA device is %d", fn, h->device, cur);
+    RC_TRY(check_device(h, fn));
     JpegBatch jb;
     RC_TRY(jpeg_files_plan(h, fn, files, ratios, B, out_offsets, &jb));
     for (int i = 0; i < B; ++i)
@@ -1783,26 +1758,17 @@ static int decode_jpeg_impl(vitdet_handle* h, const char* fn, const vitdet_jpeg*
     else CU_TRY(cudaEventCreateWithFlags(&h->jpeg_done, cudaEventDisableTiming));
     // descriptors and files in one pinned block, the files concatenated by the staging threads: the caller's bytes are
     // read before this returns
-    const size_t files_bytes = jb.file_off[B], pin_bytes = jb.desc.size() + files_bytes;
-    if (h->jpeg_pin_bytes < pin_bytes) {
-        if (h->jpeg_pin) cudaFreeHost(h->jpeg_pin);
-        h->jpeg_pin = nullptr; h->jpeg_pin_bytes = 0;
-        CU_TRY(cudaHostAlloc(reinterpret_cast<void**>(&h->jpeg_pin), pin_bytes, cudaHostAllocDefault));
-        h->jpeg_pin_bytes = pin_bytes;
-    }
-    memcpy(h->jpeg_pin, jb.desc.data(), jb.desc.size());
+    const size_t files_bytes = jb.file_off[B];
+    RC_TRY(h->jpeg_pin.ensure(jb.desc.size() + files_bytes));
+    char* files_pin = h->jpeg_pin.as<char>() + jb.desc.size();
     std::vector<const char*> src(B);
     for (int i = 0; i < B; ++i) src[i] = reinterpret_cast<const char*>(files[i].data);
     ensure_stage_pool(h);
-    h->stage_pool->copy(h->jpeg_pin + jb.desc.size(), src.data(), jb.file_off.data(), B);
-    RC_TRY(h->jpeg_work.ensure(jb.work_bytes));
+    h->stage_pool->copy(files_pin, src.data(), jb.file_off.data(), B);
     RC_TRY(h->jpeg_files.ensure(files_bytes));
-    CU_TRY(cudaMemcpyAsync(h->jpeg_work.p, h->jpeg_pin, jb.desc.size(), cudaMemcpyHostToDevice, st));
-    CU_TRY(cudaMemcpyAsync(h->jpeg_files.p, h->jpeg_pin + jb.desc.size(), files_bytes, cudaMemcpyHostToDevice, st));
-    h->launches += kJpegLaunches;
-    CU_TRY(jpeg_decode_launch(jb, h->jpeg_files.as<char>(), h->jpeg_work.p, out_dev, st));
+    CU_TRY(cudaMemcpyAsync(h->jpeg_files.p, files_pin, files_bytes, cudaMemcpyHostToDevice, st));
+    RC_TRY(jpeg_enqueue(h, jb, h->jpeg_pin.as<char>(), h->jpeg_files.as<char>(), h->jpeg_work, out_dev, nullptr, st));
     CU_TRY(cudaEventRecord(h->jpeg_done, st));
-    h->jpeg_stats = reinterpret_cast<const long long*>(h->jpeg_work.as<char>() + jb.o_stats);
     return 0;
 }
 
@@ -1819,29 +1785,24 @@ int vitdet_decode_jpeg_scaled(vitdet_handle* h, const vitdet_jpeg* files, const 
 static int submit_jpeg_impl(vitdet_handle* h, const char* fn, const vitdet_jpeg* files, const int32_t* ratios, int B, int mode,
                             const vitdet_decode_params* params, int want_packed, float* boxes_original_host, void* stream, int* ticket) {
     if (!h || !params || !ticket) return fail(VITDET_E_INVALID, "%s: handle, params and ticket must not be null", fn);
-    const int th = h->cfg.image_h, tw = h->cfg.image_w;
-    if (boxes_original_host && (params->image_h != static_cast<float>(th) || params->image_w != static_cast<float>(tw)))
-        return fail(VITDET_E_INVALID, "%s: boxes_original needs the decode at the model's input size %d x %d (params image_h / image_w)", fn, th, tw);
     JpegBatch jb;
     RC_TRY(jpeg_files_plan(h, fn, files, ratios, B, nullptr, &jb));
-    HostImages in;
-    in.table.resize(B);
-    in.src.resize(B);
-    in.offs.assign(jb.file_off.begin(), jb.file_off.end());
+    // the decoded images' sizes; each file's bytes are its image's host source, as the pixels are for separate images
+    std::vector<vitdet_image> images(B);
+    for (int i = 0; i < B; ++i) images[i] = vitdet_image{files[i].data, jb.height[i], jb.width[i]};
+    HostImages in{Input::Letterbox};
+    RC_TRY(letterbox_table(h, fn, images.data(), B, params, boxes_original_host != nullptr, &in.table));
     for (int i = 0; i < B; ++i) {
-        in.src[i] = reinterpret_cast<const char*>(files[i].data);
-        LetterboxImage& g = in.table[i];
-        if (!letterbox_image(nullptr, jb.height[i], jb.width[i], th, tw, &g))
-            return fail(VITDET_E_INVALID, "%s: image %d: a %d x %d image letterboxed to %d x %d resizes to %d x %d pixels", fn, i,
-                        jb.height[i], jb.width[i], th, tw, g.rh, g.rw);
+        in.add(files[i].data, static_cast<size_t>(files[i].bytes));
         // boxes_original in the file's pixels: the decoded image's box times file size / decoded size (1 at ratio 1)
+        LetterboxImage& g = in.table[i];
         g.file_h = jb.file_height[i];
         g.file_w = jb.file_width[i];
         g.file_hscale = static_cast<float>(g.file_h) / static_cast<float>(g.h);
         g.file_wscale = static_cast<float>(g.file_w) / static_cast<float>(g.w);
     }
     in.jpeg = &jb;
-    return submit_host_impl(h, in, 1, B, mode, params, want_packed, boxes_original_host, stream, ticket);
+    return submit_host_impl(h, in, B, mode, params, want_packed, boxes_original_host, stream, ticket);
 }
 
 int vitdet_submit_jpeg_host(vitdet_handle* h, const vitdet_jpeg* files, int B, int mode, const vitdet_decode_params* params,

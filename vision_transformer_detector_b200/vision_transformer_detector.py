@@ -261,15 +261,19 @@ def _is_uint8(x) -> bool:
     return str(getattr(x, "dtype", "")).endswith("uint8")
 
 
-def _pixels(x, normalize_uint8: bool) -> bool:
-    """True when `x` holds uint8 pixels AND the caller asked for the fused input normalisation x / 127.5 - 1
-    (vision_transformer_utilities.py:446-447, done inside the patch kernel).  Without the flag a uint8 array is only cast
-    to float32, which is what keras Model.predict does with it."""
-    return bool(normalize_uint8) and _is_uint8(x)
-
-
 def _is_torch_cuda(x) -> bool:
     return type(x).__module__.startswith("torch") and hasattr(x, "is_cuda") and x.is_cuda
+
+
+def _model_input(x, normalize_uint8: bool):
+    """(x as a contiguous numpy array or torch CUDA tensor, u8).  u8: `x` holds uint8 pixels AND the caller asked for the
+    fused input normalisation x / 127.5 - 1 (vision_transformer_utilities.py:446-447, done inside the patch kernel), and
+    stays uint8.  Otherwise x is cast to float32, which is what keras Model.predict does with a uint8 array."""
+    u8 = bool(normalize_uint8) and _is_uint8(x)
+    if _is_torch_cuda(x):
+        import torch
+        return (x.contiguous() if u8 else x.to(torch.float32).contiguous()), u8
+    return (np.ascontiguousarray(x) if u8 else np.ascontiguousarray(np.asarray(x, dtype=np.float32))), u8
 
 
 def _torch_stream_ptr(device) -> C.c_void_p:
@@ -330,11 +334,6 @@ def _jpeg_ratios(ratio, B: int, allow_auto: bool) -> list:
     return [code(r, f"file {i}: ") for i, r in enumerate(ratio)]
 
 
-def _full_size(ratio) -> bool:
-    """ratio is the plain default 1: the full-size entry points, exactly as before ratios existed."""
-    return isinstance(ratio, (int, np.integer)) and not isinstance(ratio, (bool, np.bool_)) and int(ratio) == 1
-
-
 def _alloc_records_np(B: int, S: int):
     return (np.empty((B, S, 6), np.float32), np.empty((B, S, 6), np.float32), np.empty((B, S), np.int32),
             np.empty((B, S), np.float32), np.empty((B, S), np.uint8), np.empty((B, S, 4), np.int32))
@@ -359,6 +358,17 @@ def _records_struct(decoded, class_id, class_conf, keep, corners, packed=None) -
     return d
 
 
+def _alloc_records(B: int, S: int, packed: bool = False, device=None) -> tuple[DetectionRecords, _capi.Detections]:
+    """Empty records of B images of S slots, the (B*S, 13) packed array only when asked for, and the Detections struct
+    that points at them: numpy arrays, or torch tensors on `device`."""
+    if device is None:
+        arrs = [*_alloc_records_np(B, S), np.empty((B * S, 13), np.float32) if packed else None]
+    else:
+        import torch
+        arrs = [*_alloc_records_torch(B, S, device), torch.empty((B * S, 13), dtype=torch.float32, device=device) if packed else None]
+    return DetectionRecords(*arrs), _records_struct(*arrs[1:])
+
+
 def decode_predictions(predictions, objectness_threshold=None, classification_threshold=None, strict=True,
                        image_size=None, use_transform_predictions=True, corner_scale=1.0) -> DetectionRecords:
     """transform_predictions + the score thresholds + class ids + corner boxes, on the GPU.
@@ -378,21 +388,19 @@ def decode_predictions(predictions, objectness_threshold=None, classification_th
         lead = tuple(x.shape[:-1])
         R = int(np.prod(lead)) if lead else 1
         with torch.cuda.device(x.device):
-            _, dec, cid, cc, keep, cor = _alloc_records_torch(R, 1, x.device)
-            st = _records_struct(dec, cid, cc, keep, cor)
+            r, st = _alloc_records(R, 1, device=x.device)
             _capi.check(lib.vitdet_decode(C.c_void_p(x.data_ptr()), R, C.byref(params), C.byref(st), _torch_stream_ptr(x.device)))
-        return DetectionRecords(predictions, dec.reshape(*lead, 6), cid.reshape(lead), cc.reshape(lead),
-                                keep.reshape(lead), cor.reshape(*lead, 4))
+        return DetectionRecords(predictions, r.decoded.reshape(*lead, 6), r.class_id.reshape(lead), r.class_conf.reshape(lead),
+                                r.keep.reshape(lead), r.corners.reshape(*lead, 4))
     x = np.ascontiguousarray(np.asarray(predictions, dtype=np.float32))
     if x.shape[-1] != 6:
         raise ValueError(f"predictions must have a last dimension of 6, got shape {x.shape}")
     lead = x.shape[:-1]
     R = int(np.prod(lead)) if lead else 1
-    _, dec, cid, cc, keep, cor = _alloc_records_np(R, 1)
-    st = _records_struct(dec, cid, cc, keep, cor)
+    r, st = _alloc_records(R, 1)
     _capi.check(lib.vitdet_decode_host(_capi.np_ptr(x), R, C.byref(params), C.byref(st)))
-    return DetectionRecords(x, dec.reshape(*lead, 6), cid.reshape(lead), cc.reshape(lead), keep.reshape(lead),
-                            cor.reshape(*lead, 4))
+    return DetectionRecords(x, r.decoded.reshape(*lead, 6), r.class_id.reshape(lead), r.class_conf.reshape(lead),
+                            r.keep.reshape(lead), r.corners.reshape(*lead, 4))
 
 
 def transform_predictions(inputs, image_size=None):
@@ -584,6 +592,7 @@ class VisionTransformerDetector:
         self.config = config
         self._lib = _capi.load()
         self._h = C.c_void_p()
+        self._inflight = {}     # ticket -> (B, packed, the submitted buffers, boxes_original or None)
         cfg_c = config.to_c()
         _capi.check(self._lib.vitdet_create(C.byref(cfg_c), C.byref(self._h)))
         self.compute_mode = compute_mode or os.environ.get("VITDET_MODE", "bf16")
@@ -766,29 +775,23 @@ class VisionTransformerDetector:
             image_size = self.config.input_shape[:2]
         params = _decode_params(objectness_threshold, classification_threshold, strict, image_size)
         mode = self._mode(compute_mode)
-        u8 = _pixels(x, normalize_uint8)
-        if _is_torch_cuda(x):
+        xi, u8 = _model_input(x, normalize_uint8)
+        if _is_torch_cuda(xi):
             import torch
-            xi = x.contiguous() if u8 else x.to(torch.float32).contiguous()
             with torch.cuda.device(xi.device):
-                logits, dec, cid, cc, keep, cor = _alloc_records_torch(B, S, xi.device)
-                pk = torch.empty((B * S, 13), dtype=torch.float32, device=xi.device) if packed else None
-                st = _records_struct(dec, cid, cc, keep, cor, pk)
+                recs, st = _alloc_records(B, S, packed, xi.device)
+                logits = C.c_void_p(recs.logits.data_ptr())
                 if u8:
-                    _capi.check(self._lib.vitdet_forward_u8(self._h, C.c_void_p(xi.data_ptr()), B, C.c_void_p(logits.data_ptr()), mode,
-                                                            C.byref(params), C.byref(st), _torch_stream_ptr(xi.device)))
+                    _capi.check(self._lib.vitdet_forward_u8(self._h, C.c_void_p(xi.data_ptr()), B, logits, mode, C.byref(params),
+                                                            C.byref(st), _torch_stream_ptr(xi.device)))
                 else:
-                    _capi.check(self._lib.vitdet_forward_decode(self._h, C.c_void_p(xi.data_ptr()), B, mode, C.byref(params),
-                                                                C.c_void_p(logits.data_ptr()), C.byref(st),
-                                                                _torch_stream_ptr(xi.device)))
-            return DetectionRecords(logits, dec, cid, cc, keep, cor, pk)
-        xi = np.ascontiguousarray(x) if u8 else np.ascontiguousarray(np.asarray(x, dtype=np.float32))
-        logits, dec, cid, cc, keep, cor = _alloc_records_np(B, S)
-        pk = np.empty((B * S, 13), np.float32) if packed else None
-        st = _records_struct(dec, cid, cc, keep, cor, pk)
+                    _capi.check(self._lib.vitdet_forward_decode(self._h, C.c_void_p(xi.data_ptr()), B, mode, C.byref(params), logits,
+                                                                C.byref(st), _torch_stream_ptr(xi.device)))
+            return recs
+        recs, st = _alloc_records(B, S, packed)
         fn = self._lib.vitdet_predict_host_u8 if u8 else self._lib.vitdet_predict_host
-        _capi.check(fn(self._h, _capi.np_ptr(xi), B, mode, C.byref(params), _capi.np_ptr(logits), C.byref(st), None))
-        return DetectionRecords(logits, dec, cid, cc, keep, cor, pk)
+        _capi.check(fn(self._h, _capi.np_ptr(xi), B, mode, C.byref(params), _capi.np_ptr(recs.logits), C.byref(st), None))
+        return recs
 
     def submit(self, x, objectness_threshold=None, classification_threshold=None, strict=True, image_size=None,
                compute_mode: str | None = None, packed: bool = False, normalize_uint8: bool = False) -> int:
@@ -799,28 +802,29 @@ class VisionTransformerDetector:
         if image_size is None:
             image_size = self.config.input_shape[:2]
         params = _decode_params(objectness_threshold, classification_threshold, strict, image_size)
-        u8 = _pixels(x, normalize_uint8)
-        xi = np.ascontiguousarray(x) if u8 else np.ascontiguousarray(np.asarray(x, dtype=np.float32))
+        xi, u8 = _model_input(x, normalize_uint8)
         ticket = C.c_int(-1)
         _capi.check(self._lib.vitdet_submit_host(self._h, _capi.np_ptr(xi), 1 if u8 else 0, B, self._mode(compute_mode), C.byref(params),
                                                  1 if packed else 0, None, C.byref(ticket)))
-        self._inflight = getattr(self, "_inflight", {})
-        self._inflight[ticket.value] = (B, packed, xi, None)    # xi kept alive: a page-locked buffer is read asynchronously
+        return self._in_flight(ticket, B, packed, xi)
+
+    def _in_flight(self, ticket: C.c_int, B: int, packed: bool, sources, boxes=None) -> int:
+        """Registers a submission for collect(); `sources` stay alive until then, as a page-locked buffer is read
+        asynchronously."""
+        self._inflight[ticket.value] = (B, packed, sources, boxes)
         return ticket.value
 
     def collect(self, ticket: int) -> DetectionRecords:
         """Waits for a submit() ticket and returns its records as numpy arrays."""
-        entry = getattr(self, "_inflight", {}).pop(ticket, None)
+        entry = self._inflight.pop(ticket, None)
         if entry is None:
             # not (or no longer) in flight: fail with the library's error type, like vitdet_collect itself does
             raise _capi.VitdetError(_capi.E_INVALID, f"collect: ticket {ticket} is not in flight")
         B, packed, _, boxes = entry
-        S = Constants.MAX_DETECT_OBJECTS_QUANTITY.value
-        logits, dec, cid, cc, keep, cor = _alloc_records_np(B, S)
-        pk = np.empty((B * S, 13), np.float32) if packed else None
-        st = _records_struct(dec, cid, cc, keep, cor, pk)
-        _capi.check(self._lib.vitdet_collect(self._h, int(ticket), _capi.np_ptr(logits), C.byref(st)))
-        return DetectionRecords(logits, dec, cid, cc, keep, cor, pk, boxes)
+        recs, st = _alloc_records(B, Constants.MAX_DETECT_OBJECTS_QUANTITY.value, packed)
+        recs.boxes_original = boxes
+        _capi.check(self._lib.vitdet_collect(self._h, int(ticket), _capi.np_ptr(recs.logits), C.byref(st)))
+        return recs
 
     # -- decoded images of any size ------------------------------------------------------------------
     @staticmethod
@@ -865,14 +869,12 @@ class VisionTransformerDetector:
         table = self._image_table(imgs, lambda t: t.data_ptr())
         dev = imgs[0].device
         with torch.cuda.device(dev):
-            logits, dec, cid, cc, keep, cor = _alloc_records_torch(B, S, dev)
-            pk = torch.empty((B * S, 13), dtype=torch.float32, device=dev) if packed else None
-            boxes = torch.empty((B, S, 4), dtype=torch.float32, device=dev)
-            st = _records_struct(dec, cid, cc, keep, cor, pk)
+            recs, st = _alloc_records(B, S, packed, dev)
+            recs.boxes_original = torch.empty((B, S, 4), dtype=torch.float32, device=dev)
             _capi.check(self._lib.vitdet_forward_images(self._h, table, B, self._mode(compute_mode), C.byref(params),
-                                                        C.c_void_p(logits.data_ptr()), C.byref(st), C.c_void_p(boxes.data_ptr()),
-                                                        _torch_stream_ptr(dev)))
-        return DetectionRecords(logits, dec, cid, cc, keep, cor, pk, boxes)
+                                                        C.c_void_p(recs.logits.data_ptr()), C.byref(st),
+                                                        C.c_void_p(recs.boxes_original.data_ptr()), _torch_stream_ptr(dev)))
+        return recs
 
     def submit_images(self, images, objectness_threshold=None, classification_threshold=None, strict=True,
                       compute_mode: str | None = None, packed: bool = False) -> int:
@@ -888,9 +890,7 @@ class VisionTransformerDetector:
         _capi.check(self._lib.vitdet_submit_images_host(self._h, self._image_table(imgs, lambda a: a.ctypes.data), B,
                                                         self._mode(compute_mode), C.byref(params), 1 if packed else 0,
                                                         _capi.np_ptr(boxes), None, C.byref(ticket)))
-        self._inflight = getattr(self, "_inflight", {})
-        self._inflight[ticket.value] = (B, packed, imgs, boxes)
-        return ticket.value
+        return self._in_flight(ticket, B, packed, imgs, boxes)
 
     # -- JPEG files ---------------------------------------------------------------------------------
     def detect_jpeg(self, files, objectness_threshold=None, classification_threshold=None, strict=True,
@@ -908,7 +908,7 @@ class VisionTransformerDetector:
 
     def submit_jpeg(self, files, objectness_threshold=None, classification_threshold=None, strict=True,
                     compute_mode: str | None = None, packed: bool = False, ratio=1) -> int:
-        """Asynchronous detect_jpeg() (vitdet_submit_jpeg_host[_scaled]), completed by collect(ticket); shares the two
+        """Asynchronous detect_jpeg() (vitdet_submit_jpeg_host_scaled), completed by collect(ticket); shares the two
         submission slots of submit().  Page-locked files are read directly and must stay alive until their ticket is
         collected."""
         arrs = _jpeg_arrays(files)
@@ -917,16 +917,10 @@ class VisionTransformerDetector:
         params = _decode_params(objectness_threshold, classification_threshold, strict, self.config.input_shape[:2])
         boxes = np.empty((B, S, 4), np.float32)
         ticket = C.c_int(-1)
-        if _full_size(ratio):
-            _capi.check(self._lib.vitdet_submit_jpeg_host(self._h, _jpeg_table(arrs), B, self._mode(compute_mode), C.byref(params),
-                                                          1 if packed else 0, _capi.np_ptr(boxes), None, C.byref(ticket)))
-        else:
-            _capi.check(self._lib.vitdet_submit_jpeg_host_scaled(self._h, _jpeg_table(arrs), (C.c_int32 * B)(*ratios), B,
-                                                                 self._mode(compute_mode), C.byref(params), 1 if packed else 0,
-                                                                 _capi.np_ptr(boxes), None, C.byref(ticket)))
-        self._inflight = getattr(self, "_inflight", {})
-        self._inflight[ticket.value] = (B, packed, arrs, boxes)
-        return ticket.value
+        _capi.check(self._lib.vitdet_submit_jpeg_host_scaled(self._h, _jpeg_table(arrs), (C.c_int32 * B)(*ratios), B,
+                                                             self._mode(compute_mode), C.byref(params), 1 if packed else 0,
+                                                             _capi.np_ptr(boxes), None, C.byref(ticket)))
+        return self._in_flight(ticket, B, packed, arrs, boxes)
 
     def predict(self, x, batch_size=None, verbose="auto", steps=None, callbacks=None, normalize_uint8: bool = False, **kwargs):
         """keras Model.predict: host array in, numpy (B, 17, 6) raw logits out.  `batch_size` only
@@ -935,8 +929,7 @@ class VisionTransformerDetector:
         if _is_torch_cuda(x):
             return self(x, normalize_uint8=normalize_uint8).cpu().numpy()
         B = self._check_images(np.shape(x))
-        u8 = _pixels(x, normalize_uint8)
-        xi = np.ascontiguousarray(x) if u8 else np.ascontiguousarray(np.asarray(x, dtype=np.float32))
+        xi, u8 = _model_input(x, normalize_uint8)
         logits = np.empty((B, Constants.MAX_DETECT_OBJECTS_QUANTITY.value, 6), np.float32)
         params = _decode_params(None, None, True, self.config.input_shape[:2])
         fn = self._lib.vitdet_predict_host_u8 if u8 else self._lib.vitdet_predict_host
@@ -952,8 +945,7 @@ class VisionTransformerDetector:
             return self.predict(x, normalize_uint8=normalize_uint8)
         import torch
         B = self._check_images(x.shape)
-        u8 = _pixels(x, normalize_uint8)
-        xi = x.contiguous() if u8 else x.to(torch.float32).contiguous()
+        xi, u8 = _model_input(x, normalize_uint8)
         with torch.cuda.device(xi.device):
             logits = torch.empty((B, Constants.MAX_DETECT_OBJECTS_QUANTITY.value, 6), dtype=torch.float32, device=xi.device)
             if u8:

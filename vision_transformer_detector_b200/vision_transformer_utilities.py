@@ -15,8 +15,8 @@ import ctypes as C
 import numpy as np
 
 from . import _capi
-from .vision_transformer_detector import (Constants, DetectorConfig, _full_size, _is_torch_cuda, _jpeg_arrays, _jpeg_ratios,
-                                          _jpeg_table, _torch_stream_ptr)
+from .vision_transformer_detector import (Constants, DetectorConfig, _is_torch_cuda, _jpeg_arrays, _jpeg_ratios, _jpeg_table,
+                                          _torch_stream_ptr)
 
 MODEL_IMAGE_HEIGHT, MODEL_IMAGE_WIDTH = Constants.MODEL_IMAGE_SIZE.value       # vision_transformer_utilities.py:23-24
 
@@ -115,11 +115,6 @@ def decode_jpeg(files, device=None, ratio=1) -> list:
         total += (h * w * 3 + 255) // 256 * 256
     with torch.cuda.device(index):
         buf = torch.empty(total, dtype=torch.uint8, device=dev)
-        off_c = (C.c_int64 * len(arrs))(*offs)
-        if _full_size(ratio):
-            _capi.check(lib.vitdet_decode_jpeg(_decoder(index), _jpeg_table(arrs), len(arrs), C.c_void_p(buf.data_ptr()), off_c,
-                                               _torch_stream_ptr(dev)))
-        else:
-            _capi.check(lib.vitdet_decode_jpeg_scaled(_decoder(index), _jpeg_table(arrs), (C.c_int32 * len(arrs))(*ratios),
-                                                      len(arrs), C.c_void_p(buf.data_ptr()), off_c, _torch_stream_ptr(dev)))
+        _capi.check(lib.vitdet_decode_jpeg_scaled(_decoder(index), _jpeg_table(arrs), (C.c_int32 * len(arrs))(*ratios), len(arrs),
+                                                  C.c_void_p(buf.data_ptr()), (C.c_int64 * len(arrs))(*offs), _torch_stream_ptr(dev)))
     return [buf[o:o + h * w * 3].view(h, w, 3) for o, (h, w, _) in zip(offs, shapes)]
